@@ -2,7 +2,7 @@
 """Benchmark of the Polya-Gamma hot path (bench contract: see the task statement).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl engine|reference]
-                    [--workload hybrid|pg1] [--num DRAWS | --draws DRAWS]
+                    [--workload hybrid|pg1] [--num DRAWS | --draws DRAWS] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d "C2"): 100M mixed-shape
 PG(b,z) draws per GPU -- b: 50% real U(0.5,200), 50% integer U{1..200};
@@ -21,6 +21,11 @@ host cores, on a bounded sample of the same workload.
 
 N > 1: one process per GPU under torchrun; observations are sharded, rank r draws
 global observations [r*num, (r+1)*num) -- no data-path collective ("weak").
+
+--dump-outputs DIR writes the draws of the last timed step to DIR/omega.npy (float64;
+DIR/omega_rank<r>.npy per rank under torchrun), so that two builds can be compared draw
+for draw on the same inputs.  A batch larger than DUMP_DRAWS is sampled: one draw from
+each of DUMP_DRAWS equal strata, at offsets drawn from a fixed seed.
 """
 import argparse
 import json
@@ -40,6 +45,7 @@ BYTES_PER_DRAW = {"hybrid": 24, "pg1": 20}
 # fp64-equivalent flop model per draw, SURVEY.md section 8(d): 0.9 kFLOP for a Devroye
 # PG(1,z) draw; the mixed workload is weighted by its regime shares (SP ~ 10x).
 KFLOP_PER_DRAW = {"pg1": 0.9, "hybrid": 0.786 * 9.0 + 0.058 * 3.0 + 0.15 * 0.3 + 0.005 * 1.35 + 0.0013 * 60.0}
+DUMP_DRAWS = 4 << 20            # 32 MB of fp64 draws per run, over all ranks
 
 
 def parse():
@@ -55,7 +61,25 @@ def parse():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the PG(1,z) and logit-Gibbs extras")
     ap.add_argument("--gibbs-iters", type=int, default=200)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the draws of the last timed step to DIR/omega.npy")
     return ap.parse_args()
+
+
+def dump_index(num, world=1):
+    """Which of a rank's num draws --dump-outputs writes: None for all of them, else the fixed
+    stratified sample the module docstring describes."""
+    import numpy as np
+    k = DUMP_DRAWS // world
+    if num <= k:
+        return None
+    rng = np.random.default_rng([SEED, num])
+    return np.arange(k, dtype=np.int64) * num // k + rng.integers(0, num // k, k)
+
+
+def dump_outputs(directory, name, x):
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), np.asarray(x, dtype=np.float64))
 
 
 def make_inputs_numpy(workload, num, obs0=0):
@@ -128,15 +152,15 @@ def load_oracle():
 
 
 def time_cpu(workload, sample, nthreads):
-    """Reference CPU sampler on `sample` draws of the workload; returns (seconds, kind)."""
+    """Reference CPU sampler on `sample` draws of the workload; returns (seconds, kind, draws)."""
     O = load_oracle()
     shape, z = make_inputs_numpy(workload, sample)
     t = time.perf_counter()
     if workload == "pg1":
-        O.rpg_devroye(shape, z, seed=SEED, nthreads=nthreads)
+        x = O.rpg_devroye(shape, z, seed=SEED, nthreads=nthreads)
     else:
-        O.rpg_hybrid(shape, z, seed=SEED, nthreads=nthreads)
-    return time.perf_counter() - t, O.kind
+        x = O.rpg_hybrid(shape, z, seed=SEED, nthreads=nthreads)
+    return time.perf_counter() - t, O.kind, x
 
 
 def measured_pipe_peaks(L):
@@ -217,12 +241,15 @@ def run_reference(args, rank, world):
     t = 0.0
     kind = "port"
     for _ in range(args.steps):
-        dt, kind = time_cpu(args.workload, sample, cores)
+        dt, kind, x = time_cpu(args.workload, sample, cores)
         t += dt
+    if args.dump_outputs:
+        idx = dump_index(sample)
+        dump_outputs(args.dump_outputs, "omega", x if idx is None else x[idx])
     value = sample * args.steps / t
     desc = f"first {sample} draws of the workload per step, all {cores} host threads (OpenMP, one RNG+sampler per thread)"
     one = max(sample // 8, 1)
-    dt1, _ = time_cpu(args.workload, one, 1)
+    dt1, _, _ = time_cpu(args.workload, one, 1)
     print(json.dumps({
         "impl": "reference", "metric": "pg_draws_per_sec", "value": value, "unit": "draws/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -343,6 +370,10 @@ def main():
     clocks = sampler.stop(t_wall0, t_wall1, t_warm0) if sampler else None
     value = world * num * args.steps / (total_ms * 1e-3)
     mean_omega = float(x_d[: 1 << 20].mean().item())
+    if args.dump_outputs:            # now: the passes below overwrite x_d
+        idx = dump_index(num, world)
+        x = x_d if idx is None else x_d[torch.from_numpy(idx).to(dev)]
+        dump_outputs(args.dump_outputs, "omega" if world == 1 else f"omega_rank{rank}", x.cpu().numpy())
     # dominant kernel of the step, timed live with CUDA events on the launch stream (separate,
     # untimed pass so the event records do not sit inside the headline region)
     stage_ms, stage_launches, regime_counts = None, None, None
@@ -455,9 +486,9 @@ def main():
         cores = os.cpu_count() or 1
         sample = min(CPU_SAMPLE[wl], num)
         time_cpu(wl, max(sample // 16, 1), cores)
-        dt, kind = time_cpu(wl, sample, cores)
+        dt, kind, _ = time_cpu(wl, sample, cores)
         one = max(sample // 8, 1)
-        dt1, _ = time_cpu(wl, one, 1)
+        dt1, _, _ = time_cpu(wl, one, 1)
         cpu = {"value": sample / dt, "unit": "draws/s", "cores": cores, "kind": kind,
                "sample": f"first {sample} draws of the workload, all {cores} host threads, {dt:.2f} s wall",
                "value_1_core": one / dt1,

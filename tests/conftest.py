@@ -21,18 +21,6 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The reference's own sampler sources compiled in place (oracle/_ref)."""
-    from oracle import loader
-    if not loader.available("reference"):
-        if os.path.isdir("/root/reference/Code/C"):
-            loader.build(("ref",))
-        else:
-            pytest.skip("oracle/_ref not built and /root/reference not mounted")
-    return loader.Oracle("reference")
-
-
-@pytest.fixture(scope="session")
 def oracle(request):
     """Best available checker: the compiled reference if present, else the port."""
     from oracle import loader

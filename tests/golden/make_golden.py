@@ -106,9 +106,22 @@ def main():
     y = np.concatenate([2.0 ** rng.uniform(-6, 6, 500), [0.0625, 1.0, 15.999, 0.05, 17.0, 0.999999, 1.000001]])
     out.update(vev_y=y, vev_v=np.array([R.v_eval(t) for t in y]))
 
+    zero_unread_tape_entries(out)
     np.savez_compressed(OUT, **out)
     print("wrote", OUT, os.path.getsize(OUT), "bytes;",
           "exhausted:", {k: int(v[:, 4].sum()) for k, v in out.items() if k.endswith("_trace")})
+
+
+def zero_unread_tape_entries(out):
+    """Zero every tape entry past the count of variates its observation consumed (trace columns
+    u, e, n, g): a tape row is read from its start, one entry per variate, so these entries never
+    reach a sampler and the draws do not change, while the file shrinks to a quarter of its size."""
+    for key in [k for k in out if k.endswith("_trace")]:
+        p, used = key[:-len("_trace")], out[key]
+        for col, k in enumerate("ueng"):
+            t = out.get(f"{p}_t{k}")
+            if t is not None:
+                t[np.arange(t.shape[1])[None, :] >= used[:, col:col + 1]] = 0.0
 
 
 if __name__ == "__main__":

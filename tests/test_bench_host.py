@@ -1,5 +1,6 @@
-"""CPU tests of bench.py's host logic: workload generation (BASELINE.json configs[1], SURVEY.md 8d "C2"),
-clock-sample parsing, and the reference arm's JSON contract on a tiny sample."""
+"""Tests of bench.py: on the CPU its host logic -- workload generation (BASELINE.json configs[1], SURVEY.md
+8d "C2"), clock-sample parsing, the reference arm's JSON contract and --dump-outputs on a tiny sample; on the
+GPU, --dump-outputs of the engine arm."""
 import json
 import os
 import subprocess
@@ -7,6 +8,7 @@ import sys
 import time
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -51,9 +53,10 @@ def test_clock_sampler_parsing():
     assert c.stop(t - 0.5, t + 0.5, t - 10)["reasons"] == ["no samples"]
 
 
-def test_reference_arm_prints_one_json_line_with_the_contract_keys():
+def test_reference_arm_prints_one_json_line_with_the_contract_keys(tmp_path):
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                          "--warmup", "1", "--num", "200000"], capture_output=True, text=True, timeout=600)
+                          "--warmup", "1", "--num", "200000", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
     lines = [ln for ln in out.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, out.stdout + out.stderr[-500:]
     d = json.loads(lines[0])
@@ -62,6 +65,40 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert d["cpu_baseline"]["kind"] in ("reference", "port") and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"] == {"value": d["value"], "unit": "draws/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["config"]["draws_per_gpu_per_step"] == 200000
+    # --dump-outputs: the draws of the timed step, as the sampler computed them
+    from oracle import loader
+    assert os.listdir(tmp_path) == ["omega.npy"]
+    x = np.load(tmp_path / "omega.npy")
+    h, z = bench.make_inputs_numpy("hybrid", 200000)
+    assert x.dtype == np.float64
+    assert np.array_equal(x, loader.Oracle(d["cpu_baseline"]["kind"]).rpg_hybrid(h, z, seed=bench.SEED, nthreads=4))
+
+
+def test_dump_sample_is_fixed_and_spans_the_batch():
+    assert bench.dump_index(bench.DUMP_DRAWS) is None
+    num = 100_000_000
+    idx = bench.dump_index(num)
+    k = bench.DUMP_DRAWS
+    assert idx.size == k and idx.size * 8 <= 64 << 20
+    stratum = np.arange(k, dtype=np.int64)                     # one draw inside each of k equal strata
+    assert np.all(stratum * num // k <= idx) and np.all(idx < (stratum + 1) * num // k)
+    assert np.array_equal(idx, bench.dump_index(num))
+    assert bench.dump_index(num, world=8).size == bench.DUMP_DRAWS // 8
+
+
+@pytest.mark.gpu
+def test_engine_dump_is_the_last_timed_step(engine, tmp_path):
+    """bench.py --dump-outputs writes the draws of the last timed step (call id steps - 1), sampled when the
+    batch is larger than DUMP_DRAWS."""
+    num, steps = bench.DUMP_DRAWS + 1_000_003, 3
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1",
+                          "--num", str(num), "--no-extras", "--no-cpu-baseline", "--no-e2e",
+                          "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout)["steps"] == steps
+    h, z = bench.make_inputs_numpy("hybrid", num)
+    want = engine.rpg_seeded("hybrid", h, z, seed=bench.SEED, call_id=steps - 1)[bench.dump_index(num)]
+    assert np.array_equal(np.load(tmp_path / "omega.npy"), want)
 
 
 def test_reference_arm_under_torchrun_prints_on_rank_0_only():
