@@ -386,7 +386,7 @@ int bl_logit_chains_dev(double *beta, const double *y, const double *tX, const d
 {
     if (bl_ensure_ready_internal()) return 1;
     std::string err;
-    if (logit_chains_device(beta, y, tX, n, m0, P0, chains, N, P, samp, burn, seed, flags, (cudaStream_t)stream, err))
+    if (logit_chains_device(beta, y, tX, n, m0, P0, chains, N, P, samp, burn, seed, flags, false, (cudaStream_t)stream, err))
         return report(err, nullptr);
     return 0;
 }
@@ -403,7 +403,41 @@ int bl_logit_chains(double *beta, const double *y, const double *tX, const doubl
     double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
     double *dbeta = d.put(nullptr, (size_t)chains * P * samp, err);
     if (!err.empty()) return report(err, nullptr);
-    if (logit_chains_device(dbeta, dy, dX, dn, dm0, dP0, chains, N, P, samp, burn, seed, flags,
+    if (logit_chains_device(dbeta, dy, dX, dn, dm0, dP0, chains, N, P, samp, burn, seed, flags, false,
+                            (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * (size_t)chains * P * samp, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
+int bl_logit_multichain_dev(double *beta, const double *y, const double *tX, const double *n, const double *m0,
+                            const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
+                            int flags, void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    std::string err;
+    if (logit_chains_device(beta, y, tX, n, m0, P0, chains, N, P, samp, burn, seed, flags, true, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
+int bl_logit_multichain(double *beta, const double *y, const double *tX, const double *n, const double *m0,
+                        const double *P0, int chains, int N, int P, int samp, int burn, uint64_t seed, int flags)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    // checked before any buffer is made: the device driver repeats the checks
+    if (chains <= 0 || N <= 0 || P <= 0 || samp <= 0 || burn < 0) return report("logit_multichain: bad dimensions", nullptr);
+    if ((int64_t)chains * N >= (1LL << 31))
+        return report("logit_multichain: chains * N must stay below 2^31 observations per call", nullptr);
+    if (P > 256) return report("P > 256 covariates is not supported by the single-CTA beta draw", nullptr);
+    std::string err;
+    Dev d;
+    double *dy = d.put(y, N, err), *dX = d.put(tX, (size_t)N * P, err), *dn = d.put(n, N, err);     // one copy of X
+    double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
+    double *dbeta = d.put(nullptr, (size_t)chains * P * samp, err);
+    if (!err.empty()) return report(err, nullptr);
+    if (logit_chains_device(dbeta, dy, dX, dn, dm0, dP0, chains, N, P, samp, burn, seed, flags, true,
                             (cudaStream_t)bl_stream_internal(), err))
         return report(err, nullptr);
     cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * (size_t)chains * P * samp, cudaMemcpyDeviceToHost);

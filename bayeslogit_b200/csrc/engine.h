@@ -60,6 +60,10 @@ bool devroye_binned(int64_t num, int64_t bin_min);         // whether a batch of
 bool logit_psi_draw_ok(const double *tX, int P);
 cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, const double *tX, const double *beta,
                                   int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream);
+// The same for `chains` chains that share ONE set of N rows (n [N], tX P x N): chain c meets beta + c * beta_stride
+// and the streams of id.seed + c; x: omega [chains][N].  Same conditions on P and tX.
+cudaError_t launch_logit_psi_draw_shared(double *x, const int *n, const double *tX, const double *beta,
+                                         int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream);
 
 // rpg_hybrid through regime binning (pg_hybrid.cu); num <= 2^31-1, `work` = device scratch of
 // hybrid_workspace_bytes(num) bytes that stays valid until the stream has drained.
@@ -82,9 +86,10 @@ int nb_gibbs_device(double *w_out, double *beta_out, const double *y, const doub
 int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const double *y, const double *tX,
                        double d0, const double *m0, const double *P0, int64_t N, int P, int samp, int burn,
                        uint64_t seed, uint64_t obs0, bool sharded, int real_d, cudaStream_t st, std::string &err);
+// shared_rows: every chain runs on the same N rows (y, n [N], tX P x N) instead of rows [c N, (c+1) N) of its own
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
-                        uint64_t seed, int flags, cudaStream_t st, std::string &err);
+                        uint64_t seed, int flags, bool shared_rows, cudaStream_t st, std::string &err);
 int logit_em_device(double *beta, const double *y, const double *tX, const double *n, int64_t N,
                     int P, double tol, int max_iter, int *iters, cudaStream_t st, std::string &err);
 // duplicate-row merge on device-resident data (merge.cu); returns M, -1 (CUDA error), -2 (needs the exact host merge)

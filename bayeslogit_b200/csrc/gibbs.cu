@@ -518,7 +518,7 @@ struct Sweep {
     {
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));
         if (xbeta_mma_ok(tX, P))
-            launch_pdl(k_xbeta_mma<false>, dim3(grid), dim3(256), 0, st, out, tX, beta, 0, 1, N, P, off, off_scale, shift, MlogitNext{});
+            launch_pdl(k_xbeta_mma<false>, dim3(grid), dim3(256), 0, st, out, tX, N * P, beta, 0, 1, N, P, off, off_scale, shift, MlogitNext{});
         else
             k_xbeta<<<grid, 256, P * sizeof(double), st>>>(out, tX, beta, off, off_scale, shift, N, P);
         count_launch();
@@ -528,7 +528,7 @@ struct Sweep {
     void xbeta_mlogit(double *out, const double *beta, const MlogitNext &mn)
     {
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));
-        launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, out, tX, beta, 0, 1, N, P, nullptr, 0.0, 0.0, mn);
+        launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, out, tX, N * P, beta, 0, 1, N, P, nullptr, 0.0, 0.0, mn);
         count_launch();
     }
 
@@ -543,11 +543,11 @@ struct Sweep {
         int tiles = nt * (nt + 1) / 2;
         const bool packed = gram_packed(P);
         if (nt > 1)
-            launch_pdl(k_gram_partial<kGramRows, false>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(true), st, part, tX, wv, N, P, nt, nslab_diag, nullptr);
+            launch_pdl(k_gram_partial<kGramRows, false>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(true), st, part, tX, N * P, wv, N, P, nt, nslab_diag, nullptr);
         else if (packed)
-            launch_pdl(k_gram_partial<kGramRowsDiag, true, true>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(false, true), st, part, tX, wv, N, P, nt, 0, cvec);
+            launch_pdl(k_gram_partial<kGramRowsDiag, true, true>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(false, true), st, part, tX, N * P, wv, N, P, nt, 0, cvec);
         else
-            launch_pdl(k_gram_partial<kGramRowsDiag, true>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(false), st, part, tX, wv, N, P, nt, 0, nullptr);
+            launch_pdl(k_gram_partial<kGramRowsDiag, true>, dim3(nslab, tiles), dim3(256), gram_smem_bytes(false), st, part, tX, N * P, wv, N, P, nt, 0, nullptr);
         const int tail_in_part = packed && cvec ? 1 : 0;
         PeerPush px{};
         pending = PeerWait{};
@@ -745,22 +745,28 @@ int logit_gibbs_device(double *w_out, double *beta_out, const double *y, const d
 // with seed + c (same streams, same slot semantics); every kernel of the sweep is launched once
 // for the whole batch with the chain as a grid dimension, so the one-CTA beta draws of the chains
 // run side by side instead of sitting on each chain's critical path.  omega is not returned.
+// shared_rows (bl_logit_multichain): every chain runs on the same N rows of tX / y / n -- the usual
+// several chains from different seeds on one data set.  X is held and read once: kappa, the shapes and
+// X' kappa are formed once, psi + omega of all chains come from one pass over X (k_logit_psi_draw_shared),
+// the Gram kernels read X with a chain stride of 0.  Chain c is bit for bit the chain of the replicated
+// call (chains copies of the rows, same seed).
 // beta_out: [chains][samp][P].
 // ------------------------------------------------------------------------------------
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
-                        uint64_t seed, int flags, cudaStream_t st, std::string &err)
+                        uint64_t seed, int flags, bool shared_rows, cudaStream_t st, std::string &err)
 {
-    if (chains <= 0 || N <= 0 || P <= 0 || samp <= 0 || burn < 0) { err = "logit_chains: bad dimensions"; return 1; }
+    const char *who = shared_rows ? "logit_multichain" : "logit_chains";
+    if (chains <= 0 || N <= 0 || P <= 0 || samp <= 0 || burn < 0) { err = std::string(who) + ": bad dimensions"; return 1; }
     const int64_t T = (int64_t)chains * N;
-    if (T >= (1LL << 31)) { err = "logit_chains: chains * N must stay below 2^31 observations per call"; return 1; }
+    if (T >= (1LL << 31)) { err = std::string(who) + ": chains * N must stay below 2^31 observations per call"; return 1; }
     if (P > 256) { err = "P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
     const int mode = (flags & BL_GIBBS_PLAIN_BETA) ? kBetaPlain : kBetaConstrained;
     const size_t beta_smem = mode == kBetaConstrained
         ? beta_tn_doubles(P) * sizeof(double)
         : std::max((2 * (size_t)(P | 1) * P + 5 * (size_t)P) * sizeof(double),
                    P <= 64 ? (beta_fast_e_offset(P) + 64) * sizeof(double) : (size_t)0);
-    if (beta_smem > 200 * 1024) { err = "logit_chains: P too large for the shared-memory beta draw"; return 1; }
+    if (beta_smem > 200 * 1024) { err = std::string(who) + ": P too large for the shared-memory beta draw"; return 1; }
     DevMem mem;
     mem.st = st;
     const int nt = cdiv(P, kGramTile), tiles = nt * (nt + 1) / 2;
@@ -768,16 +774,23 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
                                        std::max<int64_t>(1, N / (4 * kGramRows)));
     const int slabs_total = nt > 1 ? 2 * nslab : nslab;
     const size_t accn = (size_t)P * P + P;
+    const bool fused = !(flags & BL_GIBBS_UNFUSED) && logit_psi_draw_ok(tX, P);
+    const int xchains = shared_rows ? 1 : chains;          // copies of the rows held
+    const int64_t R = xchains * N;
+    const int64_t x_stride = shared_rows ? 0 : N * P;      // chain c's rows: tX + c x_stride
+    // the fused shared-rows kernel reads the N shapes of the shared rows; the refill kernel (unfused) walks all
+    // chains * N (row, chain) pairs and reads one shape per pair
+    const int64_t nshape = shared_rows && fused ? N : T;
     double *psi, *w, *kappa, *acc, *part, *xtv_part, *b0, *bP;
     int *shape, *status;
     void *work;
     GB_CK(mem.get(&psi, T));
     GB_CK(mem.get(&w, T));
-    GB_CK(mem.get(&kappa, T));
-    GB_CK(mem.get(&shape, T));
+    GB_CK(mem.get(&kappa, R));
+    GB_CK(mem.get(&shape, nshape));
     GB_CK(mem.get(&acc, accn * chains));
     GB_CK(mem.get(&part, (size_t)chains * tiles * slabs_total * kGramTile * kGramTile));
-    GB_CK(mem.get(&xtv_part, (size_t)chains * P));
+    GB_CK(mem.get(&xtv_part, (size_t)xchains * P));
     GB_CK(mem.get(&b0, P));
     GB_CK(mem.get(&bP, (size_t)chains * P));
     GB_CK(mem.get(&status, 1));
@@ -796,25 +809,28 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
     }
     const int64_t bstride = (int64_t)P * samp;
 
-    // bP_c = P0 m0 + X_c'(n (y - 1/2))
-    k_kappa<<<cdiv(T, 256), 256, 0, st>>>(kappa, y, n, 0.0, T);
-    k_shape_int<<<cdiv(T, 256), 256, 0, st>>>(shape, n, T);
+    // bP_c = P0 m0 + X_c'(n (y - 1/2)); with shared rows the same for every chain: formed once, then copied
+    k_kappa<<<cdiv(R, 256), 256, 0, st>>>(kappa, y, n, 0.0, R);
+    k_shape_int<<<cdiv(R, 256), 256, 0, st>>>(shape, n, R);
     k_matvec<<<cdiv(P, 128), 128, 0, st>>>(b0, P0, m0, P);
-    launch_xtv(dim3(1, chains), st, xtv_part, tX, kappa, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
-    k_xtv_reduce<<<dim3(cdiv(P, 128), chains), 128, 0, st>>>(bP, b0, nullptr, xtv_part, P, 1);
+    launch_xtv(dim3(1, xchains), st, xtv_part, tX, kappa, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
+    k_xtv_reduce<<<dim3(cdiv(P, 128), xchains), 128, 0, st>>>(bP, b0, nullptr, xtv_part, P, 1);
     count_launch(5);
+    for (int c = xchains; c < chains; ++c)
+        GB_CK(cudaMemcpyAsync(bP + (size_t)c * P, bP, sizeof(double) * P, cudaMemcpyDeviceToDevice, st));
+    for (int64_t c = R; c < nshape; c += N)
+        GB_CK(cudaMemcpyAsync(shape + c, shape, sizeof(int) * N, cudaMemcpyDeviceToDevice, st));
     GB_CK(cudaMemsetAsync(beta_out, 0, sizeof(double) * (size_t)bstride * chains, st));
 
     auto xbeta = [&](const double *beta) {
         const int64_t trips = (int64_t)chains * ((N + 31) / 32);
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (trips + 7) / 8));
         if (xbeta_mma_ok(tX, P))
-            k_xbeta_mma<false><<<grid, 256, 0, st>>>(psi, tX, beta, bstride, chains, N, P, nullptr, 0.0, 0.0, MlogitNext{});
+            k_xbeta_mma<false><<<grid, 256, 0, st>>>(psi, tX, x_stride, beta, bstride, chains, N, P, nullptr, 0.0, 0.0, MlogitNext{});
         else
-            k_xbeta_chains<<<grid, 256, 0, st>>>(psi, tX, beta, bstride, chains, (int)N, P);
+            k_xbeta_chains<<<grid, 256, 0, st>>>(psi, tX, x_stride, beta, bstride, chains, (int)N, P);
         count_launch();
     };
-    const bool fused = !(flags & BL_GIBBS_UNFUSED) && logit_psi_draw_ok(tX, P);
     const bool timing = getenv("BL_GIBBS_TIMING") != nullptr;
     cudaEvent_t ev[6];
     if (timing) for (auto &x : ev) cudaEventCreate(&x);
@@ -828,16 +844,19 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
             const bool tm = timing && phase == 1 && m == iters;       // BL_GIBBS_TIMING=1: stage times
             if (tm) cudaEventRecord(ev[0], st);
             StreamId id{seed, 0, t, (uint32_t)N};
-            cudaError_t e = fused ? launch_logit_psi_draw(w, nullptr, shape, tX, bpsi, bstride, chains, N, P, id, st)
-                                  : launch_devroye_refill(w, shape, psi, T, id, st, work);
+            // one chain: shared and own rows are the same layout, and k_logit_psi_draw is the faster kernel for it
+            // (no trip through shared memory: 146 against 153 us at N = 1M, P = 64)
+            cudaError_t e = !fused                    ? launch_devroye_refill(w, shape, psi, T, id, st, work)
+                            : shared_rows && chains > 1 ? launch_logit_psi_draw_shared(w, shape, tX, bpsi, bstride, chains, N, P, id, st)
+                                                        : launch_logit_psi_draw(w, nullptr, shape, tX, bpsi, bstride, chains, N, P, id, st);
             if (e != cudaSuccess) { err = cudaGetErrorString(e); return 1; }
             if (tm) cudaEventRecord(ev[1], st);
             if (nt > 1)
-                k_gram_partial<kGramRows, false><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(true), st>>>(part, tX, w, N, P, nt);
+                k_gram_partial<kGramRows, false><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(true), st>>>(part, tX, x_stride, w, N, P, nt);
             else if (packed)
-                k_gram_partial<kGramRowsDiag, true, true><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(false, true), st>>>(part, tX, w, N, P, nt);
+                k_gram_partial<kGramRowsDiag, true, true><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(false, true), st>>>(part, tX, x_stride, w, N, P, nt);
             else
-                k_gram_partial<kGramRowsDiag, true><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(false), st>>>(part, tX, w, N, P, nt);
+                k_gram_partial<kGramRowsDiag, true><<<dim3(nslab, tiles, chains), 256, gram_smem_bytes(false), st>>>(part, tX, x_stride, w, N, P, nt);
             if (tm) cudaEventRecord(ev[2], st);
             k_gram_reduce<<<dim3(cdiv((int64_t)P * P, 32), chains), 256, 0, st>>>(acc, nullptr, part, P, nt, slabs_total, PeerPush{}, packed ? 1 : 0);
             if (tm) cudaEventRecord(ev[3], st);
@@ -856,8 +875,8 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
                 cudaEventSynchronize(ev[5]);
                 float d[5];
                 for (int k = 0; k < 5; ++k) cudaEventElapsedTime(&d[k], ev[k], ev[k + 1]);
-                fprintf(stderr, "[bl chains timing, us] draw %.1f gram %.1f reduce %.1f beta %.1f xbeta %.1f\n",
-                        d[0] * 1e3, d[1] * 1e3, d[2] * 1e3, d[3] * 1e3, d[4] * 1e3);
+                fprintf(stderr, "[bl %s timing, us] draw %.1f gram %.1f reduce %.1f beta %.1f xbeta %.1f\n",
+                        shared_rows ? "multichain" : "chains", d[0] * 1e3, d[1] * 1e3, d[2] * 1e3, d[3] * 1e3, d[4] * 1e3);
                 for (auto &x : ev) cudaEventDestroy(x);
             }
             if (phase == 1) {
@@ -870,7 +889,7 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
     int h = 0;
     GB_CK(cudaMemcpyAsync(&h, status, sizeof(int), cudaMemcpyDeviceToHost, st));
     GB_CK(cudaStreamSynchronize(st));
-    if (h != 0) { err = "logit_chains: a chain's posterior precision is not positive definite"; return 1; }
+    if (h != 0) { err = std::string(who) + ": a chain's posterior precision is not positive definite"; return 1; }
     return 0;
 }
 

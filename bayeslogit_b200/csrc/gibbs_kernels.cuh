@@ -75,10 +75,11 @@ k_xbeta(double *__restrict__ psi, const double *__restrict__ tX, const double *_
     }
 }
 
-// The same for a batch of independent chains: rows [c N, (c+1) N) belong to chain c and meet
-// beta_c = beta[c * beta_stride ..).  Trips of 32 rows never straddle two chains.
+// The same for a batch of independent chains: chain c reads the N rows at tX + c * x_stride (N P: its own
+// rows; 0: rows shared by all chains), meets beta_c = beta[c * beta_stride ..) and writes psi[c N ..).
+// Trips of 32 rows never straddle two chains.
 static __global__ void __launch_bounds__(256, 2)
-k_xbeta_chains(double *__restrict__ psi, const double *__restrict__ tX, const double *__restrict__ beta,
+k_xbeta_chains(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ beta,
                int64_t beta_stride, int chains, int N, int P)
 {
     const int lane = threadIdx.x & 31;
@@ -90,7 +91,7 @@ k_xbeta_chains(double *__restrict__ psi, const double *__restrict__ tX, const do
         const int ch = (int)(trip / tpc);
         const int i0 = (int)(trip - (int64_t)ch * tpc) << 5;
         const double *bc = beta + ch * beta_stride;
-        const double *base = tX + ((size_t)ch * N + i0) * P;
+        const double *base = tX + ch * x_stride + (size_t)i0 * P;
         double acc[32];
 #pragma unroll
         for (int r = 0; r < 32; ++r) acc[r] = 0.0;
@@ -179,7 +180,7 @@ __device__ __forceinline__ void dmma884(double &c0, double &c1, double a, double
 // of the 8 rows.  No cross-lane reduction and two accumulator registers per 8 rows, so a warp
 // keeps a whole 32-row trip of loads in flight; the lane-strided k_xbeta spends ~150 of its ~220
 // instructions per trip in the transposing butterfly and idles HBM meanwhile (4.6 TB/s at P = 64,
-// 2.4 TB/s at P = 32).  Chains: rows [c N, (c+1) N) meet beta + c * beta_stride.
+// 2.4 TB/s at P = 32).  Chains: the N rows at tX + c * x_stride meet beta + c * beta_stride, psi goes to [c N ..).
 // ---------------------------------------------------------------------------------
 // mlogit epilogue (MultLogit.hpp:246-258, 275-277): the category whose coefficients were just drawn gets its new
 // linear predictor XB_j = X beta_j and E_j = exp(XB_j) (cached so that no category's exponentials are recomputed
@@ -199,7 +200,7 @@ struct MlogitNext {
 
 template <bool kMlogit>
 static __global__ void __launch_bounds__(256, 2)
-k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, const double *__restrict__ beta,
+k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ beta,
             int64_t beta_stride, int chains, int64_t N, int P,
             const double *__restrict__ off, double off_scale, double shift, MlogitNext mn)
 {
@@ -213,7 +214,7 @@ k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, const doubl
         const int64_t ch = chains > 1 ? trip / tpc : 0;
         const int64_t i0 = (trip - ch * tpc) << 5;
         const double *bc = beta + ch * beta_stride + 2 * tig;
-        const double *base = tX + ((size_t)ch * N + i0 + gid) * P + 2 * tig;
+        const double *base = tX + ch * x_stride + (i0 + gid) * P + 2 * tig;
         double c[4][2] = {};
         bool rv[4];
 #pragma unroll
@@ -409,14 +410,15 @@ __device__ __forceinline__ void gram_pack_store(const double (&c)[9][2], double 
 
 template <int kRows, bool kBalancedDiag, bool kPacked = false>
 __global__ void __launch_bounds__(256)
-k_gram_partial(double *__restrict__ part, const double *__restrict__ tX, const double *__restrict__ w,
+k_gram_partial(double *__restrict__ part, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ w,
                int64_t N, int P, int nt, int nslab_diag = 0, const double *__restrict__ cv = nullptr)
 {
     BL_PDL_ENTER();
     extern __shared__ __align__(16) double gsm[];
     const int nthr = blockDim.x;
-    // batched independent chains: blockIdx.z = chain (its own rows, weights and partial tiles)
-    tX += (size_t)blockIdx.z * N * P;
+    // batched independent chains: blockIdx.z = chain (its weights and partial tiles; its rows at tX + chain x_stride:
+    // N P for rows of its own, 0 for rows shared by the chains)
+    tX += (size_t)blockIdx.z * x_stride;
     w += (size_t)blockIdx.z * N;
     if (cv) cv += (size_t)blockIdx.z * N;
     part += (size_t)blockIdx.z * gridDim.y * gridDim.x * (kBalancedDiag ? 1 : 2) * (kGramTile * kGramTile);

@@ -216,6 +216,21 @@ def logit_chains(y, X, n, m0, P0, samp, burn, seed, flags=0):
     return beta
 
 
+def logit_multichain(y, X, n, m0, P0, samp, burn, seed, chains, flags=0):
+    """`chains` independent chains on one data set: y, n [N], X [N x P], shared by all chains.  Chain c is the
+    chain logit_chains runs on `chains` copies of the data with the same seed (so it uses the streams of
+    seed + c), bit for bit, with X held and read once.  Returns beta [chains x samp x P]."""
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    N, P = X.shape
+    y, n, m0 = _f(y).ravel(), _f(n).ravel(), _f(m0).ravel()
+    P0c = np.asfortranarray(_f(P0))
+    beta = np.zeros((max(int(chains), 0), samp, P))
+    st = _lib.lib().bl_logit_multichain(_p(beta), _p(y), _p(X), _p(n), _p(m0), P0c.ctypes.data, int(chains), N, P,
+                                        samp, burn, int(seed), int(flags))
+    _lib.check(st)
+    return beta
+
+
 def mlogit_gibbs(y, X, n, m0, P0, samp, burn, seed, flags=0, keep_w=True):
     """y: N x (J-1) proportions.  Returns (w [samp x (J-1) x N] or None, beta [samp x (J-1) x P])."""
     X = np.ascontiguousarray(X, dtype=np.float64)

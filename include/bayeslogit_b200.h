@@ -241,6 +241,22 @@ int bl_logit_chains_dev(double *beta, const double *y, const double *tX, const d
                         const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
                         int flags, void *stream);
 
+/* Several independent logit chains on ONE data set (the usual 4-8 chains from different seeds that R-hat and
+ * effective-sample-size checks need).  y, n: [N], tX: P x N, shared by all chains, with m0 / P0.  Chain c is
+ * bit for bit the chain bl_logit_chains runs when given `chains` copies of the data and the same seed, so it
+ * uses the streams of seed + c; but X is held once and read once per iteration for all chains.
+ * beta: [chains][samp][P]; omega is not returned.  flags: BL_GIBBS_PLAIN_BETA or 0 (the reference's constrained
+ * draw), optionally BL_GIBBS_UNFUSED.  chains * N < 2^31; P as bl_logit_chains takes it (each chain's beta is drawn
+ * by one CTA out of shared memory: P <= 91 with the constrained draw, P <= 111 with the plain one).  Duplicate rows
+ * are not merged.  One chain runs faster through bl_logit_gibbs (a different, equally valid chain).
+ * Spread the chains over GPUs by giving each rank the whole X and a block of chains, called with
+ * seed + first chain of the block.  The host entry copies X to the device once. */
+int bl_logit_multichain(double *beta, const double *y, const double *tX, const double *n, const double *m0,
+                        const double *P0, int chains, int N, int P, int samp, int burn, uint64_t seed, int flags);
+int bl_logit_multichain_dev(double *beta, const double *y, const double *tX, const double *n, const double *m0,
+                            const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
+                            int flags, void *stream);
+
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */
 int bl_comm_unique_id(void *out128);

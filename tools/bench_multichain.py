@@ -1,0 +1,161 @@
+#!/usr/bin/env python3
+"""Several logit chains on one data set (bl_logit_multichain) against the two ways to get them without it.
+
+    python tools/bench_multichain.py [--N 1000000 --P 64 --chains 1,2,4,8 --iters 20 --reps 3]
+
+For every chain count K and both beta draws, three arms are timed alternately in the same process, on the same
+device-resident data, and reported as ms per iteration of all K chains (median over the repetitions):
+  (a) multichain: bl_logit_multichain_dev, one copy of X shared by the K chains;
+  (b) replicated: bl_logit_chains_dev on K copies of X (the batch entry for chains that own their rows);
+  (c) sequential: K calls of bl_logit_gibbs_dev, one chain after the other.
+(a) and (b) start from the same seed and must give the same beta bit for bit (max_abs_diff_a_b).  The
+BL_GIBBS_TIMING stage split of one iteration of (a) and (b) comes from a separate, untimed call.  X is 512 MB at
+the default size, larger than L2, so every pass reads it from HBM.  Prints one JSON line.
+"""
+import argparse
+import json
+import os
+import re
+import subprocess
+import sys
+import tempfile
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def card():
+    """Name and power limit of the device, read where the numbers are measured."""
+    import torch
+    name = torch.cuda.get_device_name()
+    try:
+        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits",
+                              "-i", str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30)
+        power = float(out.stdout.strip().splitlines()[0]) if out.returncode == 0 else None
+    except (OSError, ValueError, IndexError, subprocess.TimeoutExpired):
+        power = None
+    return name, power
+
+
+def stage_split(fn):
+    """Run fn() with BL_GIBBS_TIMING set and return the stage times (us) the driver prints to stderr."""
+    import torch
+    torch.cuda.synchronize()
+    sys.stderr.flush()
+    saved = os.dup(2)
+    with tempfile.TemporaryFile(mode="w+") as f:
+        os.dup2(f.fileno(), 2)
+        os.environ["BL_GIBBS_TIMING"] = "1"
+        try:
+            fn()
+            torch.cuda.synchronize()
+        finally:
+            del os.environ["BL_GIBBS_TIMING"]
+            os.dup2(saved, 2)
+            os.close(saved)
+        f.seek(0)
+        text = f.read()
+    lines = [l for l in text.splitlines() if "timing, us]" in l]
+    if not lines:
+        return None
+    return {k: float(v) for k, v in re.findall(r"([a-z+]+) ([0-9.]+)", lines[-1].split("]", 1)[1])}
+
+
+def run(N, P, ks, iters, reps):
+    import torch
+    from bayeslogit_b200 import _lib
+    L = _lib.lib()
+    dev = torch.device("cuda")
+    g = torch.Generator(device=dev); g.manual_seed(20240007)
+    X = torch.randn(N, P, generator=g, device=dev, dtype=torch.float64)
+    X[:, P - 1] = 1.0
+    bt = torch.randn(P, generator=g, device=dev, dtype=torch.float64).abs() * 0.25
+    bt[P - 1] = -0.5
+    y = (torch.rand(N, generator=g, device=dev, dtype=torch.float64) < torch.sigmoid(X @ bt)).double()
+    n = torch.ones(N, device=dev, dtype=torch.float64)
+    m0 = torch.zeros(P, device=dev, dtype=torch.float64)
+    P0 = (0.01 * torch.eye(P, device=dev, dtype=torch.float64)).contiguous()
+    st = torch.cuda.current_stream().cuda_stream
+    seed = 20240007
+    row_bytes = (P + 2) * 8                                  # a row of X, its y and its n
+    out = {"N": N, "P": P, "iters": iters, "reps": reps, "results": []}
+
+    for constrained in (True, False):
+        flags = 0 if constrained else 1
+        for K in ks:
+            Xr = X.unsqueeze(0).expand(K, N, P).contiguous()
+            yr = y.unsqueeze(0).expand(K, N).contiguous()
+            nr = n.unsqueeze(0).expand(K, N).contiguous()
+
+            def multichain(k):
+                beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+                _lib.check(L.bl_logit_multichain_dev(beta.data_ptr(), y.data_ptr(), X.data_ptr(), n.data_ptr(),
+                                                     m0.data_ptr(), P0.data_ptr(), K, N, P, k, 0, seed, flags, st))
+                return beta
+
+            def replicated(k):
+                beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+                _lib.check(L.bl_logit_chains_dev(beta.data_ptr(), yr.data_ptr(), Xr.data_ptr(), nr.data_ptr(),
+                                                 m0.data_ptr(), P0.data_ptr(), K, N, P, k, 0, seed, flags, st))
+                return beta
+
+            def sequential(k):
+                beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+                for c in range(K):
+                    _lib.check(L.bl_logit_gibbs_dev(None, beta[c].data_ptr(), y.data_ptr(), X.data_ptr(), n.data_ptr(),
+                                                    m0.data_ptr(), P0.data_ptr(), N, P, k, 0, seed + c, flags | 2, 0, st))
+                return beta
+
+            arms = {"multichain": multichain, "replicated": replicated, "sequential": sequential}
+            for fn in arms.values():                     # warm-up: modules, pools, every kernel of the timed window
+                fn(2)
+            torch.cuda.synchronize()
+            times = {a: [] for a in arms}
+            betas = {}
+            e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            for _ in range(reps):
+                for a, fn in arms.items():               # alternated: drifts of the shared machine hit every arm
+                    e0.record()
+                    betas[a] = fn(iters)
+                    e1.record()
+                    torch.cuda.synchronize()
+                    times[a].append(e0.elapsed_time(e1) / iters)
+            med = {a: sorted(v)[len(v) // 2] for a, v in times.items()}
+            diff = float((betas["multichain"] - betas["replicated"]).abs().max().item())
+            out["results"].append({
+                "beta_draw": "constrained" if constrained else "plain", "chains": K,
+                "ms_per_iteration_of_all_chains": med,
+                "ms_all_reps": times,
+                "multichain_over_replicated": med["multichain"] / med["replicated"],
+                "sequential_over_multichain": med["sequential"] / med["multichain"],
+                "max_abs_diff_a_b": diff,
+                "stages_us": {"multichain": stage_split(lambda: multichain(2)),
+                              "replicated": stage_split(lambda: replicated(2))},
+                "input_bytes_on_device": {"multichain": N * row_bytes, "replicated": K * N * row_bytes,
+                                          "sequential": N * row_bytes},
+            })
+            del Xr, yr, nr
+            torch.cuda.empty_cache()
+    return out
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--N", type=int, default=1_000_000)
+    ap.add_argument("--P", type=int, default=64)
+    ap.add_argument("--chains", default="1,2,4,8")
+    ap.add_argument("--iters", type=int, default=20)
+    ap.add_argument("--reps", type=int, default=3)
+    a = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        sys.exit("bench_multichain: no CUDA device")
+    name, power = card()
+    out = run(a.N, a.P, [int(k) for k in a.chains.split(",")], a.iters, a.reps)
+    out["device"] = name
+    out["power_limit_w"] = power
+    print(json.dumps(out))
+
+
+if __name__ == "__main__":
+    main()
