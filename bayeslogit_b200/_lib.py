@@ -99,6 +99,8 @@ def lib():
     L.bl_logit_chains_dev.argtypes = [vp] * 6 + [ci, i64, ci, ci, ci, u64, ci, vp]
     L.bl_logit_multichain.argtypes = [vp] * 6 + [ci, ci, ci, ci, ci, u64, ci]
     L.bl_logit_multichain_dev.argtypes = [vp] * 6 + [ci, i64, ci, ci, ci, u64, ci, vp]
+    L.bl_mlogit_multichain.argtypes = [vp] * 6 + [ci, ci, ci, ci, ci, ci, u64, ci]
+    L.bl_mlogit_multichain_dev.argtypes = [vp] * 6 + [ci, i64, ci, ci, ci, ci, u64, ci, vp]
     L.bl_comm_unique_id.argtypes = [vp]
     L.bl_comm_init.argtypes = [vp, ci, ci]
     L.bl_comm_init_local.argtypes = [ci, ci]

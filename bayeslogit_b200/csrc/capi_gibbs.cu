@@ -445,6 +445,39 @@ int bl_logit_multichain(double *beta, const double *y, const double *tX, const d
     return 0;
 }
 
+int bl_mlogit_multichain_dev(double *beta, const double *ty, const double *tX, const double *n, const double *m0,
+                             const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
+                             int flags, void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    std::string err;
+    if (mlogit_multichain_device(beta, ty, tX, n, m0, P0, chains, N, P, J, samp, burn, seed, flags, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
+int bl_mlogit_multichain(double *beta, const double *ty, const double *tX, const double *n, const double *m0,
+                         const double *P0, int chains, int N, int P, int J, int samp, int burn, uint64_t seed, int flags)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    std::string err;
+    // checked before any buffer is made: the device driver repeats the checks
+    if (mlogit_multichain_check(chains, N, P, J, samp, burn, flags, err)) return report(err, nullptr);
+    const int U = J - 1;
+    Dev d;
+    double *dy = d.put(ty, (size_t)N * U, err), *dX = d.put(tX, (size_t)N * P, err), *dn = d.put(n, N, err);   // one copy
+    double *dm0 = d.put(m0, (size_t)P * U, err), *dP0 = d.put(P0, (size_t)P * P * U, err);
+    const size_t nb = (size_t)chains * samp * U * P;
+    double *dbeta = d.put(nullptr, nb, err);
+    if (!err.empty()) return report(err, nullptr);
+    if (mlogit_multichain_device(dbeta, dy, dX, dn, dm0, dP0, chains, N, P, J, samp, burn, seed, flags,
+                                 (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * nb, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
 int bl_mlogit_gibbs_dev(double *w, double *beta, const double *ty, const double *tX, const double *n,
                         const double *m0, const double *P0, int64_t N, int P, int J, int samp, int burn,
                         uint64_t seed, int flags, uint64_t obs0, void *stream)

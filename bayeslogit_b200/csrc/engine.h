@@ -90,6 +90,12 @@ int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const dou
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
                         uint64_t seed, int flags, bool shared_rows, cudaStream_t st, std::string &err);
+// Several multinomial logit chains on one data set (ty (J-1) x N, tX P x N, n [N], shared); beta_out: [chains][samp]
+// blocks of P x (J-1).  The check refuses what the driver cannot run, before anything is allocated or launched.
+int mlogit_multichain_check(int chains, int64_t N, int P, int J, int samp, int burn, int flags, std::string &err);
+int mlogit_multichain_device(double *beta_out, const double *ty, const double *tX, const double *n, const double *m0,
+                             const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
+                             int flags, cudaStream_t st, std::string &err);
 int logit_em_device(double *beta, const double *y, const double *tX, const double *n, int64_t N,
                     int P, double tol, int max_iter, int *iters, cudaStream_t st, std::string &err);
 // duplicate-row merge on device-resident data (merge.cu); returns M, -1 (CUDA error), -2 (needs the exact host merge)

@@ -397,8 +397,9 @@ struct DevMem {
 inline int cdiv(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
 // part[chain][slab][P] = per-slab sums of X'(c0 v0 + c1 v1 v2): streaming kernel for power-of-two P,
-// tensor-core kernel for other even P, scalar kernel otherwise.
-void launch_xtv(dim3 grid, cudaStream_t st, double *part, const double *tX, const double *v0, double c0,
+// tensor-core kernel for other even P, scalar kernel otherwise.  Chain c (grid.y) reads its rows at
+// tX + c x_stride and its weights at + c N.
+void launch_xtv(dim3 grid, cudaStream_t st, double *part, const double *tX, int64_t x_stride, const double *v0, double c0,
                 const double *v1, const double *v2, double c1, int64_t N, int P, const double *c1_dev)
 {
     const size_t smem = 8 * P * sizeof(double);
@@ -406,7 +407,7 @@ void launch_xtv(dim3 grid, cudaStream_t st, double *part, const double *tX, cons
     const int64_t slab_pairs = ((N + grid.x - 1) / grid.x) * (P / 2);
     const int l2 = slab_pairs < (1LL << 31) - 4096 ? xtv_stream_log2l(tX, P) : 0;
     const int mode = (v0 && !v1 && !v2) ? 0 : (!v0 && v1 && v2) ? 1 : (v0 && v1 && !v2) ? 2 : -1;
-#define BL_XTV(L2, M) launch_pdl(k_xtv_stream<L2, M>, dim3(grid), dim3(256), smem, st, part, tX, v0, c0, v1, v2, c1, N, c1_dev)
+#define BL_XTV(L2, M) launch_pdl(k_xtv_stream<L2, M>, dim3(grid), dim3(256), smem, st, part, tX, x_stride, v0, c0, v1, v2, c1, N, c1_dev)
 #define BL_XTV_L(L2) (mode == 0 ? BL_XTV(L2, 0) : mode == 1 ? BL_XTV(L2, 1) : BL_XTV(L2, 2))
     if (mode >= 0 && l2 == 2) BL_XTV_L(2);
     else if (mode >= 0 && l2 == 3) BL_XTV_L(3);
@@ -416,8 +417,8 @@ void launch_xtv(dim3 grid, cudaStream_t st, double *part, const double *tX, cons
     else if (mode >= 0 && l2 == 7) BL_XTV_L(7);
 #undef BL_XTV_L
 #undef BL_XTV
-    else if (xbeta_mma_ok(tX, P)) launch_pdl(k_xtv_mma, dim3(grid), dim3(256), smem, st, part, tX, v0, c0, v1, v2, c1, N, P, c1_dev);
-    else launch_pdl(k_xtv_partial, dim3(grid), dim3(256), smem, st, part, tX, v0, c0, v1, v2, c1, N, P, c1_dev);
+    else if (xbeta_mma_ok(tX, P)) launch_pdl(k_xtv_mma, dim3(grid), dim3(256), smem, st, part, tX, x_stride, v0, c0, v1, v2, c1, N, P, c1_dev);
+    else launch_pdl(k_xtv_partial, dim3(grid), dim3(256), smem, st, part, tX, x_stride, v0, c0, v1, v2, c1, N, P, c1_dev);
 }
 
 // BL_GIBBS_TIMING=1: CUDA-event stage times of one iteration (the one armed by the driver), to stderr.
@@ -451,6 +452,32 @@ struct StageTimer {
     }
 };
 
+// Gram and X'v slab partition of N rows: one wave of 2 CTAs per SM (Sweep::init; the multinomial multichain
+// driver takes the single chain's partition so that every chain sums its rows in the single chain's order).
+struct Slabs {
+    int nt = 1, nslab = 1, nslab_diag = 0, xtv_slabs = 1;
+};
+
+Slabs slab_partition(int64_t N, int P)
+{
+    Slabs g;
+    g.nt = cdiv(P, kGramTile);
+    const int tiles = g.nt * (g.nt + 1) / 2;
+    g.nslab = (int)std::min<int64_t>(std::max<int64_t>(1, 148 * 2 / tiles), std::max<int64_t>(1, N / (4 * kGramRows)));   // 2 CTAs/SM resident: one wave
+    if (g.nslab < 1) g.nslab = 1;
+    if (g.nt > 1) {
+        // one wave of 2 CTAs per SM, slabs in proportion to the tile's cost (diagonal 36, off-diagonal 64
+        // MMA tiles per k-step): P = 256 -> 4 x 20 + 6 x 35 CTAs instead of 10 x 29 of unequal length
+        const int nd = g.nt, no = g.nt * (g.nt - 1) / 2, total = nd * 36 + no * 64;
+        const int64_t cap = std::max<int64_t>(1, N / (4 * kGramRows));
+        g.nslab = (int)std::min<int64_t>(std::max(1, 148 * 2 * 64 / total), cap);
+        g.nslab_diag = (int)std::min<int64_t>(std::max(1, 148 * 2 * 36 / total), cap);
+        if (g.nslab_diag > g.nslab) g.nslab_diag = g.nslab;
+    }
+    g.xtv_slabs = (int)std::min<int64_t>(148 * 2, std::max<int64_t>(1, N / 64));
+    return g;
+}
+
 // Shared machinery of the three sweeps.
 struct Sweep {
     int64_t N = 0;          // local observations
@@ -472,20 +499,9 @@ struct Sweep {
     {
         // the beta draws keep a vector in registers, 8 entries per lane of one warp (gibbs_beta.cuh)
         if (P > 256) { err = "P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
-        nt = cdiv(P, kGramTile);
+        const Slabs g = slab_partition(N, P);
+        nt = g.nt; nslab = g.nslab; nslab_diag = g.nslab_diag; xtv_slabs = g.xtv_slabs;
         int tiles = nt * (nt + 1) / 2;
-        nslab = (int)std::min<int64_t>(std::max<int64_t>(1, 148 * 2 / tiles), std::max<int64_t>(1, N / (4 * kGramRows)));   // 2 CTAs/SM resident: one wave
-        if (nslab < 1) nslab = 1;
-        if (nt > 1) {
-            // one wave of 2 CTAs per SM, slabs in proportion to the tile's cost (diagonal 36, off-diagonal 64
-            // MMA tiles per k-step): P = 256 -> 4 x 20 + 6 x 35 CTAs instead of 10 x 29 of unequal length
-            const int nd = nt, no = nt * (nt - 1) / 2, total = nd * 36 + no * 64;
-            const int64_t cap = std::max<int64_t>(1, N / (4 * kGramRows));
-            nslab = (int)std::min<int64_t>(std::max(1, 148 * 2 * 64 / total), cap);
-            nslab_diag = (int)std::min<int64_t>(std::max(1, 148 * 2 * 36 / total), cap);
-            if (nslab_diag > nslab) nslab_diag = nslab;
-        }
-        xtv_slabs = (int)std::min<int64_t>(148 * 2, std::max<int64_t>(1, N / 64));
         GB_CK(m.get(&psi, N));
         GB_CK(m.get(&w, N));
         GB_CK(m.get(&acc, (size_t)P * P + P));
@@ -518,7 +534,7 @@ struct Sweep {
     {
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));
         if (xbeta_mma_ok(tX, P))
-            launch_pdl(k_xbeta_mma<false>, dim3(grid), dim3(256), 0, st, out, tX, N * P, beta, 0, 1, N, P, off, off_scale, shift, MlogitNext{});
+            launch_pdl(k_xbeta_mma<false>, dim3(grid), dim3(256), 0, st, out, N, tX, N * P, beta, 0, 1, N, P, off, off_scale, shift, MlogitNext{});
         else
             k_xbeta<<<grid, 256, P * sizeof(double), st>>>(out, tX, beta, off, off_scale, shift, N, P);
         count_launch();
@@ -528,7 +544,7 @@ struct Sweep {
     void xbeta_mlogit(double *out, const double *beta, const MlogitNext &mn)
     {
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));
-        launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, out, tX, N * P, beta, 0, 1, N, P, nullptr, 0.0, 0.0, mn);
+        launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, out, N, tX, N * P, beta, 0, 1, N, P, nullptr, 0.0, 0.0, mn);
         count_launch();
     }
 
@@ -565,8 +581,9 @@ struct Sweep {
     void xtv(const double *v0, double c0, const double *v1, const double *v2, double c1,
              const double *c1_dev = nullptr)
     {
-        launch_xtv(dim3(xtv_slabs), st, xtv_part, tX, v0, c0, v1, v2, c1, N, P, c1_dev);
-        launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128)), dim3(128), 0, st, acc + (size_t)P * P, nullptr, nullptr, xtv_part, P, xtv_slabs);
+        launch_xtv(dim3(xtv_slabs), st, xtv_part, tX, N * P, v0, c0, v1, v2, c1, N, P, c1_dev);
+        launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128)), dim3(128), 0, st, acc + (size_t)P * P, nullptr, nullptr, xtv_part, P, xtv_slabs,
+                   (int64_t)P);
         count_launch(2);
     }
 
@@ -675,7 +692,7 @@ int logit_gibbs_device(double *w_out, double *beta_out, const double *y, const d
     count_launch(3);
     s.xtv(kappa, 1.0, nullptr, nullptr, 0.0);
     if (sharded && small_allreduce(s.acc + (size_t)P * P, (size_t)P, kOpSumF64, s.status, st, err)) return 1;
-    k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(bP, b0, s.acc + (size_t)P * P, s.xtv_part, P, 0);
+    k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(bP, b0, s.acc + (size_t)P * P, s.xtv_part, P, 0, P);
     count_launch();
 
     GB_CK(cudaMemsetAsync(beta_out, 0, sizeof(double) * (size_t)P * samp, st));
@@ -813,8 +830,8 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
     k_kappa<<<cdiv(R, 256), 256, 0, st>>>(kappa, y, n, 0.0, R);
     k_shape_int<<<cdiv(R, 256), 256, 0, st>>>(shape, n, R);
     k_matvec<<<cdiv(P, 128), 128, 0, st>>>(b0, P0, m0, P);
-    launch_xtv(dim3(1, xchains), st, xtv_part, tX, kappa, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
-    k_xtv_reduce<<<dim3(cdiv(P, 128), xchains), 128, 0, st>>>(bP, b0, nullptr, xtv_part, P, 1);
+    launch_xtv(dim3(1, xchains), st, xtv_part, tX, N * P, kappa, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
+    k_xtv_reduce<<<dim3(cdiv(P, 128), xchains), 128, 0, st>>>(bP, b0, nullptr, xtv_part, P, 1, P);
     count_launch(5);
     for (int c = xchains; c < chains; ++c)
         GB_CK(cudaMemcpyAsync(bP + (size_t)c * P, bP, sizeof(double) * P, cudaMemcpyDeviceToDevice, st));
@@ -826,9 +843,9 @@ int logit_chains_device(double *beta_out, const double *y, const double *tX, con
         const int64_t trips = (int64_t)chains * ((N + 31) / 32);
         int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (trips + 7) / 8));
         if (xbeta_mma_ok(tX, P))
-            k_xbeta_mma<false><<<grid, 256, 0, st>>>(psi, tX, x_stride, beta, bstride, chains, N, P, nullptr, 0.0, 0.0, MlogitNext{});
+            k_xbeta_mma<false><<<grid, 256, 0, st>>>(psi, N, tX, x_stride, beta, bstride, chains, N, P, nullptr, 0.0, 0.0, MlogitNext{});
         else
-            k_xbeta_chains<<<grid, 256, 0, st>>>(psi, tX, x_stride, beta, bstride, chains, (int)N, P);
+            k_xbeta_chains<<<grid, 256, 0, st>>>(psi, N, tX, x_stride, beta, bstride, chains, (int)N, P);
         count_launch();
     };
     const bool timing = getenv("BL_GIBBS_TIMING") != nullptr;
@@ -939,7 +956,7 @@ int mlogit_gibbs_device(double *w_out, double *beta_out, const double *ty, const
         count_launch(2);
         s.xtv(cj, 1.0, nullptr, nullptr, 0.0);
         if (sharded && small_allreduce(s.acc + (size_t)P * P, (size_t)P, kOpSumF64, s.status, st, err)) return 1;
-        k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(base + (size_t)P * j, b0 + (size_t)P * j, s.acc + (size_t)P * P, s.xtv_part, P, 0);
+        k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(base + (size_t)P * j, b0 + (size_t)P * j, s.acc + (size_t)P * P, s.xtv_part, P, 0, P);
         count_launch();
     }
     GB_CK(cudaMemsetAsync(beta_out, 0, sizeof(double) * (size_t)P * U * samp, st));
@@ -994,6 +1011,194 @@ int mlogit_gibbs_device(double *w_out, double *beta_out, const double *ty, const
     }
     GB_CK(cudaGetLastError());
     return s.check_status(err, "mult_gibbs");
+}
+
+// ------------------------------------------------------------------------------------
+// Several multinomial logit chains on ONE data set (bl_mlogit_multichain): chain c is, bit for bit, the chain
+// mlogit_gibbs_device runs with seed + c and omega dropped (BL_GIBBS_UNFUSED: the one it runs with
+// BL_MLOGIT_UNFUSED set).  Every category update is one launch per kernel for all chains:
+//   psi   : XB_j of all chains from one pass over X (k_mlogit_psi_shared: 8 chains' beta_j in the 8 B columns
+//           of the MMAs), which also forms E_j, the next category's offsets and the next draw's class-ordered
+//           index list over all chains * N (chain, row) pairs.  Unfused: the single chain's psi kernel with an X
+//           stride of 0, then k_mlogit_offsets, both with a chain dimension.
+//   draw  : one refill over chains * N draws, stream of (chain, row) = (seed + c, row, t U + j).
+//   sums  : the single chain's slab partition and kernels with a chain grid dimension (X stride 0).
+//   beta  : one CTA per chain, the single chain's k_beta_draw instantiation out of shared memory; base_j =
+//           P0_j m0_j + X' kappa_j is formed once and copied to every chain.
+// The launches of an iteration do not depend on the number of chains.  beta_out: [chains][samp] blocks of P x U.
+// ------------------------------------------------------------------------------------
+// shared memory of one chain's mvn beta draw (A, B, 5 P of vectors; P <= 64: the layout of cta_plain_fast)
+static size_t mlogit_multichain_beta_smem(int P)
+{
+    return std::max((2 * (size_t)(P | 1) * P + 5 * (size_t)P) * sizeof(double),
+                    P <= 64 ? (beta_fast_e_offset(P) + 64) * sizeof(double) : (size_t)0);
+}
+
+int mlogit_multichain_check(int chains, int64_t N, int P, int J, int samp, int burn, int flags, std::string &err)
+{
+    if (chains <= 0 || N <= 0 || P <= 0 || J < 2 || samp <= 0 || burn < 0) { err = "mlogit_multichain: bad dimensions"; return 1; }
+    if (flags & ~BL_GIBBS_UNFUSED) { err = "mlogit_multichain: unsupported flags (only BL_GIBBS_UNFUSED is accepted)"; return 1; }
+    if ((int64_t)chains * N >= (1LL << 31)) { err = "mlogit_multichain: chains * N must stay below 2^31 observations per call"; return 1; }
+    // each chain's mvn draw runs in one CTA out of shared memory: P <= 111
+    if (P > 256 || mlogit_multichain_beta_smem(P) > 200 * 1024) { err = "mlogit_multichain: P too large for the shared-memory beta draw"; return 1; }
+    return 0;
+}
+
+int mlogit_multichain_device(double *beta_out, const double *ty, const double *tX, const double *n, const double *m0,
+                             const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
+                             int flags, cudaStream_t st, std::string &err)
+{
+    if (mlogit_multichain_check(chains, N, P, J, samp, burn, flags, err)) return 1;
+    const int U = J - 1, K = chains;
+    const int64_t T = (int64_t)K * N, UN = (int64_t)U * N;
+    const size_t beta_smem = mlogit_multichain_beta_smem(P);
+    const Slabs g = slab_partition(N, P);
+    const int nt = g.nt, tiles = nt * (nt + 1) / 2, slabs_total = nt > 1 ? 2 * g.nslab : g.nslab;
+    const bool packed = gram_packed(P);                 // P = 32: X'(Omega c_j) comes out of the Gram pass
+    const size_t accn = (size_t)P * P + P;
+    const bool fuse_next = !(flags & BL_GIBBS_UNFUSED) && xbeta_mma_ok(tX, P) && U <= kMlogitMaxU;
+    const bool prebin = fuse_next && devroye_binned(T, 1 << 18);
+    DevMem mem;
+    mem.st = st;
+    double *XB, *EX = nullptr, *cj, *eta, *w, *acc, *part, *xtv_part, *b0, *base, *yj;
+    int *shape, *status;
+    void *work;
+    GB_CK(mem.get(&XB, (size_t)K * UN));
+    if (fuse_next) GB_CK(mem.get(&EX, (size_t)K * UN));
+    GB_CK(mem.get(&cj, T));
+    GB_CK(mem.get(&eta, T));
+    GB_CK(mem.get(&w, T));
+    GB_CK(mem.get(&shape, T));                          // the refill reads one shape per (chain, row)
+    GB_CK(mem.get(&acc, accn * K));
+    GB_CK(mem.get(&part, (size_t)K * tiles * g.nslab * 2 * kGramTile * kGramTile));
+    GB_CK(mem.get(&xtv_part, (size_t)K * g.xtv_slabs * P));
+    GB_CK(mem.get(&b0, (size_t)P * U));
+    GB_CK(mem.get(&base, (size_t)U * K * P));           // [U][K][P]: k_beta_draw reads chain c's rhs at + c P
+    GB_CK(mem.get(&yj, N));
+    GB_CK(mem.get(&status, 1));
+    GB_CK(mem.get((char **)&work, (32 + (size_t)T) * sizeof(int)));      // branch-class binning: [meta][index list]
+    GB_CK(cudaMemsetAsync(status, 0, sizeof(int), st));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRows, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(true)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false, true)));
+    const bool lean = P <= 64 && !kSlowBeta;            // the single chain's mvn draw instantiation
+    if (beta_smem > 48 * 1024)
+        GB_CK(cudaFuncSetAttribute(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)beta_smem));
+    const int64_t bstride = (int64_t)P * U * samp;      // chain stride of beta_out
+
+    k_shape_int<<<cdiv(N, 256), 256, 0, st>>>(shape, n, N);
+    count_launch();
+    for (int64_t r = N; r < T; r += N)
+        GB_CK(cudaMemcpyAsync(shape + r, shape, sizeof(int) * N, cudaMemcpyDeviceToDevice, st));
+    // base_j = b0_j + X'(n (y_j - 1/2)), b0_j = P0_j m0_j, as the single chain forms it (MultLogit.hpp:214-219, :271-273)
+    for (int j = 0; j < U; ++j) {
+        GB_CK(cudaMemcpy2DAsync(yj, sizeof(double), ty + j, sizeof(double) * U, sizeof(double), N,
+                                cudaMemcpyDeviceToDevice, st));
+        k_kappa<<<cdiv(N, 256), 256, 0, st>>>(cj, yj, n, 0.0, N);
+        k_matvec<<<cdiv(P, 128), 128, 0, st>>>(b0 + (size_t)P * j, P0 + (size_t)P * P * j, m0 + (size_t)P * j, P);
+        launch_xtv(dim3(g.xtv_slabs), st, xtv_part, tX, N * P, cj, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
+        launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128)), dim3(128), 0, st, acc + (size_t)P * P, nullptr, nullptr, xtv_part, P,
+                   g.xtv_slabs, (int64_t)P);
+        double *bj = base + (size_t)K * P * j;
+        k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(bj, b0 + (size_t)P * j, acc + (size_t)P * P, xtv_part, P, 0, P);
+        count_launch(5);
+        for (int c = 1; c < K; ++c)
+            GB_CK(cudaMemcpyAsync(bj + (size_t)P * c, bj, sizeof(double) * P, cudaMemcpyDeviceToDevice, st));
+    }
+    GB_CK(cudaMemsetAsync(beta_out, 0, sizeof(double) * (size_t)bstride * K, st));
+    GB_CK(cudaMemsetAsync(XB, 0, sizeof(double) * (size_t)K * UN, st));
+    if (fuse_next) {
+        k_fill<<<(int)std::min<int64_t>(148 * 8, cdiv((int64_t)K * UN, 256)), 256, 0, st>>>(EX, 1.0, (int64_t)K * UN);   // exp(0)
+        count_launch();
+    }
+    static const int tn_flags = getenv("BL_BETA_NO_SPEC") ? 3 : 1;
+    const int total = burn + samp;
+    StageTimer tmr;
+    tmr.st = st;
+    for (int t = 0; t < total; ++t) {
+        const int slice = t <= burn ? 0 : t - burn;
+        double *bS = beta_out + (size_t)P * U * slice;
+        for (int j = 0; j < U; ++j) {
+            const uint32_t call = (uint32_t)t * (uint32_t)U + (uint32_t)j;
+            const bool first = t == 0 && j == 0;
+            tmr.arm(t == total - 1 && j == U - 1);
+            if (!fuse_next || first) {
+                k_mlogit_offsets<<<dim3(cdiv(N, 256), K), 256, 0, st>>>(cj, eta, XB, N, U, j);
+                count_launch();
+            }
+            tmr.mark("offsets");
+            cudaError_t e = launch_devroye_refill(w, shape, eta, T, StreamId{seed, 0, call, (uint32_t)N}, st, work, 1 << 18,
+                                                  prebin && !first);
+            if (e != cudaSuccess) { err = cudaGetErrorString(e); return 1; }
+            tmr.mark("draw");
+            if (!packed) {
+                // X'(Omega c_j) of every chain into the tail of its sums
+                launch_xtv(dim3(g.xtv_slabs, K), st, xtv_part, tX, 0, nullptr, 0.0, w, cj, 1.0, N, P, nullptr);
+                launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128), K), dim3(128), 0, st, acc + (size_t)P * P, nullptr, nullptr,
+                           xtv_part, P, g.xtv_slabs, (int64_t)accn);
+                count_launch(2);
+                tmr.mark("xtv");
+            }
+            if (nt > 1)
+                launch_pdl(k_gram_partial<kGramRows, false>, dim3(g.nslab, tiles, K), dim3(256), gram_smem_bytes(true), st,
+                           part, tX, (int64_t)0, w, N, P, nt, g.nslab_diag, nullptr);
+            else if (packed)
+                launch_pdl(k_gram_partial<kGramRowsDiag, true, true>, dim3(g.nslab, tiles, K), dim3(256),
+                           gram_smem_bytes(false, true), st, part, tX, (int64_t)0, w, N, P, nt, 0, cj);
+            else
+                launch_pdl(k_gram_partial<kGramRowsDiag, true>, dim3(g.nslab, tiles, K), dim3(256), gram_smem_bytes(false),
+                           st, part, tX, (int64_t)0, w, N, P, nt, 0, nullptr);
+            launch_pdl(k_gram_reduce, dim3(cdiv((int64_t)P * P + (packed ? P : 0), 32), K), dim3(256), 0, st, acc, nullptr,
+                       part, P, nt, slabs_total, PeerPush{}, packed ? 1 : 0, 2 * g.nslab_diag, packed ? 1 : 0);
+            count_launch(2);
+            tmr.mark("gram");
+            launch_pdl(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>, dim3(K), dim3(256), beta_smem, st,
+                       (int)kBetaMvn, (const double *)acc, P0 + (size_t)P * P * j, (const double *)(base + (size_t)K * P * j),
+                       1, (const double *)nullptr, bS + (size_t)P * j, (double *)nullptr, P, seed, call, status, PeerWait{},
+                       bstride, (const double *)nullptr, tn_flags);
+            count_launch();
+            tmr.mark("beta");
+            const double *bj = bS + (size_t)P * j;
+            if (fuse_next) {
+                // the next draw's class-ordered index list comes out of the same pass (cursors zeroed first)
+                int *bm = prebin ? (int *)work : nullptr;
+                if (prebin) GB_CK(cudaMemsetAsync(bm, 0, 32 * sizeof(int), st));
+                const MlogitNext mn{EX, XB, cj, eta, U, j, (j + 1) % U, bm, bm ? bm + 32 : nullptr};
+                if (K == 1) {
+                    // one chain: the single chain's kernel (no trip through shared memory)
+                    const int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));
+                    launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, XB + (size_t)N * j, N, tX, N * P, bj,
+                               (int64_t)0, 1, N, P, nullptr, 0.0, 0.0, mn);
+                } else {
+                    const int64_t items = (N + 31) / 32 * ((K + kMlogitGroup - 1) / kMlogitGroup);
+                    const int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (items + 7) / 8));
+                    launch_pdl(k_mlogit_psi_shared, dim3(grid), dim3(256), 0, st, XB, tX, bj, bstride, K, N, P, mn);
+                }
+            } else {
+                // XB_j of chain c at XB + c U N + j N: the single chain's psi kernel, rows shared (X stride 0)
+                const int64_t trips = (int64_t)K * ((N + 31) / 32);
+                const int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (trips + 7) / 8));
+                if (xbeta_mma_ok(tX, P))
+                    launch_pdl(k_xbeta_mma<false>, dim3(grid), dim3(256), 0, st, XB + (size_t)N * j, UN, tX, (int64_t)0, bj,
+                               bstride, K, N, P, nullptr, 0.0, 0.0, MlogitNext{});
+                else
+                    k_xbeta_chains<<<grid, 256, 0, st>>>(XB + (size_t)N * j, UN, tX, 0, bj, bstride, K, (int)N, P);
+            }
+            count_launch();
+            tmr.mark("xbeta");
+            tmr.report("mlogit multichain");
+        }
+    }
+    GB_CK(cudaGetLastError());
+    int h = 0;
+    GB_CK(cudaMemcpyAsync(&h, status, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (h != 0) { err = "mlogit_multichain: a chain's posterior precision is not positive definite"; return 1; }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------
@@ -1208,7 +1413,7 @@ int logit_em_device(double *beta, const double *y, const double *tX, const doubl
     k_kappa<<<cdiv(N, 256), 256, 0, st>>>(kappa, y, n, 0.0, N);
     count_launch();
     s.xtv(kappa, 1.0, nullptr, nullptr, 0.0);                       // bP = X' kappa (default prior b0 = 0)
-    k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(bP, s.acc + (size_t)P * P, nullptr, s.xtv_part, P, 0);
+    k_xtv_reduce<<<cdiv(P, 128), 128, 0, st>>>(bP, s.acc + (size_t)P * P, nullptr, s.xtv_part, P, 0, P);
     count_launch();
     GB_CK(cudaMemsetAsync(beta, 0, sizeof(double) * P, st));
     size_t smem = ((size_t)(P | 1) * P + P) * sizeof(double);

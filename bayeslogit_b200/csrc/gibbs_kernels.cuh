@@ -76,11 +76,12 @@ k_xbeta(double *__restrict__ psi, const double *__restrict__ tX, const double *_
 }
 
 // The same for a batch of independent chains: chain c reads the N rows at tX + c * x_stride (N P: its own
-// rows; 0: rows shared by all chains), meets beta_c = beta[c * beta_stride ..) and writes psi[c N ..).
+// rows; 0: rows shared by all chains), meets beta_c = beta[c * beta_stride ..) and writes psi[c psi_stride ..)
+// (N: chains side by side; U N: category j of a multinomial chain's [U][N] linear predictors).
 // Trips of 32 rows never straddle two chains.
 static __global__ void __launch_bounds__(256, 2)
-k_xbeta_chains(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ beta,
-               int64_t beta_stride, int chains, int N, int P)
+k_xbeta_chains(double *__restrict__ psi, int64_t psi_stride, const double *__restrict__ tX, int64_t x_stride,
+               const double *__restrict__ beta, int64_t beta_stride, int chains, int N, int P)
 {
     const int lane = threadIdx.x & 31;
     const int tpc = (N + 31) >> 5;                                   // trips per chain
@@ -118,7 +119,7 @@ k_xbeta_chains(double *__restrict__ psi, const double *__restrict__ tX, int64_t 
                 acc[k] = keep + __shfl_xor_sync(0xffffffffu, send, o);
             }
         }
-        if (i0 + lane < N) psi[(size_t)ch * N + i0 + lane] = acc[0];
+        if (i0 + lane < N) psi[ch * psi_stride + i0 + lane] = acc[0];
     }
 }
 
@@ -180,7 +181,8 @@ __device__ __forceinline__ void dmma884(double &c0, double &c1, double a, double
 // of the 8 rows.  No cross-lane reduction and two accumulator registers per 8 rows, so a warp
 // keeps a whole 32-row trip of loads in flight; the lane-strided k_xbeta spends ~150 of its ~220
 // instructions per trip in the transposing butterfly and idles HBM meanwhile (4.6 TB/s at P = 64,
-// 2.4 TB/s at P = 32).  Chains: the N rows at tX + c * x_stride meet beta + c * beta_stride, psi goes to [c N ..).
+// 2.4 TB/s at P = 32).  Chains: the N rows at tX + c * x_stride meet beta + c * beta_stride, psi goes to
+// [c psi_stride ..) (off is read at [c N ..)).
 // ---------------------------------------------------------------------------------
 // mlogit epilogue (MultLogit.hpp:246-258, 275-277): the category whose coefficients were just drawn gets its new
 // linear predictor XB_j = X beta_j and E_j = exp(XB_j) (cached so that no category's exponentials are recomputed
@@ -198,10 +200,60 @@ struct MlogitNext {
                                // shared cursors' atomics per 32 rows instead of a pass over eta
 };
 
+// The loads of the epilogue that do not depend on the new product: row i's exponentials of the categories other
+// than j and jn, and XB_jn (zero for rows past N).
+__device__ __forceinline__ void mlogit_next_load(double (&ek)[kMlogitMaxU], double &xbn, const MlogitNext &mn,
+                                                 int64_t i, int64_t N)
+{
+#pragma unroll
+    for (int k = 0; k < kMlogitMaxU; ++k)
+        ek[k] = (k < mn.U && k != mn.j && k != mn.jn && i < N) ? __ldcg(mn.E + i + (size_t)N * k) : 0.0;
+    xbn = 0.0;
+    if (mn.jn != mn.j && i < N) xbn = __ldcg(mn.XB + i + (size_t)N * mn.jn);
+}
+
+// The epilogue of one row per lane, called by the whole warp: row i (< N) gets XB_j = xb (at psi[i]), E_j = exp(xb),
+// the next category's offset c and tilt eta; with mn.bin_idx the warp's rows then enter the next draw's class-ordered
+// index list of `total` entries as the values gi (class 0 from the front, class 1 from the back, one atomic per class).
+__device__ __forceinline__ void mlogit_next_epilogue(double *psi, const MlogitNext &mn, double xb,
+                                                     const double (&ek)[kMlogitMaxU], double xbn, int64_t i, int64_t N,
+                                                     int gi, int total, int lane)
+{
+    int cls = -1;
+    if (i < N) {
+        psi[i] = xb;
+        const double ej = exp(xb);
+        mn.E[i + (size_t)N * mn.j] = ej;
+        double A = 0.0;
+#pragma unroll
+        for (int k = 0; k < kMlogitMaxU; ++k)
+            if (k < mn.U && k != mn.jn) A += k == mn.j ? ej : ek[k];
+        A += 1.0;
+        const double cj = log(A);
+        mn.c[i] = cj;
+        const double et = (mn.jn == mn.j ? xb : xbn) - cj;
+        mn.eta[i] = et;
+        if (mn.bin_idx) cls = fabs(et) * 0.5 >= 1.0 / 0.64 ? 1 : 0;        // dev_class (pg_devroye_kernel.cu), kTrunc = 0.64
+    }
+    if (mn.bin_idx) {
+        const unsigned m1 = __ballot_sync(0xffffffffu, cls == 1), m0 = __ballot_sync(0xffffffffu, cls == 0);
+        int b0 = 0, b1 = 0;
+        if (lane == 0) {
+            if (m0) b0 = atomicAdd(&mn.bin_meta[1], __popc(m0));
+            if (m1) b1 = atomicAdd(&mn.bin_meta[2], __popc(m1));
+        }
+        b0 = __shfl_sync(0xffffffffu, b0, 0);
+        b1 = __shfl_sync(0xffffffffu, b1, 0);
+        const unsigned lt = (1u << lane) - 1u;
+        if (cls == 0) mn.bin_idx[b0 + __popc(m0 & lt)] = gi;
+        else if (cls == 1) mn.bin_idx[total - 1 - (b1 + __popc(m1 & lt))] = gi;
+    }
+}
+
 template <bool kMlogit>
 static __global__ void __launch_bounds__(256, 2)
-k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ beta,
-            int64_t beta_stride, int chains, int64_t N, int P,
+k_xbeta_mma(double *__restrict__ psi, int64_t psi_stride, const double *__restrict__ tX, int64_t x_stride,
+            const double *__restrict__ beta, int64_t beta_stride, int chains, int64_t N, int P,
             const double *__restrict__ off, double off_scale, double shift, MlogitNext mn)
 {
     BL_PDL_ENTER();
@@ -221,14 +273,8 @@ k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_s
         for (int rb = 0; rb < 4; ++rb) rv[rb] = i0 + 8 * rb + gid < N;
         // mlogit: this lane's row is 8 tig + gid; the other categories' exponentials and the next category's
         // linear predictor do not depend on this trip's product -- their loads go out with the first loads of X
-        double ek[kMlogit ? kMlogitMaxU : 1], xbn = 0.0;
-        if (kMlogit) {
-            const int64_t i = i0 + 8 * tig + gid;
-#pragma unroll
-            for (int k = 0; k < kMlogitMaxU; ++k)
-                ek[k] = (k < mn.U && k != mn.j && k != mn.jn && i < N) ? __ldcg(mn.E + i + (size_t)N * k) : 0.0;
-            if (mn.jn != mn.j && i < N) xbn = __ldcg(mn.XB + i + (size_t)N * mn.jn);
-        }
+        double ek[kMlogitMaxU], xbn = 0.0;
+        if (kMlogit) mlogit_next_load(ek, xbn, mn, i0 + 8 * tig + gid, N);
 #pragma unroll 4
         for (int c0 = 0; c0 < P; c0 += 8) {
             const bool cv = c0 + 2 * tig < P;
@@ -248,43 +294,13 @@ k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_s
             // every column of an accumulator tile holds psi of its 8 rows: lane (gid, tig) takes row 8 tig + gid
             const double xb = tig == 0 ? c[0][0] : tig == 1 ? c[1][0] : tig == 2 ? c[2][0] : c[3][0];
             const int64_t i = i0 + 8 * tig + gid;
-            int cls = -1;
-            if (i < N) {
-                psi[i] = xb;
-                const double ej = exp(xb);
-                mn.E[i + (size_t)N * mn.j] = ej;
-                double A = 0.0;
-#pragma unroll
-                for (int k = 0; k < kMlogitMaxU; ++k)
-                    if (k < mn.U && k != mn.jn) A += k == mn.j ? ej : ek[k];
-                A += 1.0;
-                const double cj = log(A);
-                mn.c[i] = cj;
-                const double et = (mn.jn == mn.j ? xb : xbn) - cj;
-                mn.eta[i] = et;
-                if (mn.bin_idx) cls = fabs(et) * 0.5 >= 1.0 / 0.64 ? 1 : 0;        // dev_class (pg_devroye_kernel.cu), kTrunc = 0.64
-            }
-            if (mn.bin_idx) {
-                // class 0 from the front, class 1 from the back, a warp's rows in one atomic per class
-                const unsigned m1 = __ballot_sync(0xffffffffu, cls == 1), m0 = __ballot_sync(0xffffffffu, cls == 0);
-                int b0 = 0, b1 = 0;
-                if (lane == 0) {
-                    if (m0) b0 = atomicAdd(&mn.bin_meta[1], __popc(m0));
-                    if (m1) b1 = atomicAdd(&mn.bin_meta[2], __popc(m1));
-                }
-                b0 = __shfl_sync(0xffffffffu, b0, 0);
-                b1 = __shfl_sync(0xffffffffu, b1, 0);
-                const unsigned lt = (1u << lane) - 1u;
-                if (cls == 0) mn.bin_idx[b0 + __popc(m0 & lt)] = (int)i;
-                else if (cls == 1) mn.bin_idx[(int)N - 1 - (b1 + __popc(m1 & lt))] = (int)i;
-            }
+            mlogit_next_epilogue(psi, mn, xb, ek, xbn, i, N, (int)i, (int)N, lane);
         } else if (tig == 0) {
 #pragma unroll
             for (int rb = 0; rb < 4; ++rb) {
                 const int64_t i = i0 + 8 * rb + gid;
                 if (i < N) {
-                    const int64_t g = ch * N + i;
-                    psi[g] = (off ? c[rb][0] + off_scale * off[g] : c[rb][0]) + shift;
+                    psi[ch * psi_stride + i] = (off ? c[rb][0] + off_scale * off[ch * N + i] : c[rb][0]) + shift;
                 }
             }
         }
@@ -292,6 +308,90 @@ k_xbeta_mma(double *__restrict__ psi, const double *__restrict__ tX, int64_t x_s
 }
 
 inline bool xbeta_mma_ok(const double *tX, int P) { return P % 2 == 0 && (reinterpret_cast<uintptr_t>(tX) & 15) == 0; }
+
+// ---------------------------------------------------------------------------------
+// k_xbeta_mma<true> for `chains` multinomial chains on ONE set of rows (bl_mlogit_multichain).  The chains multiply
+// the same X by their own beta_j, so the B operand that k_xbeta_mma fills with one beta in all 8 columns carries the
+// beta_j of 8 chains instead -- lane (gid, tig) feeds B[tig][gid] = beta_j of chain g0 + gid -- and one read of X
+// gives column k of every accumulator tile = XB_j of chain g0 + k (the MMA forms each output element from its own
+// row and column only: the bits of the single chain's XB_j).  More than 8 chains: further passes over the trip's
+// rows, 8 chains each, on neighbouring warps.
+//   hand-over: the warp's 32 x 8 tile goes through shared memory; lane l then runs row i0 + l's epilogue
+//           (mlogit_next_epilogue, the single chain's arithmetic) for each chain of the group in turn.
+//   state : chain c's XB and E at [c][U][N] (XB is also where XB_j is written), its c and eta at mn.c / mn.eta +
+//           c N.  The next draw's index list (optional) holds all chains * N (chain, row) pairs as c N + i.
+// ---------------------------------------------------------------------------------
+constexpr int kMlogitGroup = 8;                  // chains per pass: the 8 columns of an m8n8k4 tile
+constexpr int kMlogitTileLd = kMlogitGroup + 1;  // odd row stride: lane l reading row l is conflict-free
+
+static __global__ void __launch_bounds__(256, 2)
+k_mlogit_psi_shared(double *XB, const double *__restrict__ tX, const double *__restrict__ beta,
+                    int64_t beta_stride, int chains, int64_t N, int P, MlogitNext mn)
+{
+    BL_PDL_ENTER();
+    __shared__ double tile[8][32 * kMlogitTileLd];
+    const int lane = threadIdx.x & 31, gid = lane >> 2, tig = lane & 3;
+    double *pt = tile[threadIdx.x >> 5];
+    const int groups = (chains + kMlogitGroup - 1) / kMlogitGroup;
+    const int64_t UN = (int64_t)mn.U * N;
+    const int64_t items = ((N + 31) >> 5) * groups;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const int64_t wid = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    for (int64_t item = wid; item < items; item += warps) {
+        const int64_t trip = groups > 1 ? item / groups : item;
+        const int g0 = (int)(item - trip * groups) * kMlogitGroup, kg = min(kMlogitGroup, chains - g0);
+        const int64_t i0 = trip << 5, i = i0 + lane;
+        bool rv[4];
+#pragma unroll
+        for (int rb = 0; rb < 4; ++rb) rv[rb] = i0 + 8 * rb + gid < N;
+        // the first chain's loads of the epilogue go out with the first loads of X
+        MlogitNext m = mn;
+        m.E += g0 * UN; m.XB += g0 * UN; m.c += g0 * N; m.eta += g0 * N;
+        double ek[kMlogitMaxU], xbn;
+        mlogit_next_load(ek, xbn, m, i, N);
+        const double *base = tX + (i0 + gid) * P + 2 * tig;
+        const double *bc = beta + (int64_t)(g0 + min(gid, kg - 1)) * beta_stride + 2 * tig;
+        const bool bv = gid < kg;                                     // padding columns multiply zeros
+        double c[4][2] = {};
+#pragma unroll 2
+        for (int c0 = 0; c0 < P; c0 += 8) {
+            const bool cv = c0 + 2 * tig < P;
+            double2 a[4];
+#pragma unroll
+            for (int rb = 0; rb < 4; ++rb)
+                a[rb] = (cv && rv[rb]) ? __ldg(reinterpret_cast<const double2 *>(base + (size_t)(8 * rb) * P + c0))
+                                       : make_double2(0.0, 0.0);
+            const bool bl = cv && bv;
+            const double b0 = bl ? __ldg(bc + c0) : 0.0, b1 = bl ? __ldg(bc + c0 + 1) : 0.0;
+#pragma unroll
+            for (int rb = 0; rb < 4; ++rb) {
+                dmma884(c[rb][0], c[rb][1], a[rb].x, b0);
+                dmma884(c[rb][0], c[rb][1], a[rb].y, b1);
+            }
+        }
+        __syncwarp();                                                // the previous item's reads of the tile are done
+#pragma unroll
+        for (int rb = 0; rb < 4; ++rb) {
+            pt[(8 * rb + gid) * kMlogitTileLd + 2 * tig] = c[rb][0];
+            pt[(8 * rb + gid) * kMlogitTileLd + 2 * tig + 1] = c[rb][1];
+        }
+        __syncwarp();
+        for (int k = 0; k < kg; ++k) {
+            const int ch = g0 + k;
+            // the next chain's loads are in flight while this chain's epilogue runs
+            MlogitNext mnext = m;
+            mnext.E += UN; mnext.XB += UN; mnext.c += N; mnext.eta += N;
+            double en[kMlogitMaxU], xn;
+            mlogit_next_load(en, xn, mnext, k + 1 < kg ? i : N, N);
+            mlogit_next_epilogue(XB + ch * UN + (int64_t)mn.j * N, m, pt[lane * kMlogitTileLd + k], ek, xbn, i, N,
+                                 (int)(ch * N + i), (int)(chains * N), lane);
+            m = mnext;
+#pragma unroll
+            for (int u = 0; u < kMlogitMaxU; ++u) ek[u] = en[u];
+            xbn = xn;
+        }
+    }
+}
 
 // Weighted Gram on the FP64 tensor cores (DMMA).  A register-tiled DFMA version of this kernel
 // was bound by shared-memory bandwidth (LSU data pipe 75% busy, FP64 pipe 11%: every 16 FMAs
@@ -855,15 +955,16 @@ k_gram_reduce(double *__restrict__ PP, const double *__restrict__ P0,
 
 // out_p = sum_i x_i[p] * v_i  (X'v), v_i = c0*v0_i + c1*v1_i*v2_i  (v1/v2 optional).
 // Per-CTA partial sums then a fixed-order reduce (k_xtv_reduce).
+// Batched chains (this kernel and the two below): blockIdx.y = chain, its rows at tX + chain x_stride (N P: rows of
+// its own; 0: rows shared by the chains), its weights at + chain N.
 static __global__ void __launch_bounds__(256)
-k_xtv_partial(double *__restrict__ part, const double *__restrict__ tX, const double *__restrict__ v0,
+k_xtv_partial(double *__restrict__ part, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ v0,
               double c0, const double *__restrict__ v1, const double *__restrict__ v2, double c1,
               int64_t N, int P, const double *__restrict__ c1_dev = nullptr)
 {
     BL_PDL_ENTER();
     if (c1_dev) c1 = *c1_dev;                  // coefficient produced on the device (NB: log d)
-    // batched independent chains: blockIdx.y = chain
-    tX += (size_t)blockIdx.y * N * P;
+    tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     if (v0) v0 += (size_t)blockIdx.y * N;
     if (v1) v1 += (size_t)blockIdx.y * N;
@@ -899,13 +1000,13 @@ k_xtv_partial(double *__restrict__ part, const double *__restrict__ tX, const do
 // group of 16 rows of the CTA's slab, 16 loads of 16 bytes in flight per lane; the scalar
 // k_xtv_partial above keeps 4 rows in flight per warp and reaches 1.1 TB/s.
 static __global__ void __launch_bounds__(256, 2)
-k_xtv_mma(double *__restrict__ part, const double *__restrict__ tX, const double *__restrict__ v0,
+k_xtv_mma(double *__restrict__ part, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ v0,
           double c0, const double *__restrict__ v1, const double *__restrict__ v2, double c1,
           int64_t N, int P, const double *__restrict__ c1_dev)
 {
     BL_PDL_ENTER();
     if (c1_dev) c1 = *c1_dev;
-    tX += (size_t)blockIdx.y * N * P;
+    tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     if (v0) v0 += (size_t)blockIdx.y * N;
     if (v1) v1 += (size_t)blockIdx.y * N;
@@ -980,7 +1081,7 @@ __device__ __forceinline__ double xtv_weight(const double *w0, double c0, const 
 
 template <int kLog2L, int kMode>
 __global__ void __launch_bounds__(256, 2)
-k_xtv_stream(double *__restrict__ part, const double *__restrict__ tX, const double *__restrict__ v0,
+k_xtv_stream(double *__restrict__ part, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ v0,
              double c0, const double *__restrict__ v1, const double *__restrict__ v2, double c1,
              int64_t N, const double *__restrict__ c1_dev)
 {
@@ -988,7 +1089,7 @@ k_xtv_stream(double *__restrict__ part, const double *__restrict__ tX, const dou
     constexpr int L = 1 << kLog2L, P = 2 * L;            // column pairs per row, columns
     constexpr int kQ = L > 32 ? L / 32 : 1;              // column pairs a lane rotates through
     if (c1_dev) c1 = *c1_dev;
-    tX += (size_t)blockIdx.y * N * P;
+    tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     extern __shared__ double sacc[];                     // [warps][P]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
@@ -1068,13 +1169,14 @@ inline int xtv_stream_log2l(const double *tX, int P)
 
 static __global__ void k_xtv_reduce(double *__restrict__ out, const double *__restrict__ add0,
                              const double *__restrict__ add1, const double *__restrict__ part,
-                             int P, int nslab)
+                             int P, int nslab, int64_t out_stride)
 {
     BL_PDL_ENTER();
     int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= P) return;
-    // batched independent chains: blockIdx.y = chain (add0 is shared by the chains, add1 is not)
-    out += (size_t)blockIdx.y * P;
+    // batched independent chains: blockIdx.y = chain (add0 is shared by the chains, add1 is not); chain c's sums go
+    // to out + c out_stride (P: vectors side by side; P^2 + P: the X'v tail behind each chain's Gram sums)
+    out += (size_t)blockIdx.y * out_stride;
     part += (size_t)blockIdx.y * nslab * P;
     if (add1) add1 += (size_t)blockIdx.y * P;
     double s = 0.0;
@@ -1307,11 +1409,15 @@ static __global__ void k_fill(double *__restrict__ x, double v, int64_t n)
 // mlogit offsets for category j: A = sum_{k != j, k < J-1} exp(XB_k) + exp(0),
 // c = log A, eta = XB_j - c.  XB is N x (J-1) column-major (the reference's J-th
 // column is identically 0, MultLogit.hpp:275-277).  No max-subtraction, as there.
+// Several chains (blockIdx.y = chain): chain c's XB at XB + c U N, its c and eta at + c N.
 static __global__ void k_mlogit_offsets(double *__restrict__ c, double *__restrict__ eta,
                                  const double *__restrict__ XB, int64_t N, int U, int j)
 {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
+    XB += (size_t)blockIdx.y * U * N;
+    c += (size_t)blockIdx.y * N;
+    eta += (size_t)blockIdx.y * N;
     // the reference sums columns of XB_no_j in order: categories 0..J-1 without j, the
     // all-zero last column included (exp(0) = 1 added last)
     double A = 0.0;

@@ -248,6 +248,24 @@ def mlogit_gibbs(y, X, n, m0, P0, samp, burn, seed, flags=0, keep_w=True):
     return w, beta
 
 
+def mlogit_multichain(y, X, n, m0, P0, samp, burn, seed, chains, flags=0):
+    """`chains` independent multinomial logit chains on one data set: y [N x (J-1)], X [N x P], n [N], m0, P0 as
+    mlogit_gibbs takes them, shared by all chains.  Chain c is, bit for bit, mlogit_gibbs(..., seed=seed + c,
+    keep_w=False)[1], with X held once and read once per category update for up to 8 chains.  flags: 0 or UNFUSED.
+    Returns beta [chains x samp x (J-1) x P]."""
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    y = np.ascontiguousarray(y, dtype=np.float64)
+    N, P = X.shape
+    U = y.shape[1]
+    n = _f(n).ravel()
+    m0c, P0c = np.asfortranarray(_f(m0)), np.asfortranarray(_f(P0))
+    beta = np.zeros((max(int(chains), 0), samp, U, P))
+    st = _lib.lib().bl_mlogit_multichain(_p(beta), _p(y), _p(X), _p(n), m0c.ctypes.data, P0c.ctypes.data, int(chains),
+                                         N, P, U + 1, samp, burn, int(seed), int(flags))
+    _lib.check(st)
+    return beta
+
+
 def nb_gibbs(y, X, d, m0, P0, samp, seed):
     """NB regression with fixed dispersion d.  Returns (w_last [N], beta [samp x P])."""
     X = np.ascontiguousarray(X, dtype=np.float64)

@@ -257,6 +257,25 @@ int bl_logit_multichain_dev(double *beta, const double *y, const double *tX, con
                             const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
                             int flags, void *stream);
 
+/* Several independent multinomial logit chains on ONE data set (the multinomial counterpart of
+ * bl_logit_multichain).  ty: (J-1) x N, tX: P x N, n: [N], m0: P x (J-1), P0: P x P x (J-1), laid out as for
+ * bl_mlogit_gibbs and shared by all chains.  beta: [chains][samp] blocks of P x (J-1); chain c's block is, bit for
+ * bit, what bl_mlogit_gibbs(..., seed + c, BL_GIBBS_NO_W) returns.  omega is not returned.  X is held once and read
+ * once per category update for up to 8 chains; the launches per iteration do not depend on the number of chains.
+ * flags: 0 or BL_GIBBS_UNFUSED (separate psi and offsets kernels in every category update: the chains then equal
+ * the single chain run with BL_MLOGIT_UNFUSED=1 in the environment); any other flag is refused.  Limits, checked
+ * before anything is allocated: chains >= 1, J >= 2, chains * N < 2^31, P <= 111 (each chain's beta is drawn by one
+ * CTA out of shared memory; the single-chain entry takes P <= 256).  Device memory beyond the data: 2 chains (J-1)
+ * N doubles of linear predictors and their exponentials, and 32 bytes per (chain, row) of offsets, tilts, draws,
+ * shapes and the draw's index list.  Duplicate rows are not
+ * merged.  Spread the chains over GPUs by giving each rank the whole data set and a block of chains, called with
+ * seed + first chain of the block.  The host entry copies ty, X and n to the device once. */
+int bl_mlogit_multichain(double *beta, const double *ty, const double *tX, const double *n, const double *m0,
+                         const double *P0, int chains, int N, int P, int J, int samp, int burn, uint64_t seed, int flags);
+int bl_mlogit_multichain_dev(double *beta, const double *ty, const double *tX, const double *n, const double *m0,
+                             const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
+                             int flags, void *stream);
+
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */
 int bl_comm_unique_id(void *out128);

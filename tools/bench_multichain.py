@@ -2,6 +2,7 @@
 """Several logit chains on one data set (bl_logit_multichain) against the two ways to get them without it.
 
     python tools/bench_multichain.py [--N 1000000 --P 64 --chains 1,2,4,8 --iters 20 --reps 3]
+    python tools/bench_multichain.py --model mlogit [--N 1000000 --P 32 --J 10 --chains 1,2,4,8 --iters 20 --reps 3]
 
 For every chain count K and both beta draws, three arms are timed alternately in the same process, on the same
 device-resident data, and reported as ms per iteration of all K chains (median over the repetitions):
@@ -11,6 +12,13 @@ device-resident data, and reported as ms per iteration of all K chains (median o
 (a) and (b) start from the same seed and must give the same beta bit for bit (max_abs_diff_a_b).  The
 BL_GIBBS_TIMING stage split of one iteration of (a) and (b) comes from a separate, untimed call.  X is 512 MB at
 the default size, larger than L2, so every pass reads it from HBM.  Prints one JSON line.
+
+--model mlogit: multinomial logit chains (bl_mlogit_multichain), two arms alternated the same way:
+  (a) multichain: bl_mlogit_multichain_dev, one copy of X shared by the K chains;
+  (b) sequential: K calls of bl_mlogit_gibbs_dev with seed + c and omega dropped.
+Chain c of (a) must equal call c of (b) bit for bit (max_abs_diff_a_b).  Also reported: the stage split of the last
+category update of both arms and the kernel launches per iteration (bl_kernel_launches over a timed call / its
+iterations).  X is 256 MB at the default size (N = 1M, P = 32).
 """
 import argparse
 import json
@@ -139,10 +147,78 @@ def run(N, P, ks, iters, reps):
     return out
 
 
+def run_mlogit(N, P, J, ks, iters, reps):
+    import torch
+    from bayeslogit_b200 import _lib
+    L = _lib.lib()
+    dev = torch.device("cuda")
+    U = J - 1
+    g = torch.Generator(device=dev); g.manual_seed(20240011)
+    X = torch.randn(N, P, generator=g, device=dev, dtype=torch.float64) / (P - 1) ** 0.5
+    X[:, P - 1] = 1.0
+    B = torch.randn(P, U, generator=g, device=dev, dtype=torch.float64) * 0.5
+    logits = torch.cat([X @ B, torch.zeros(N, 1, device=dev, dtype=torch.float64)], dim=1)
+    cat = torch.multinomial(torch.softmax(logits, dim=1), 1, generator=g).squeeze(1)
+    Y = torch.nn.functional.one_hot(cat, J)[:, :U].double().contiguous()     # N x U row-major = ty, U x N column-major
+    n = torch.ones(N, device=dev, dtype=torch.float64)
+    m0 = torch.zeros(U, P, device=dev, dtype=torch.float64)                  # P x U column-major
+    P0 = (0.01 * torch.eye(P, device=dev, dtype=torch.float64)).expand(U, P, P).contiguous()
+    st = torch.cuda.current_stream().cuda_stream
+    seed = 20240011
+    out = {"model": "mlogit", "N": N, "P": P, "J": J, "iters": iters, "reps": reps, "results": []}
+
+    for K in ks:
+        def multichain(k):
+            beta = torch.zeros(K, k, U, P, device=dev, dtype=torch.float64)
+            _lib.check(L.bl_mlogit_multichain_dev(beta.data_ptr(), Y.data_ptr(), X.data_ptr(), n.data_ptr(),
+                                                  m0.data_ptr(), P0.data_ptr(), K, N, P, J, k, 0, seed, 0, st))
+            return beta
+
+        def sequential(k):
+            beta = torch.zeros(K, k, U, P, device=dev, dtype=torch.float64)
+            for c in range(K):
+                _lib.check(L.bl_mlogit_gibbs_dev(None, beta[c].data_ptr(), Y.data_ptr(), X.data_ptr(), n.data_ptr(),
+                                                 m0.data_ptr(), P0.data_ptr(), N, P, J, k, 0, seed + c, 2, 0, st))
+            return beta
+
+        arms = {"multichain": multichain, "sequential": sequential}
+        for fn in arms.values():                         # warm-up: modules, pools, every kernel of the timed window
+            fn(2)
+        torch.cuda.synchronize()
+        times = {a: [] for a in arms}
+        launches = {}
+        betas = {}
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        for _ in range(reps):
+            for a, fn in arms.items():                   # alternated: drifts of the shared machine hit every arm
+                l0 = L.bl_kernel_launches()
+                e0.record()
+                betas[a] = fn(iters)
+                e1.record()
+                torch.cuda.synchronize()
+                launches[a] = (L.bl_kernel_launches() - l0) / iters
+                times[a].append(e0.elapsed_time(e1) / iters)
+        med = {a: sorted(v)[len(v) // 2] for a, v in times.items()}
+        diff = float((betas["multichain"] - betas["sequential"]).abs().max().item())
+        out["results"].append({
+            "chains": K,
+            "ms_per_iteration_of_all_chains": med,
+            "ms_all_reps": times,
+            "sequential_over_multichain": med["sequential"] / med["multichain"],
+            "max_abs_diff_a_b": diff,
+            "launches_per_iteration": launches,
+            "stages_us": {"multichain": stage_split(lambda: multichain(2)),
+                          "sequential_one_chain": stage_split(lambda: sequential(2))},
+        })
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--model", choices=["logit", "mlogit"], default="logit")
     ap.add_argument("--N", type=int, default=1_000_000)
-    ap.add_argument("--P", type=int, default=64)
+    ap.add_argument("--P", type=int, default=None, help="default 64 (logit), 32 (mlogit)")
+    ap.add_argument("--J", type=int, default=10, help="categories (mlogit)")
     ap.add_argument("--chains", default="1,2,4,8")
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--reps", type=int, default=3)
@@ -151,7 +227,11 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("bench_multichain: no CUDA device")
     name, power = card()
-    out = run(a.N, a.P, [int(k) for k in a.chains.split(",")], a.iters, a.reps)
+    ks = [int(k) for k in a.chains.split(",")]
+    if a.model == "mlogit":
+        out = run_mlogit(a.N, a.P or 32, a.J, ks, a.iters, a.reps)
+    else:
+        out = run(a.N, a.P or 64, ks, a.iters, a.reps)
     out["device"] = name
     out["power_limit_w"] = power
     print(json.dumps(out))
