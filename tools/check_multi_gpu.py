@@ -1,6 +1,6 @@
 #!/usr/bin/env python3
 """Multi-GPU check of the sharded sweeps (run under torchrun, one rank per GPU): the row-sharded logit /
-NB chains equal the single-GPU chains and beta is bit-identical on every rank -- on the peer-window
+multinomial logit / NB chains (the NB ones with the dispersion fixed, drawn on the integers and drawn on the reals) equal the single-GPU chains and beta is bit-identical on every rank -- on the peer-window
 exchange (NCCL communicator + NVLink windows), on ncclAllReduce alone (BL_PEER_EXCHANGE=0), and on the
 windows alone (bl_comm_init_local: no NCCL communicator, the set-up sums go through k_peer_put /
 k_peer_combine too).  Prints MULTI_GPU_OK on rank 0.  One-GPU boxes: tests/test_gpu_multi.py runs the
@@ -106,6 +106,53 @@ def nb_df_chain(X, yc, lo, hi):
     return beta.cpu().numpy(), dd.cpu().numpy()
 
 
+def nb_dfreal_chain(X, yc, lo, hi):
+    """NB sweep with the dispersion walking on the reals (draw.df.real.mean): b = y + d is non-integer."""
+    P = X.shape[1]
+    Xd = torch.from_numpy(X[lo:hi].copy()).to(dev); yd = torch.from_numpy(yc[lo:hi].copy()).to(dev)
+    m0 = torch.zeros(P, device=dev, dtype=torch.float64)
+    P0 = (0.1 * torch.eye(P, device=dev, dtype=torch.float64)).contiguous()
+    beta = torch.zeros(10, P, device=dev, dtype=torch.float64)
+    dd = torch.zeros(10, device=dev, dtype=torch.float64)
+    rc = L.bl_nb_gibbs_dfreal_dev(None, beta.data_ptr(), dd.data_ptr(), yd.data_ptr(), Xd.data_ptr(), 2.5,
+                                  m0.data_ptr(), P0.data_ptr(), hi - lo, P, 10, 6, 4713, lo, st)
+    if rc:
+        _lib.check(rc)
+    torch.cuda.synchronize()
+    return beta.cpu().numpy(), dd.cpu().numpy()
+
+
+def make_mlogit(N, P, J, seed):
+    rng = np.random.default_rng(seed)
+    X = np.c_[rng.standard_normal((N, P - 1)) / np.sqrt(max(P - 1, 1)), np.ones(N)]
+    eta = np.c_[X @ rng.normal(0, 0.4, (P, J - 1)), np.zeros(N)]
+    pr = np.exp(eta)
+    pr /= pr.sum(1, keepdims=True)
+    cat = (pr.cumsum(1) < rng.random(N)[:, None]).sum(1)
+    Y = np.eye(J)[np.minimum(cat, J - 1)][:, :J - 1]
+    m0 = rng.normal(0, 0.05, (P, J - 1))
+    P0 = np.stack([(0.5 + 0.05 * j) * np.eye(P) for j in range(J - 1)], axis=2)
+    return X, Y, m0, P0
+
+
+def mlogit_chain(X, Y, m0, P0, lo, hi):
+    """Multinomial logit sweep: each category's X'kappa set-up and its 2 exchanges per update are all-reduced;
+    at P = 32 X'(Omega c_j) travels in the packed Gram's partial tile with the P^2 sums."""
+    P, U = X.shape[1], Y.shape[1]
+    Xd = torch.from_numpy(X[lo:hi].copy()).to(dev); yd = torch.from_numpy(Y[lo:hi].copy()).to(dev)
+    nd = torch.ones(hi - lo, device=dev, dtype=torch.float64)
+    m0d = torch.from_numpy(np.asfortranarray(m0).ravel(order="F")).to(dev)
+    P0d = torch.from_numpy(np.asfortranarray(P0).ravel(order="F")).to(dev)
+    beta = torch.zeros(5, U, P, device=dev, dtype=torch.float64)
+    w = torch.zeros(5, U, hi - lo, device=dev, dtype=torch.float64)
+    rc = L.bl_mlogit_gibbs_dev(w.data_ptr(), beta.data_ptr(), yd.data_ptr(), Xd.data_ptr(), nd.data_ptr(),
+                               m0d.data_ptr(), P0d.data_ptr(), hi - lo, P, U + 1, 5, 2, 808, 0, lo, st)
+    if rc:
+        _lib.check(rc)
+    torch.cuda.synchronize()
+    return beta.cpu().numpy(), w.cpu().numpy()
+
+
 # P = 16: the vectorised slot copy; P = 7, 15: odd P (P*P sums without a tail is an odd count -- the last
 # Gram entry travels on its own); N not a multiple of anything convenient
 CASES = [(200_003, 16), (50_001, 7), (60_001, 15)]
@@ -114,6 +161,11 @@ full = {(c, f): chain(data[c][0], data[c][1], 0, c[0], f) for c in CASES for f i
 c0 = CASES[0]
 nb_full = nb_chain(data[c0][0], data[c0][2], 0, c0[0])
 nbdf_full = nb_df_chain(data[c0][0], data[c0][2], 0, c0[0])
+nbdfreal_full = nb_dfreal_chain(data[c0][0], data[c0][2], 0, c0[0])
+# (N, P, J): P = 16 vectorised slot copy; P = 7 odd P^2 count; P = 32 the packed Gram's X'(Omega c_j) tail
+MCASES = [(200_003, 16, 4), (50_001, 7, 3), (60_001, 32, 5)]
+mdata = {c: make_mlogit(c[0], c[1], c[2], 20 + c[1]) for c in MCASES}
+mfull = {c: mlogit_chain(*mdata[c], 0, c[0]) for c in MCASES}
 
 ok = True
 
@@ -150,6 +202,27 @@ def sharded_pass(tag):
         print(f"[{tag}] nb with dispersion update: max rel diff beta {e_df:.2e}; d chain identical to the single-GPU chain "
               f"on every rank: {bad_d == 0.0} (d: {d_df[0]:.0f} .. {d_df[-1]:.0f})", flush=True)
     ok = ok and e_df < 1e-8 and bad_d == 0.0
+    b_dr, d_dr = nb_dfreal_chain(data[c0][0], data[c0][2], lo, hi)
+    e_dr = float(np.max(np.abs(b_dr - nbdfreal_full[0]) / np.abs(nbdfreal_full[0])))
+    ed_dr = float(np.max(np.abs(d_dr - nbdfreal_full[1]) / np.abs(nbdfreal_full[1])))
+    same_dr = same_on_all_ranks(d_dr) and same_on_all_ranks(b_dr)
+    e_dr, ed_dr = allmax([e_dr, ed_dr])
+    if rank == 0:
+        print(f"[{tag}] nb with real-valued dispersion: max rel diff beta {e_dr:.2e} d {ed_dr:.2e}; beta and d "
+              f"bit-identical across ranks: {same_dr} (d: {d_dr[0]:.3f} .. {d_dr[-1]:.3f})", flush=True)
+    ok = ok and e_dr < 1e-8 and ed_dr < 1e-12 and same_dr
+    for c in MCASES:
+        lo, hi = bdist.shard_range(rank, world, c[0])
+        b, w = mlogit_chain(*mdata[c], lo, hi)
+        fb, fw = mfull[c]
+        eb = np.max(np.abs(b - fb) / np.abs(fb))
+        ew = np.max(np.abs(w - fw[..., lo:hi]) / fw[..., lo:hi])
+        eb, ew = allmax([eb, ew])
+        same = same_on_all_ranks(b)
+        if rank == 0:
+            print(f"[{tag}] mlogit N={c[0]} P={c[1]} J={c[2]}: world={world} max rel diff beta {eb:.2e} omega {ew:.2e}; "
+                  f"beta bit-identical across ranks: {same}", flush=True)
+        ok = ok and max(eb, ew) < 1e-8 and same
 
 
 open_comm()
