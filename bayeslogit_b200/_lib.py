@@ -101,6 +101,8 @@ def lib():
     L.bl_logit_multichain_dev.argtypes = [vp] * 6 + [ci, i64, ci, ci, ci, u64, ci, vp]
     L.bl_mlogit_multichain.argtypes = [vp] * 6 + [ci, ci, ci, ci, ci, ci, u64, ci]
     L.bl_mlogit_multichain_dev.argtypes = [vp] * 6 + [ci, i64, ci, ci, ci, ci, u64, ci, vp]
+    L.bl_nb_multichain.argtypes = [vp, vp, vp, vp, cd, vp, vp, ci, ci, ci, ci, ci, u64, ci]
+    L.bl_nb_multichain_dev.argtypes = [vp, vp, vp, vp, cd, vp, vp, ci, i64, ci, ci, ci, u64, ci, vp]
     L.bl_comm_unique_id.argtypes = [vp]
     L.bl_comm_init.argtypes = [vp, ci, ci]
     L.bl_comm_init_local.argtypes = [ci, ci]

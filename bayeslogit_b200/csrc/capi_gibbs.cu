@@ -478,6 +478,40 @@ int bl_mlogit_multichain(double *beta, const double *ty, const double *tX, const
     return 0;
 }
 
+int bl_nb_multichain_dev(double *beta, double *d_out, const double *y, const double *tX, double d0,
+                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
+                         uint64_t seed, int dmode, void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    std::string err;
+    if (nb_multichain_device(beta, d_out, y, tX, d0, m0, P0, chains, N, P, samp, burn, seed, dmode, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
+int bl_nb_multichain(double *beta, double *d_out, const double *y, const double *tX, double d0,
+                     const double *m0, const double *P0, int chains, int N, int P, int samp, int burn,
+                     uint64_t seed, int dmode)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    std::string err;
+    // checked before any buffer is made: the device driver repeats the checks
+    if (nb_multichain_check(chains, N, P, samp, burn, d0, dmode, err)) return report(err, nullptr);
+    Dev d;
+    double *dy = d.put(y, N, err), *dX = d.put(tX, (size_t)N * P, err);        // one copy of the data
+    double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
+    const size_t nb = (size_t)chains * samp * P, nd = (size_t)chains * samp;
+    double *dbeta = d.put(nullptr, nb, err), *dd = d_out ? d.put(nullptr, nd, err) : nullptr;
+    if (!err.empty()) return report(err, nullptr);
+    if (nb_multichain_device(dbeta, dd, dy, dX, d0, dm0, dP0, chains, N, P, samp, burn, seed, dmode,
+                             (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * nb, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && d_out) e = cudaMemcpy(d_out, dd, sizeof(double) * nd, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
 int bl_mlogit_gibbs_dev(double *w, double *beta, const double *ty, const double *tX, const double *n,
                         const double *m0, const double *P0, int64_t N, int P, int J, int samp, int burn,
                         uint64_t seed, int flags, uint64_t obs0, void *stream)

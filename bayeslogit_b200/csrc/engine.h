@@ -30,7 +30,8 @@ struct DevTape {
     int lu, le, ln, lg;
 };
 
-// Batch draw, Philox streams.  shape: int32 for kDevroye, double otherwise.
+// Batch draw, Philox streams.  shape: int32 for kDevroye, double otherwise.  id.chain_len keys the streams by chain for
+// kDevroye and kHybrid (launch_hybrid_binned likewise).
 cudaError_t launch_rpg(Method m, double *x, const void *shape, const double *z, int64_t num,
                        int trunc, int *iter, StreamId id, cudaStream_t stream);
 
@@ -96,6 +97,13 @@ int mlogit_multichain_check(int chains, int64_t N, int P, int J, int samp, int b
 int mlogit_multichain_device(double *beta_out, const double *ty, const double *tX, const double *n, const double *m0,
                              const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
                              int flags, cudaStream_t st, std::string &err);
+// Several negative-binomial chains on one data set (y [N], tX P x N, shared); beta_out: [chains][samp][P], d_out:
+// [chains][samp] or null.  dmode: BL_NB_D_FIXED / _INT / _REAL.  The check refuses what the driver cannot run, before
+// anything is allocated or launched.
+int nb_multichain_check(int chains, int64_t N, int P, int samp, int burn, double d0, int dmode, std::string &err);
+int nb_multichain_device(double *beta_out, double *d_out, const double *y, const double *tX, double d0, const double *m0,
+                         const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int dmode,
+                         cudaStream_t st, std::string &err);
 int logit_em_device(double *beta, const double *y, const double *tX, const double *n, int64_t N,
                     int P, double tol, int max_iter, int *iters, cudaStream_t st, std::string &err);
 // duplicate-row merge on device-resident data (merge.cu); returns M, -1 (CUDA error), -2 (needs the exact host merge)

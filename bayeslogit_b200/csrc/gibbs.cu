@@ -240,6 +240,13 @@ constexpr bool kSlowBeta = true;          // A/B build: the panel factorisation 
 constexpr bool kSlowBeta = false;
 #endif
 
+// Global scratch of one k_beta_draw<false> CTA: A, B (ld x P each), 5 P of vectors, the constrained draw's P^2 + 2P
+// rejection normals.  Batched chains (grid = chains) take one such block each.
+__host__ __device__ inline size_t beta_gwork_doubles(int P)
+{
+    return 2 * (size_t)(P + 1) * P + 5 * (size_t)P + (size_t)P * P + 2 * (size_t)P;
+}
+
 // kPlainOnly: the plain / mvn draw with P <= 64 alone (cta_plain_fast) -- a tenth of the code, and registers for two
 // CTAs per SM: the batched chains run one CTA per chain.
 template <bool SMEM, bool kPlainOnly = false>
@@ -264,7 +271,7 @@ k_beta_draw(int mode, const double *__restrict__ acc, const double *__restrict__
     long long k0 = clock64();
 #endif
     const int ld = P | 1;                     // odd leading dimension: row and column walks both conflict-free
-    double *A = SMEM ? sm : gwork;
+    double *A = SMEM ? sm : gwork + blockIdx.x * beta_gwork_doubles(P);
     double *B = A + (size_t)ld * P;
     double *v = B + (size_t)ld * P;
     double *rhs = v + 4 * P;
@@ -478,6 +485,24 @@ Slabs slab_partition(int64_t N, int P)
     return g;
 }
 
+// The single chain's beta draw workspace: `plain` bytes of shared memory for the plain / mvn draw, `tn` with the
+// constrained draw's rejection normals; above 200 KB of `tn` every draw runs out of global scratch (k_beta_draw<false>).
+struct BetaSmem {
+    size_t plain = 0, tn = 0;
+    bool use_smem = true;
+};
+
+BetaSmem beta_smem_of(int P)
+{
+    BetaSmem b;
+    // A, B (ld x P each), 5 P vector scratch; the constrained draw's P^2 + 2P rejection normals behind them
+    b.plain = (2 * (size_t)(P | 1) * P + 5 * (size_t)P) * sizeof(double);
+    if (P <= 64) b.plain = (beta_fast_e_offset(P) + 64) * sizeof(double);      // cta_plain_fast: + its normals
+    b.tn = std::max(b.plain + ((size_t)P * P + 2 * (size_t)P) * sizeof(double), beta_tn_doubles(P) * sizeof(double));
+    b.use_smem = b.tn <= 200 * 1024;
+    return b;
+}
+
 // Shared machinery of the three sweeps.
 struct Sweep {
     int64_t N = 0;          // local observations
@@ -507,14 +532,13 @@ struct Sweep {
         GB_CK(m.get(&acc, (size_t)P * P + P));
         GB_CK(m.get(&part, (size_t)tiles * nslab * 2 * kGramTile * kGramTile));
         GB_CK(m.get(&xtv_part, (size_t)xtv_slabs * P));
-        GB_CK(m.get(&gwork, 2 * (size_t)(P + 1) * P + 5 * (size_t)P + (size_t)P * P + 2 * (size_t)P));
+        GB_CK(m.get(&gwork, beta_gwork_doubles(P)));
         GB_CK(m.get(&status, 1));
         GB_CK(cudaMemsetAsync(status, 0, sizeof(int), st));
         GB_CK(cudaMemsetAsync(acc, 0, ((size_t)P * P + P) * sizeof(double), st));
-        // A, B (ld x P each), 5 P vector scratch; the constrained draw's P^2 + 2P rejection normals behind them
-        beta_smem = (2 * (size_t)(P | 1) * P + 5 * (size_t)P) * sizeof(double);
-        if (P <= 64) beta_smem = (beta_fast_e_offset(P) + 64) * sizeof(double);      // cta_plain_fast: + its normals
-        beta_smem_tn = std::max(beta_smem + ((size_t)P * P + 2 * (size_t)P) * sizeof(double), beta_tn_doubles(P) * sizeof(double));
+        const BetaSmem bs = beta_smem_of(P);
+        beta_smem = bs.plain;
+        beta_smem_tn = bs.tn;
         GB_CK(m.get(&tnbuf, (size_t)P * P + 2 * (size_t)P));
         GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRows, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)gram_smem_bytes(true)));
@@ -522,7 +546,7 @@ struct Sweep {
                                    (int)gram_smem_bytes(false)));
         GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                    (int)gram_smem_bytes(false, true)));
-        use_smem = beta_smem_tn <= 200 * 1024;
+        use_smem = bs.use_smem;
         if (use_smem && beta_smem_tn > 48 * 1024)
             GB_CK(cudaFuncSetAttribute(k_beta_draw<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)beta_smem_tn));
         if (use_smem && beta_smem > 48 * 1024)
@@ -1034,11 +1058,15 @@ static size_t mlogit_multichain_beta_smem(int P)
                     P <= 64 ? (beta_fast_e_offset(P) + 64) * sizeof(double) : (size_t)0);
 }
 
+constexpr int kMaxGridChains = 65535;   // largest y / z grid dimension
+
 int mlogit_multichain_check(int chains, int64_t N, int P, int J, int samp, int burn, int flags, std::string &err)
 {
     if (chains <= 0 || N <= 0 || P <= 0 || J < 2 || samp <= 0 || burn < 0) { err = "mlogit_multichain: bad dimensions"; return 1; }
     if (flags & ~BL_GIBBS_UNFUSED) { err = "mlogit_multichain: unsupported flags (only BL_GIBBS_UNFUSED is accepted)"; return 1; }
     if ((int64_t)chains * N >= (1LL << 31)) { err = "mlogit_multichain: chains * N must stay below 2^31 observations per call"; return 1; }
+    // the chain is a y or z grid dimension of the offsets, X'v and Gram launches
+    if (chains > kMaxGridChains) { err = "mlogit_multichain: chains must be at most 65535"; return 1; }
     // each chain's mvn draw runs in one CTA out of shared memory: P <= 111
     if (P > 256 || mlogit_multichain_beta_smem(P) > 200 * 1024) { err = "mlogit_multichain: P too large for the shared-memory beta draw"; return 1; }
     return 0;
@@ -1174,7 +1202,7 @@ int mlogit_multichain_device(double *beta_out, const double *ty, const double *t
                     launch_pdl(k_xbeta_mma<true>, dim3(grid), dim3(256), 0, st, XB + (size_t)N * j, N, tX, N * P, bj,
                                (int64_t)0, 1, N, P, nullptr, 0.0, 0.0, mn);
                 } else {
-                    const int64_t items = (N + 31) / 32 * ((K + kMlogitGroup - 1) / kMlogitGroup);
+                    const int64_t items = (N + 31) / 32 * ((K + kGroupChains - 1) / kGroupChains);
                     const int grid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (items + 7) / 8));
                     launch_pdl(k_mlogit_psi_shared, dim3(grid), dim3(256), 0, st, XB, tX, bj, bstride, K, N, P, mn);
                 }
@@ -1349,6 +1377,217 @@ int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const dou
     }
     GB_CK(cudaGetLastError());
     return s.check_status(err, "nb_gibbs_df");
+}
+
+// ------------------------------------------------------------------------------------
+// Several negative-binomial chains on ONE data set (bl_nb_multichain): chain c is, bit for bit, the chain
+// nb_gibbs_df_device runs with seed + c (dmode BL_NB_D_INT / BL_NB_D_REAL), or, with d fixed (BL_NB_D_FIXED),
+// iterations burn .. burn + samp - 1 of nb_gibbs_device with seed + c.  Every stage is one launch for all chains and
+// follows the single chain's stage, with its summation order:
+//   phi   : X beta of all chains from one read of X (k_xbeta_shared, 8 chains per pass; one chain: k_xbeta_mma; odd
+//           P or unaligned X: k_xbeta with a chain grid dimension).  Fixed d: psi = phi - log d in the same pass.
+//   d     : (sampled d) the single chain's dispersion kernels with a chain dimension over its nblk slabs; ymax, the
+//           histogram and G depend on y alone and are formed once.
+//   omega : one rpg_hybrid batch over chains * N (chain, row) pairs, the stream of (chain, row) keyed by (seed + c,
+//           row).  The binned or per-lane sampler is picked by N, as the single chain picks it, so every draw runs
+//           the single chain's sampler code.
+//   sums  : the single chain's X'v and Gram slab partition and kernels with a chain grid dimension, X stride 0.
+//   beta  : one plain draw per chain side by side, the single chain's instantiation (shared memory; above P ~ 92
+//           global scratch, one block per chain).
+// Per-chain state: psi, omega, kappa, shapes [chains][N]; d at dvec[c], log d at dvec[chains + c] (one chain: the
+// single chain's (d, log d) pair).  beta_out: [chains][samp][P]; d_out: [chains][samp] or null.
+// ------------------------------------------------------------------------------------
+int nb_multichain_check(int chains, int64_t N, int P, int samp, int burn, double d0, int dmode, std::string &err)
+{
+    if (chains < 1) { err = "nb_multichain: chains must be at least 1"; return 1; }
+    if (N < 1 || P < 1 || samp < 1 || burn < 0) { err = "nb_multichain: bad dimensions"; return 1; }
+    if ((int64_t)chains * N >= (1LL << 31)) { err = "nb_multichain: chains * N must stay below 2^31 observations per call"; return 1; }
+    // the chain is a y or z grid dimension of the dispersion, X'v and Gram launches
+    if (chains > kMaxGridChains) { err = "nb_multichain: chains must be at most 65535"; return 1; }
+    if (P > 256) { err = "nb_multichain: P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
+    if (dmode != BL_NB_D_FIXED && dmode != BL_NB_D_INT && dmode != BL_NB_D_REAL) {
+        err = "nb_multichain: unknown dmode (BL_NB_D_FIXED, BL_NB_D_INT or BL_NB_D_REAL)";
+        return 1;
+    }
+    if (dmode == BL_NB_D_INT && (!(d0 >= 1.0) || d0 != floor(d0))) { err = "nb_multichain: bad arguments (d0 must be a positive integer)"; return 1; }
+    if (dmode != BL_NB_D_INT && !(d0 > 0.0)) { err = "nb_multichain: bad arguments (d0 must be positive)"; return 1; }
+    return 0;
+}
+
+int nb_multichain_device(double *beta_out, double *d_out, const double *y, const double *tX, double d0, const double *m0,
+                         const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int dmode,
+                         cudaStream_t st, std::string &err)
+{
+    if (nb_multichain_check(chains, N, P, samp, burn, d0, dmode, err)) return 1;
+    const int K = chains;
+    const int64_t T = (int64_t)K * N;
+    const bool fixed = dmode == BL_NB_D_FIXED, real_d = dmode == BL_NB_D_REAL;
+    const Slabs g = slab_partition(N, P);
+    const int nt = g.nt, tiles = nt * (nt + 1) / 2, slabs_total = nt > 1 ? 2 * g.nslab : g.nslab;
+    const bool packed = gram_packed(P);
+    const size_t accn = (size_t)P * P + P;
+    const BetaSmem bs = beta_smem_of(P);
+    const bool lean = P <= 64 && !kSlowBeta;            // Sweep::beta_draw's plain-draw instantiation
+    const bool binned = N >= (1 << 15);                 // the single chain's choice of sampler path, by its own N
+    const int nblk = (int)std::min<int64_t>(148 * 4, std::max<int64_t>(1, N / 1024));   // as nb_gibbs_df_device
+    DevMem mem;
+    mem.st = st;
+    double *psi, *w, *kappa, *shape, *acc, *part, *xtv_part, *b0, *bscr, *dvec = nullptr, *dfpart = nullptr,
+           *G = nullptr, *gwork = nullptr;
+    int *status;
+    void *work = nullptr;
+    GB_CK(mem.get(&psi, T));
+    GB_CK(mem.get(&w, T));
+    GB_CK(mem.get(&kappa, T));
+    GB_CK(mem.get(&shape, T));
+    GB_CK(mem.get(&acc, accn * K));
+    GB_CK(mem.get(&part, (size_t)K * tiles * g.nslab * 2 * kGramTile * kGramTile));
+    GB_CK(mem.get(&xtv_part, (size_t)K * g.xtv_slabs * P));
+    GB_CK(mem.get(&b0, (size_t)K * P));                 // P0 m0, one copy per chain: k_beta_draw reads chain c's at + c P
+    GB_CK(mem.get(&bscr, (size_t)K * 2 * P));           // burn-in betas [chain][parity][P]
+    GB_CK(mem.get(&status, 1));
+    if (binned) GB_CK(mem.get((char **)&work, hybrid_workspace_bytes(T)));
+    if (!bs.use_smem) GB_CK(mem.get(&gwork, beta_gwork_doubles(P) * K));
+    GB_CK(cudaMemsetAsync(status, 0, sizeof(int), st));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRows, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(true)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false, true)));
+    if (bs.use_smem && bs.plain > 48 * 1024)
+        GB_CK(cudaFuncSetAttribute(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bs.plain));
+
+    k_matvec<<<cdiv(P, 128), 128, 0, st>>>(b0, P0, m0, P);
+    count_launch();
+    for (int c = 1; c < K; ++c)
+        GB_CK(cudaMemcpyAsync(b0 + (size_t)P * c, b0, sizeof(double) * P, cudaMemcpyDeviceToDevice, st));
+    const double ld0 = log(d0);
+    int ymax = 0;
+    if (fixed) {
+        // kappa = (y - d)/2 and b = y + d are the same for every chain: formed once, then copied
+        k_kappa<<<cdiv(N, 256), 256, 0, st>>>(kappa, y, nullptr, d0, N);
+        k_shape_add<<<cdiv(N, 256), 256, 0, st>>>(shape, y, d0, N);
+        count_launch(2);
+        for (int64_t r = N; r < T; r += N) {
+            GB_CK(cudaMemcpyAsync(kappa + r, kappa, sizeof(double) * N, cudaMemcpyDeviceToDevice, st));
+            GB_CK(cudaMemcpyAsync(shape + r, shape, sizeof(double) * N, cudaMemcpyDeviceToDevice, st));
+        }
+        if (d_out) {
+            k_fill<<<(int)std::min<int64_t>(148 * 8, cdiv((int64_t)K * samp, 256)), 256, 0, st>>>(d_out, d0, (int64_t)K * samp);
+            count_launch();
+        }
+    } else {
+        // ymax and G[j] = #{y_i > j}, as nb_gibbs_df_device forms them, shared by the chains
+        unsigned long long *ymax_d, *hist;
+        GB_CK(mem.get(&ymax_d, 1));
+        GB_CK(cudaMemsetAsync(ymax_d, 0, sizeof(unsigned long long), st));
+        k_nb_ymax<<<148 * 2, 256, 0, st>>>(ymax_d, y, N);
+        count_launch();
+        unsigned long long ymax64 = 0;
+        GB_CK(cudaMemcpyAsync(&ymax64, ymax_d, sizeof(ymax64), cudaMemcpyDeviceToHost, st));
+        GB_CK(cudaStreamSynchronize(st));
+        ymax = (int)ymax64;
+        GB_CK(mem.get(&hist, (size_t)ymax + 2));
+        GB_CK(mem.get(&G, (size_t)ymax + 1));
+        GB_CK(cudaMemsetAsync(hist, 0, sizeof(unsigned long long) * ((size_t)ymax + 2), st));
+        k_nb_hist<<<148 * 2, 256, 0, st>>>(hist, y, N);
+        k_nb_suffix<<<1, 1, 0, st>>>(G, hist, ymax);
+        count_launch(2);
+        GB_CK(mem.get(&dfpart, (size_t)K * nblk * 4));
+        GB_CK(mem.get(&dvec, 2 * (size_t)K));
+        std::vector<double> dinit(2 * (size_t)K, d0);
+        for (int c = 0; c < K; ++c) dinit[(size_t)K + c] = ld0;
+        GB_CK(cudaMemcpyAsync(dvec, dinit.data(), sizeof(double) * 2 * K, cudaMemcpyHostToDevice, st));
+        GB_CK(cudaStreamSynchronize(st));         // dinit is a pageable host buffer that leaves scope
+    }
+    GB_CK(cudaMemsetAsync(bscr, 0, sizeof(double) * 2 * P * (size_t)K, st));
+
+    const int64_t bstride = (int64_t)P * samp;          // chain stride of beta_out
+    const bool mma = xbeta_mma_ok(tX, P);
+    const int xgrid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));     // Sweep::xbeta's grid
+    const int64_t items = (N + 31) / 32 * ((K + kGroupChains - 1) / kGroupChains);
+    const int sgrid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (items + 7) / 8));
+    const double shift = fixed ? -ld0 : 0.0;
+    static const int tn_flags = getenv("BL_BETA_NO_SPEC") ? 3 : 1;
+    StageTimer tmr;
+    tmr.st = st;
+    for (int t = 0; t < burn + samp; ++t) {
+        // the beta every chain conditions on: the burn-in slot of parity t, or its last recorded draw
+        const double *bprev = t <= burn ? bscr + (size_t)P * (t & 1) : beta_out + (size_t)P * (t - 1 - burn);
+        const int64_t pstride = t <= burn ? 2 * (int64_t)P : bstride;
+        const bool rec = t >= burn;
+        double *bnext = rec ? beta_out + (size_t)P * (t - burn) : bscr + (size_t)P * ((t + 1) & 1);
+        const int64_t nstride = rec ? bstride : 2 * (int64_t)P;
+        tmr.arm(t == burn + samp - 1);
+        if (mma && K == 1)
+            launch_pdl(k_xbeta_mma<false>, dim3(xgrid), dim3(256), 0, st, psi, N, tX, N * P, bprev, (int64_t)0, 1, N, P,
+                       (const double *)nullptr, 0.0, shift, MlogitNext{});
+        else if (mma)
+            launch_pdl(k_xbeta_shared, dim3(sgrid), dim3(256), 0, st, psi, tX, bprev, pstride, K, N, P, shift);
+        else
+            k_xbeta<<<dim3(xgrid, K), 256, P * sizeof(double), st>>>(psi, tX, bprev, nullptr, 0.0, shift, N, P, pstride);
+        count_launch();
+        tmr.mark("xbeta");
+        if (!fixed) {
+            // d | beta of every chain, then psi = phi - log d, b = y + d, kappa = (y - d)/2
+            double *drec = rec && d_out ? d_out + (t - burn) : nullptr;
+            if (real_d) {
+                k_nb_dfreal_partial<<<dim3(nblk, K), 256, 0, st>>>(dfpart, psi, y, dvec, N, seed, (uint32_t)t);
+                k_nb_dfreal_decide<<<K, 32, 0, st>>>(dvec, dvec + K, drec, dfpart, nblk, seed, (uint32_t)t, (int64_t)samp);
+            } else {
+                k_nb_df_partial<<<dim3(nblk, K), 256, 0, st>>>(dfpart, psi, y, dvec, N, seed, (uint32_t)t);
+                k_nb_df_decide<<<K, 32, 0, st>>>(dvec, dvec + K, drec, dfpart, nblk, G, ymax, seed, (uint32_t)t, (int64_t)samp);
+            }
+            k_nb_prepare<<<dim3(cdiv(N, 256), K), 256, 0, st>>>(psi, shape, kappa, y, dvec, dvec + K, N);
+            count_launch(3);
+            tmr.mark("dispersion");
+        }
+        // one chain: the plain stream is the chain-keyed one, and the single chain's sampler kernels run
+        const StreamId id{seed, 0, (uint32_t)t, K > 1 ? (uint32_t)N : 0u};
+        cudaError_t e = binned ? launch_hybrid_binned(w, shape, psi, (int)T, id, work, st)
+                               : launch_rpg(kHybrid, w, shape, psi, T, 0, nullptr, id, st);
+        if (e != cudaSuccess) { err = cudaGetErrorString(e); return 1; }
+        tmr.mark("draw");
+        // X'(kappa + omega log d) of every chain into the tail of its sums
+        launch_xtv(dim3(g.xtv_slabs, K), st, xtv_part, tX, 0, kappa, 1.0, w, nullptr, fixed ? ld0 : 0.0, N, P,
+                   fixed ? nullptr : dvec + K);
+        launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128), K), dim3(128), 0, st, acc + (size_t)P * P, (const double *)nullptr,
+                   (const double *)nullptr, xtv_part, P, g.xtv_slabs, (int64_t)accn);
+        count_launch(2);
+        tmr.mark("xtv");
+        if (nt > 1)
+            launch_pdl(k_gram_partial<kGramRows, false>, dim3(g.nslab, tiles, K), dim3(256), gram_smem_bytes(true), st,
+                       part, tX, (int64_t)0, w, N, P, nt, g.nslab_diag, (const double *)nullptr);
+        else if (packed)
+            launch_pdl(k_gram_partial<kGramRowsDiag, true, true>, dim3(g.nslab, tiles, K), dim3(256),
+                       gram_smem_bytes(false, true), st, part, tX, (int64_t)0, w, N, P, nt, 0, (const double *)nullptr);
+        else
+            launch_pdl(k_gram_partial<kGramRowsDiag, true>, dim3(g.nslab, tiles, K), dim3(256), gram_smem_bytes(false),
+                       st, part, tX, (int64_t)0, w, N, P, nt, 0, (const double *)nullptr);
+        launch_pdl(k_gram_reduce, dim3(cdiv((int64_t)P * P, 32), K), dim3(256), 0, st, acc, (const double *)nullptr,
+                   part, P, nt, slabs_total, PeerPush{}, packed ? 1 : 0, 2 * g.nslab_diag, 0);
+        count_launch(2);
+        tmr.mark("gram");
+        if (bs.use_smem)
+            launch_pdl(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>, dim3(K), dim3(256), bs.plain, st,
+                       (int)kBetaPlain, (const double *)acc, P0, (const double *)b0, 1, (const double *)nullptr, bnext,
+                       (double *)nullptr, P, seed, (uint32_t)t, status, PeerWait{}, nstride, (const double *)nullptr,
+                       tn_flags);
+        else
+            k_beta_draw<false><<<K, 256, 0, st>>>(kBetaPlain, acc, P0, b0, 1, nullptr, bnext, gwork, P, seed, (uint32_t)t,
+                                                  status, PeerWait{}, nstride, nullptr, 0);
+        count_launch();
+        tmr.mark("beta");
+        tmr.report("nb multichain");
+    }
+    GB_CK(cudaGetLastError());
+    int h = 0;
+    GB_CK(cudaMemcpyAsync(&h, status, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (h != 0) { err = "nb_multichain: a chain's posterior precision is not positive definite"; return 1; }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------

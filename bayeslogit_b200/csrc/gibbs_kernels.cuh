@@ -30,11 +30,16 @@ namespace bl {
 // rows, lane r ending up with row r) instead of a 5-step butterfly per row -- the per-row form
 // spent 66 warp instructions per row and ran at 4.3 TB/s with the LSU and ALU pipes half busy.
 // HBM-bound: N P 8 bytes.
+// Several chains on shared rows (bl_nb_multichain, odd P or unaligned X): blockIdx.y = chain c, which meets
+// beta + c beta_stride and writes psi + c N (off is read at + c N); every row sums in the single chain's order.
 // ---------------------------------------------------------------------------------
 static __global__ void __launch_bounds__(256, 2)
 k_xbeta(double *__restrict__ psi, const double *__restrict__ tX, const double *__restrict__ beta,
-        const double *__restrict__ off, double off_scale, double shift, int64_t N, int P)
+        const double *__restrict__ off, double off_scale, double shift, int64_t N, int P, int64_t beta_stride = 0)
 {
+    beta += blockIdx.y * beta_stride;
+    psi += blockIdx.y * N;
+    if (off) off += blockIdx.y * N;
     extern __shared__ __align__(16) double sbeta[];
     for (int p = threadIdx.x; p < P; p += blockDim.x) sbeta[p] = beta[p];
     __syncthreads();
@@ -321,61 +326,71 @@ inline bool xbeta_mma_ok(const double *tX, int P) { return P % 2 == 0 && (reinte
 //   state : chain c's XB and E at [c][U][N] (XB is also where XB_j is written), its c and eta at mn.c / mn.eta +
 //           c N.  The next draw's index list (optional) holds all chains * N (chain, row) pairs as c N + i.
 // ---------------------------------------------------------------------------------
-constexpr int kMlogitGroup = 8;                  // chains per pass: the 8 columns of an m8n8k4 tile
-constexpr int kMlogitTileLd = kMlogitGroup + 1;  // odd row stride: lane l reading row l is conflict-free
+constexpr int kGroupChains = 8;                  // chains per pass: the 8 columns of an m8n8k4 tile
+constexpr int kGroupTileLd = kGroupChains + 1;   // odd row stride: lane l reading row l is conflict-free
+
+// The MMA trip of the shared-rows kernels, called by the whole warp: rows i0 .. i0 + 31 of X (P x N, even P, 16-byte
+// aligned) times the beta of chains g0 .. g0 + kg - 1 (B column gid = chain g0 + gid; padding columns multiply zeros).
+// Leaves the 32 x 8 product in the warp's tile pt (row r, chain g0 + k at r kGroupTileLd + k).
+__device__ __forceinline__ void shared_rows_tile(double *pt, const double *__restrict__ tX, const double *__restrict__ beta,
+                                                 int64_t beta_stride, int g0, int kg, int64_t i0, int64_t N, int P, int lane)
+{
+    const int gid = lane >> 2, tig = lane & 3;
+    bool rv[4];
+#pragma unroll
+    for (int rb = 0; rb < 4; ++rb) rv[rb] = i0 + 8 * rb + gid < N;
+    const double *base = tX + (i0 + gid) * P + 2 * tig;
+    const double *bc = beta + (int64_t)(g0 + min(gid, kg - 1)) * beta_stride + 2 * tig;
+    const bool bv = gid < kg;                                         // padding columns multiply zeros
+    double c[4][2] = {};
+#pragma unroll 2
+    for (int c0 = 0; c0 < P; c0 += 8) {
+        const bool cv = c0 + 2 * tig < P;
+        double2 a[4];
+#pragma unroll
+        for (int rb = 0; rb < 4; ++rb)
+            a[rb] = (cv && rv[rb]) ? __ldg(reinterpret_cast<const double2 *>(base + (size_t)(8 * rb) * P + c0))
+                                   : make_double2(0.0, 0.0);
+        const bool bl = cv && bv;
+        const double b0 = bl ? __ldg(bc + c0) : 0.0, b1 = bl ? __ldg(bc + c0 + 1) : 0.0;
+#pragma unroll
+        for (int rb = 0; rb < 4; ++rb) {
+            dmma884(c[rb][0], c[rb][1], a[rb].x, b0);
+            dmma884(c[rb][0], c[rb][1], a[rb].y, b1);
+        }
+    }
+    __syncwarp();                                                    // the previous item's reads of the tile are done
+#pragma unroll
+    for (int rb = 0; rb < 4; ++rb) {
+        pt[(8 * rb + gid) * kGroupTileLd + 2 * tig] = c[rb][0];
+        pt[(8 * rb + gid) * kGroupTileLd + 2 * tig + 1] = c[rb][1];
+    }
+    __syncwarp();
+}
 
 static __global__ void __launch_bounds__(256, 2)
 k_mlogit_psi_shared(double *XB, const double *__restrict__ tX, const double *__restrict__ beta,
                     int64_t beta_stride, int chains, int64_t N, int P, MlogitNext mn)
 {
     BL_PDL_ENTER();
-    __shared__ double tile[8][32 * kMlogitTileLd];
-    const int lane = threadIdx.x & 31, gid = lane >> 2, tig = lane & 3;
+    __shared__ double tile[8][32 * kGroupTileLd];
+    const int lane = threadIdx.x & 31;
     double *pt = tile[threadIdx.x >> 5];
-    const int groups = (chains + kMlogitGroup - 1) / kMlogitGroup;
+    const int groups = (chains + kGroupChains - 1) / kGroupChains;
     const int64_t UN = (int64_t)mn.U * N;
     const int64_t items = ((N + 31) >> 5) * groups;
     const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
     const int64_t wid = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     for (int64_t item = wid; item < items; item += warps) {
         const int64_t trip = groups > 1 ? item / groups : item;
-        const int g0 = (int)(item - trip * groups) * kMlogitGroup, kg = min(kMlogitGroup, chains - g0);
+        const int g0 = (int)(item - trip * groups) * kGroupChains, kg = min(kGroupChains, chains - g0);
         const int64_t i0 = trip << 5, i = i0 + lane;
-        bool rv[4];
-#pragma unroll
-        for (int rb = 0; rb < 4; ++rb) rv[rb] = i0 + 8 * rb + gid < N;
         // the first chain's loads of the epilogue go out with the first loads of X
         MlogitNext m = mn;
         m.E += g0 * UN; m.XB += g0 * UN; m.c += g0 * N; m.eta += g0 * N;
         double ek[kMlogitMaxU], xbn;
         mlogit_next_load(ek, xbn, m, i, N);
-        const double *base = tX + (i0 + gid) * P + 2 * tig;
-        const double *bc = beta + (int64_t)(g0 + min(gid, kg - 1)) * beta_stride + 2 * tig;
-        const bool bv = gid < kg;                                     // padding columns multiply zeros
-        double c[4][2] = {};
-#pragma unroll 2
-        for (int c0 = 0; c0 < P; c0 += 8) {
-            const bool cv = c0 + 2 * tig < P;
-            double2 a[4];
-#pragma unroll
-            for (int rb = 0; rb < 4; ++rb)
-                a[rb] = (cv && rv[rb]) ? __ldg(reinterpret_cast<const double2 *>(base + (size_t)(8 * rb) * P + c0))
-                                       : make_double2(0.0, 0.0);
-            const bool bl = cv && bv;
-            const double b0 = bl ? __ldg(bc + c0) : 0.0, b1 = bl ? __ldg(bc + c0 + 1) : 0.0;
-#pragma unroll
-            for (int rb = 0; rb < 4; ++rb) {
-                dmma884(c[rb][0], c[rb][1], a[rb].x, b0);
-                dmma884(c[rb][0], c[rb][1], a[rb].y, b1);
-            }
-        }
-        __syncwarp();                                                // the previous item's reads of the tile are done
-#pragma unroll
-        for (int rb = 0; rb < 4; ++rb) {
-            pt[(8 * rb + gid) * kMlogitTileLd + 2 * tig] = c[rb][0];
-            pt[(8 * rb + gid) * kMlogitTileLd + 2 * tig + 1] = c[rb][1];
-        }
-        __syncwarp();
+        shared_rows_tile(pt, tX, beta, beta_stride, g0, kg, i0, N, P, lane);
         for (int k = 0; k < kg; ++k) {
             const int ch = g0 + k;
             // the next chain's loads are in flight while this chain's epilogue runs
@@ -383,13 +398,42 @@ k_mlogit_psi_shared(double *XB, const double *__restrict__ tX, const double *__r
             mnext.E += UN; mnext.XB += UN; mnext.c += N; mnext.eta += N;
             double en[kMlogitMaxU], xn;
             mlogit_next_load(en, xn, mnext, k + 1 < kg ? i : N, N);
-            mlogit_next_epilogue(XB + ch * UN + (int64_t)mn.j * N, m, pt[lane * kMlogitTileLd + k], ek, xbn, i, N,
+            mlogit_next_epilogue(XB + ch * UN + (int64_t)mn.j * N, m, pt[lane * kGroupTileLd + k], ek, xbn, i, N,
                                  (int)(ch * N + i), (int)(chains * N), lane);
             m = mnext;
 #pragma unroll
             for (int u = 0; u < kMlogitMaxU; ++u) ek[u] = en[u];
             xbn = xn;
         }
+    }
+}
+
+// ---------------------------------------------------------------------------------
+// psi = X beta + shift for `chains` chains on ONE set of rows (bl_nb_multichain; even P, 16-byte aligned X): the
+// MMAs of k_xbeta_mma with the beta of 8 chains in the 8 B columns, so one read of X gives psi of 8 chains, each
+// element formed from its own row and column only (the single chain's bits).  The warp's 32 x 8 tile goes through
+// shared memory and lane l stores row i0 + l of each chain in turn: every chain's psi is written in 256-byte runs.
+// Chain c meets beta + c beta_stride and writes psi + c N.  More than 8 chains: further groups of 8.
+// ---------------------------------------------------------------------------------
+static __global__ void __launch_bounds__(256, 2)
+k_xbeta_shared(double *__restrict__ psi, const double *__restrict__ tX, const double *__restrict__ beta,
+               int64_t beta_stride, int chains, int64_t N, int P, double shift)
+{
+    BL_PDL_ENTER();
+    __shared__ double tile[8][32 * kGroupTileLd];
+    const int lane = threadIdx.x & 31;
+    double *pt = tile[threadIdx.x >> 5];
+    const int groups = (chains + kGroupChains - 1) / kGroupChains;
+    const int64_t items = ((N + 31) >> 5) * groups;
+    const int64_t warps = (int64_t)gridDim.x * (blockDim.x >> 5);
+    const int64_t wid = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    for (int64_t item = wid; item < items; item += warps) {
+        const int64_t trip = groups > 1 ? item / groups : item;
+        const int g0 = (int)(item - trip * groups) * kGroupChains, kg = min(kGroupChains, chains - g0);
+        const int64_t i0 = trip << 5, i = i0 + lane;
+        shared_rows_tile(pt, tX, beta, beta_stride, g0, kg, i0, N, P, lane);
+        if (i < N)
+            for (int k = 0; k < kg; ++k) psi[(g0 + k) * N + i] = pt[lane * kGroupTileLd + k] + shift;
     }
 }
 
@@ -956,14 +1000,14 @@ k_gram_reduce(double *__restrict__ PP, const double *__restrict__ P0,
 // out_p = sum_i x_i[p] * v_i  (X'v), v_i = c0*v0_i + c1*v1_i*v2_i  (v1/v2 optional).
 // Per-CTA partial sums then a fixed-order reduce (k_xtv_reduce).
 // Batched chains (this kernel and the two below): blockIdx.y = chain, its rows at tX + chain x_stride (N P: rows of
-// its own; 0: rows shared by the chains), its weights at + chain N.
+// its own; 0: rows shared by the chains), its weights at + chain N, its c1_dev coefficient at c1_dev[chain].
 static __global__ void __launch_bounds__(256)
 k_xtv_partial(double *__restrict__ part, const double *__restrict__ tX, int64_t x_stride, const double *__restrict__ v0,
               double c0, const double *__restrict__ v1, const double *__restrict__ v2, double c1,
               int64_t N, int P, const double *__restrict__ c1_dev = nullptr)
 {
     BL_PDL_ENTER();
-    if (c1_dev) c1 = *c1_dev;                  // coefficient produced on the device (NB: log d)
+    if (c1_dev) c1 = c1_dev[blockIdx.y];       // coefficient produced on the device, one per chain (NB: log d)
     tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     if (v0) v0 += (size_t)blockIdx.y * N;
@@ -1005,7 +1049,7 @@ k_xtv_mma(double *__restrict__ part, const double *__restrict__ tX, int64_t x_st
           int64_t N, int P, const double *__restrict__ c1_dev)
 {
     BL_PDL_ENTER();
-    if (c1_dev) c1 = *c1_dev;
+    if (c1_dev) c1 = c1_dev[blockIdx.y];
     tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     if (v0) v0 += (size_t)blockIdx.y * N;
@@ -1088,7 +1132,7 @@ k_xtv_stream(double *__restrict__ part, const double *__restrict__ tX, int64_t x
     BL_PDL_ENTER();
     constexpr int L = 1 << kLog2L, P = 2 * L;            // column pairs per row, columns
     constexpr int kQ = L > 32 ? L / 32 : 1;              // column pairs a lane rotates through
-    if (c1_dev) c1 = *c1_dev;
+    if (c1_dev) c1 = c1_dev[blockIdx.y];
     tX += (size_t)blockIdx.y * x_stride;
     part += (size_t)blockIdx.y * gridDim.x * P;
     extern __shared__ double sacc[];                     // [warps][P]
@@ -1212,6 +1256,10 @@ static __global__ void k_shape_add(double *__restrict__ out, const double *__res
 // k_nb_df_partial: per-CTA sums of the two N-term series for d and the proposal (fixed order);
 // k_nb_df_decide: one warp adds them up, adds the G series, applies the Metropolis test with the
 // stream's second uniform and publishes d, log d (and the recorded draw).
+// Several chains on shared rows (bl_nb_multichain): chain c reads phi + c N, its d at dptr[c] and log d at
+// ldptr[c], draws from the Metropolis stream of seed + c and owns partials [c][gridDim.x][4]; the partial kernels
+// take the chain as blockIdx.y, the decide kernels one warp per chain (blockIdx.x), and k_nb_prepare blockIdx.y.
+// One chain: the single chain's layout (d, log d side by side) and summation order.
 // ---------------------------------------------------------------------------------
 constexpr uint64_t kDfObs = 0xFFFFFFFFFFFFFFFEull;
 
@@ -1232,7 +1280,9 @@ k_nb_df_partial(double *__restrict__ part, const double *__restrict__ phi, const
                 const double *__restrict__ dptr, int64_t N, uint64_t seed, uint32_t call)
 {
     __shared__ double red[8][4];
-    const double d = *dptr, dp = nb_df_proposal(d, seed, call, nullptr);
+    phi += blockIdx.y * N;
+    part += (size_t)blockIdx.y * gridDim.x * 4;
+    const double d = dptr[blockIdx.y], dp = nb_df_proposal(d, seed + blockIdx.y, call, nullptr);
     const double ld = log(d), ldp = log(dp);
     double s[4] = {0.0, 0.0, 0.0, 0.0};
     const int64_t slab = (N + gridDim.x - 1) / gridDim.x;
@@ -1277,12 +1327,13 @@ static __global__ void k_nb_df_fold(double *__restrict__ sum4, const double *__r
 
 static __global__ void k_nb_df_decide(double *__restrict__ dptr, double *__restrict__ ldptr, double *__restrict__ d_rec,
                                const double *__restrict__ part, int nblk, const double *__restrict__ G, int ymax,
-                               uint64_t seed, uint32_t call)
+                               uint64_t seed, uint32_t call, int64_t rec_stride = 0)
 {
-    const int lane = threadIdx.x;
-    const double d = *dptr;
+    const int lane = threadIdx.x, ch = blockIdx.x;
+    part += (size_t)ch * nblk * 4;
+    const double d = dptr[ch];
     double u_acc;
-    const double dp = nb_df_proposal(d, seed, call, &u_acc);
+    const double dp = nb_df_proposal(d, seed + ch, call, &u_acc);
     double s[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
     for (int b = lane; b < nblk; b += 32)
         for (int k = 0; k < 4; ++k) s[k] += part[(size_t)b * 4 + k];
@@ -1298,9 +1349,9 @@ static __global__ void k_nb_df_decide(double *__restrict__ dptr, double *__restr
         double llh_prop = s[5] + dp * s[2] + s[3];
         double lppsl = log(dp == 1.0 ? 0.5 : 1.0 / 3.0) - log(d == 1.0 ? 0.5 : 1.0 / 3.0);
         double dn = u_acc < exp(llh_prop - llh_prev + lppsl) ? dp : d;
-        *dptr = dn;
-        *ldptr = log(dn);
-        if (d_rec) *d_rec = dn;
+        dptr[ch] = dn;
+        ldptr[ch] = log(dn);
+        if (d_rec) d_rec[ch * rec_stride] = dn;
     }
 }
 
@@ -1324,7 +1375,9 @@ k_nb_dfreal_partial(double *__restrict__ part, const double *__restrict__ phi, c
                     const double *__restrict__ dptr, int64_t N, uint64_t seed, uint32_t call)
 {
     __shared__ double red[8][2];
-    const double r = *dptr, rs = nb_dfreal_proposal(r, seed, call, nullptr);
+    phi += blockIdx.y * N;
+    part += (size_t)blockIdx.y * gridDim.x * 4;
+    const double r = dptr[blockIdx.y], rs = nb_dfreal_proposal(r, seed + blockIdx.y, call, nullptr);
     const double lgr = lgamma(r), lgs = lgamma(rs), lr = log(r), ls = log(rs);
     double s0 = 0.0, s1 = 0.0;
     const int64_t slab = (N + gridDim.x - 1) / gridDim.x;
@@ -1348,20 +1401,22 @@ k_nb_dfreal_partial(double *__restrict__ part, const double *__restrict__ phi, c
 }
 
 static __global__ void k_nb_dfreal_decide(double *__restrict__ dptr, double *__restrict__ ldptr, double *__restrict__ d_rec,
-                                          const double *__restrict__ part, int nblk, uint64_t seed, uint32_t call)
+                                          const double *__restrict__ part, int nblk, uint64_t seed, uint32_t call,
+                                          int64_t rec_stride = 0)
 {
-    const int lane = threadIdx.x;
-    const double r = *dptr;
+    const int lane = threadIdx.x, ch = blockIdx.x;
+    part += (size_t)ch * nblk * 4;
+    const double r = dptr[ch];
     double lu;
-    const double rs = nb_dfreal_proposal(r, seed, call, &lu);
+    const double rs = nb_dfreal_proposal(r, seed + ch, call, &lu);
     double s0 = 0.0, s1 = 0.0;
     for (int b = lane; b < nblk; b += 32) { s0 += part[(size_t)b * 4]; s1 += part[(size_t)b * 4 + 2]; }
     for (int o = 16; o; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); }
     if (lane == 0) {
         const double dn = lu < s1 - s0 ? rs : r;
-        *dptr = dn;
-        *ldptr = log(dn);
-        if (d_rec) *d_rec = dn;
+        dptr[ch] = dn;
+        ldptr[ch] = log(dn);
+        if (d_rec) d_rec[ch * rec_stride] = dn;
     }
 }
 
@@ -1372,10 +1427,11 @@ static __global__ void k_nb_prepare(double *__restrict__ psi, double *__restrict
 {
     int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
-    const double d = *dptr, ld = *ldptr;
-    psi[i] -= ld;
-    shape[i] = y[i] + d;
-    kappa[i] = 0.5 * (y[i] - d);
+    const double d = dptr[blockIdx.y], ld = ldptr[blockIdx.y];
+    const int64_t k = blockIdx.y * N + i;
+    psi[k] -= ld;
+    shape[k] = y[i] + d;
+    kappa[k] = 0.5 * (y[i] - d);
 }
 
 // ymax and G[j] = #{y_i > j} (NBPG-logmean.R:65-67)

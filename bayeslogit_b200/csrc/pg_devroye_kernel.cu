@@ -18,6 +18,7 @@
 
 #include "engine.h"
 #include "pg_devroye_fast.cuh"
+#include "pg_stream.cuh"
 
 namespace bl {
 
@@ -174,16 +175,6 @@ struct DrSlots {
     int wcnt[kDrThreads / 32][3];
 };
 
-__device__ __forceinline__ void dr_open(PhiloxSource &src, const StreamId &id, int obs)
-{
-    if (id.chain_len) {
-        const uint32_t ch = (uint32_t)obs / id.chain_len;
-        src.open(id.seed + ch, id.obs0 + ((uint32_t)obs - ch * id.chain_len), id.call_id);
-    } else {
-        src.open(id.seed, id.obs0 + (uint64_t)obs, id.call_id);
-    }
-}
-
 __global__ void __launch_bounds__(kDrThreads)
 k_devroye_regroup(double *__restrict__ x, const int *__restrict__ n, const double *__restrict__ z, int num, StreamId id)
 {
@@ -214,7 +205,7 @@ k_devroye_regroup(double *__restrict__ x, const int *__restrict__ n, const doubl
                 } else {
                     DevSetup st = dev_setup(z[obs]);
                     PhiloxSource src;
-                    dr_open(src, id, obs);
+                    open_batch_stream(src, id, obs);
                     S.phase[t] = dev_pick(src, st);
                     S.Z[t] = st.Z;
                     S.pr32[t] = st.pr32;
@@ -260,7 +251,7 @@ k_devroye_regroup(double *__restrict__ x, const int *__restrict__ n, const doubl
             const int sl = S.perm[t];
             const int obs = S.obs[sl];
             PhiloxSource src;
-            dr_open(src, id, obs);
+            open_batch_stream(src, id, obs);
             src.buf = S.buf[sl];
             src.blk = S.blk[sl];
             src.pos = S.pos[sl];

@@ -28,6 +28,7 @@
 
 #include "engine.h"
 #include "pg_devroye_fast.cuh"
+#include "pg_stream.cuh"
 
 namespace bl {
 
@@ -123,7 +124,9 @@ k_hyb_scatter(const double *__restrict__ h, int n, int *__restrict__ meta, int *
     }
 }
 
-template <int R>
+// kChains: the batch holds independent chains side by side and id.chain_len keys their streams (open_batch_stream); a
+// compile-time switch, so that the single-batch instantiations keep their code.
+template <int R, bool kChains = false>
 __global__ void __launch_bounds__(128)
 k_hyb_regime(double *__restrict__ x, const double *__restrict__ h, const double *__restrict__ z,
              const int *__restrict__ idx, const int *__restrict__ meta, StreamId id)
@@ -133,7 +136,8 @@ k_hyb_regime(double *__restrict__ x, const double *__restrict__ h, const double 
     for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < count; j += gridDim.x * blockDim.x) {
         int i = list[j];
         PhiloxSource s;
-        s.open(id.seed, id.obs0 + (uint64_t)i, id.call_id);
+        if (kChains) open_batch_stream(s, id, i);
+        else s.open(id.seed, id.obs0 + (uint64_t)i, id.call_id);
         double b = h[i], zi = z[i], v;
         if (R == kRegNormal) {
             double m = pg_m1(b, zi);
@@ -293,7 +297,7 @@ struct AltRegroup {
     }
 };
 
-template <class R>
+template <class R, bool kChains = false>
 __global__ void __launch_bounds__(kRgThreads)
 k_loop_regroup(double *__restrict__ x, const double *__restrict__ h, const double *__restrict__ z,
                const int *__restrict__ idx, const int *__restrict__ meta, const double *__restrict__ state,
@@ -329,7 +333,8 @@ k_loop_regroup(double *__restrict__ x, const double *__restrict__ h, const doubl
                 for (int k = 0; k < R::F; ++k) S.f[k][t] = __ldg(state + (size_t)k * cap + cand);
                 S.obs[t] = obs;
                 PhiloxSource src;
-                src.open(id.seed, id.obs0 + (uint64_t)obs, id.call_id);
+                if (kChains) open_batch_stream(src, id, obs);
+                else src.open(id.seed, id.obs0 + (uint64_t)obs, id.call_id);
                 R::begin(S, t, h[obs], z[obs], src);
                 S.buf[t] = src.buf;
                 S.blk[t] = src.blk;
@@ -370,7 +375,8 @@ k_loop_regroup(double *__restrict__ x, const double *__restrict__ h, const doubl
         if (t < tot1 + tot3 || t >= kRgThreads - tot2) {
             const int sl = S.perm[t];
             PhiloxSource src;
-            src.open(id.seed, id.obs0 + (uint64_t)S.obs[sl], id.call_id);
+            if (kChains) open_batch_stream(src, id, S.obs[sl]);
+            else src.open(id.seed, id.obs0 + (uint64_t)S.obs[sl], id.call_id);
             src.buf = S.buf[sl];
             src.blk = S.blk[sl];
             src.pos = S.pos[sl];
@@ -388,13 +394,13 @@ k_loop_regroup(double *__restrict__ x, const double *__restrict__ h, const doubl
     }
 }
 
-template <class R>
+template <class R, bool kChains>
 int regroup_grid()
 {
     using Slots = typename R::Slots;
-    cudaFuncSetAttribute(k_loop_regroup<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Slots));
+    cudaFuncSetAttribute(k_loop_regroup<R, kChains>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Slots));
     int per_sm = 0;
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_loop_regroup<R>, kRgThreads, sizeof(Slots)) != cudaSuccess || per_sm < 1)
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_loop_regroup<R, kChains>, kRgThreads, sizeof(Slots)) != cudaSuccess || per_sm < 1)
         per_sm = 1;
     int sms = 148, dev = 0;
     if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -445,13 +451,13 @@ int resident_grid(K kernel, int threads, int need)
     return need < cap ? (need > 0 ? need : 1) : cap;
 }
 
-template <int R>
+template <int R, bool kChains>
 void launch_regime(double *x, const double *h, const double *z, const int *idx, const int *meta,
                    StreamId id, int n, cudaStream_t st)
 {
-    static const int cap = resident_grid(k_hyb_regime<R>, 128, 1 << 30);
+    static const int cap = resident_grid(k_hyb_regime<R, kChains>, 128, 1 << 30);
     int need = (n + 127) / 128;
-    k_hyb_regime<R><<<need < cap ? need : cap, 128, 0, st>>>(x, h, z, idx, meta, id);
+    k_hyb_regime<R, kChains><<<need < cap ? need : cap, 128, 0, st>>>(x, h, z, idx, meta, id);
     count_launch();
 }
 
@@ -530,10 +536,9 @@ struct SideStream {
 };
 static SideStream g_side;
 
-// One rpg_hybrid batch of at most 2^31-1 observations.  `work` holds
-// hybrid_workspace_bytes(num) bytes of device scratch owned by the caller's stream.
-cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, int num, StreamId id,
-                                 void *work, cudaStream_t st)
+template <bool kChains>
+static cudaError_t launch_hybrid_binned_k(double *x, const double *h, const double *z, int num, StreamId id,
+                                          void *work, cudaStream_t st)
 {
     if (num <= 0) return cudaSuccess;
     int *meta = (int *)work;
@@ -564,22 +569,22 @@ cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, in
     }
     {
         HybTimer t(tm, side, kStGamma);
-        launch_regime<kRegGamma>(x, h, z, idx, meta, id, num, side);
+        launch_regime<kRegGamma, kChains>(x, h, z, idx, meta, id, num, side);
     }
     {
         HybTimer t(tm, side, kStNormal);
-        launch_regime<kRegNormal>(x, h, z, idx, meta, id, num, side);
+        launch_regime<kRegNormal, kChains>(x, h, z, idx, meta, id, num, side);
     }
     {
         HybTimer t(tm, side, kStDevroye);
-        launch_regime<kRegDevroye>(x, h, z, idx, meta, id, num, side);
+        launch_regime<kRegDevroye, kChains>(x, h, z, idx, meta, id, num, side);
     }
     double *state = (double *)((char *)work + hybrid_state_offset(num));
     const int cap = num < kStateChunk ? num : kStateChunk;
     static const int g_sp_setup = resident_grid(k_sp_setup, 128, 1 << 30);
     static const int g_alt_setup = resident_grid(k_alt_setup, 128, 1 << 30);
-    static const int g_sp_regroup = regroup_grid<SpRegroup>();
-    static const int g_alt_regroup = regroup_grid<AltRegroup>();
+    static const int g_sp_regroup = regroup_grid<SpRegroup, kChains>();
+    static const int g_alt_regroup = regroup_grid<AltRegroup, kChains>();
     const int rneed = (cap + kLaneChunk * (kRgThreads / 32) - 1) / (kLaneChunk * (kRgThreads / 32));
     const int sneed = (cap + 127) / 128;
     // One set-up/loop pair per state chunk.  The regime counts live on the device, so pairs are
@@ -591,7 +596,7 @@ cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, in
         }
         {
             HybTimer t(tm, st, kStSpLoop);
-            k_loop_regroup<SpRegroup><<<std::min(rneed, g_sp_regroup), kRgThreads, sizeof(SpRegroup::Slots), st>>>(x, h, z, idx, meta, state, c0, cap, id);
+            k_loop_regroup<SpRegroup, kChains><<<std::min(rneed, g_sp_regroup), kRgThreads, sizeof(SpRegroup::Slots), st>>>(x, h, z, idx, meta, state, c0, cap, id);
         }
         count_launch(2);
     }
@@ -602,7 +607,7 @@ cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, in
         }
         {
             HybTimer t(tm, st, kStAltLoop);
-            k_loop_regroup<AltRegroup><<<std::min(rneed, g_alt_regroup), kRgThreads, sizeof(AltRegroup::Slots), st>>>(x, h, z, idx, meta, state, c0, cap, id);
+            k_loop_regroup<AltRegroup, kChains><<<std::min(rneed, g_alt_regroup), kRgThreads, sizeof(AltRegroup::Slots), st>>>(x, h, z, idx, meta, state, c0, cap, id);
         }
         count_launch(2);
     }
@@ -611,6 +616,15 @@ cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, in
         cudaStreamWaitEvent(st, g_side.join, 0);
     }
     return cudaGetLastError();
+}
+
+// One rpg_hybrid batch of at most 2^31-1 observations.  `work` holds
+// hybrid_workspace_bytes(num) bytes of device scratch owned by the caller's stream.
+cudaError_t launch_hybrid_binned(double *x, const double *h, const double *z, int num, StreamId id,
+                                 void *work, cudaStream_t st)
+{
+    return id.chain_len ? launch_hybrid_binned_k<true>(x, h, z, num, id, work, st)
+                        : launch_hybrid_binned_k<false>(x, h, z, num, id, work, st);
 }
 
 }  // namespace bl

@@ -7,6 +7,7 @@
 // pipes, not by HBM (DESIGN.md "Rooflines").
 #include "engine.h"
 #include "pg_devroye_fast.cuh"
+#include "pg_stream.cuh"
 
 namespace bl {
 
@@ -53,7 +54,9 @@ __device__ __forceinline__ double draw_one(Src &s, const void *shape, const doub
     }
 }
 
-template <int M>
+// kChains: the batch holds independent chains side by side and id.chain_len keys their streams (open_batch_stream;
+// batch < 2^31); a compile-time switch, so that the single-batch instantiations keep their code.
+template <int M, bool kChains = false>
 __global__ void __launch_bounds__(kThreads)
 k_rpg_philox(double *__restrict__ x, const void *__restrict__ shape, const double *__restrict__ z,
              int64_t num, int trunc, int *__restrict__ iter, StreamId id)
@@ -61,7 +64,8 @@ k_rpg_philox(double *__restrict__ x, const void *__restrict__ shape, const doubl
     int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < num; i += stride) {
         PhiloxSource s;
-        s.open(id.seed, id.obs0 + (uint64_t)i, id.call_id);
+        if (kChains) open_batch_stream(s, id, i);
+        else s.open(id.seed, id.obs0 + (uint64_t)i, id.call_id);
         int aux;
         x[i] = draw_one<M>(s, shape, z, i, trunc, iter, aux);
     }
@@ -146,12 +150,12 @@ __global__ void k_probe_philox(uint32_t *out4, const uint32_t *ctr4, const uint3
     out4[0] = r.x; out4[1] = r.y; out4[2] = r.z; out4[3] = r.w;
 }
 
-template <int M>
+template <int M, bool kChains = false>
 cudaError_t launch_philox_m(double *x, const void *shape, const double *z, int64_t num, int trunc,
                             int *iter, StreamId id, cudaStream_t st)
 {
     if (num <= 0) return cudaSuccess;
-    k_rpg_philox<M><<<grid_for(num, kThreads, 16), kThreads, 0, st>>>(x, shape, z, num, trunc, iter, id);
+    k_rpg_philox<M, kChains><<<grid_for(num, kThreads, 16), kThreads, 0, st>>>(x, shape, z, num, trunc, iter, id);
     count_launch();
     return cudaGetLastError();
 }
@@ -177,7 +181,9 @@ cudaError_t launch_rpg(Method m, double *x, const void *shape, const double *z, 
     case kGamma: return launch_philox_m<kGamma>(x, shape, z, num, trunc, iter, id, st);
     case kAlt: return launch_philox_m<kAlt>(x, shape, z, num, trunc, iter, id, st);
     case kSP: return launch_philox_m<kSP>(x, shape, z, num, trunc, iter, id, st);
-    case kHybrid: return launch_philox_m<kHybrid>(x, shape, z, num, trunc, iter, id, st);
+    case kHybrid:
+        return id.chain_len ? launch_philox_m<kHybrid, true>(x, shape, z, num, trunc, iter, id, st)
+                            : launch_philox_m<kHybrid>(x, shape, z, num, trunc, iter, id, st);
     case kDevroyePlain: return launch_philox_m<kDevroyePlain>(x, shape, z, num, trunc, iter, id, st);
     }
     return cudaErrorInvalidValue;

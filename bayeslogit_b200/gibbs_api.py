@@ -295,3 +295,26 @@ def nb_gibbs_df(y, X, m0, P0, samp, burn, seed, d0=1.0, real_d=False):
     _lib.check(st)
     return w, beta, d
 
+
+NB_DMODES = {"fixed": 0, "int": 1, "real": 2}     # BL_NB_D_FIXED, BL_NB_D_INT, BL_NB_D_REAL
+
+
+def nb_multichain(y, X, m0, P0, samp, burn, seed, chains, d0=1.0, dmode="int"):
+    """`chains` independent NB chains on one data set: y [N], X [N x P], m0, P0 shared by all chains.  dmode "int":
+    chain c is, bit for bit, nb_gibbs_df(..., seed=seed + c)'s beta and d; "real": the same with real_d=True; "fixed":
+    d = d0 throughout, beta is rows burn .. burn + samp - 1 of nb_gibbs(..., samp + burn, seed=seed + c) (d is d0).
+    X is held once and read once per iteration for up to 8 chains.  Returns (beta [chains x samp x P],
+    d [chains x samp])."""
+    if dmode not in NB_DMODES:
+        raise ValueError("dmode must be one of %s" % ", ".join(map(repr, NB_DMODES)))
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    N, P = X.shape
+    y, m0 = _f(y).ravel(), _f(m0).ravel()
+    P0c = np.asfortranarray(_f(P0))
+    K = max(int(chains), 0)
+    beta = np.zeros((K, samp, P))
+    d = np.zeros((K, samp))
+    st = _lib.lib().bl_nb_multichain(_p(beta), _p(d), _p(y), _p(X), float(d0), _p(m0), P0c.ctypes.data, int(chains),
+                                     N, P, samp, burn, int(seed), NB_DMODES[dmode])
+    _lib.check(st)
+    return beta, d

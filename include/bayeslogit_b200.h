@@ -264,7 +264,7 @@ int bl_logit_multichain_dev(double *beta, const double *y, const double *tX, con
  * once per category update for up to 8 chains; the launches per iteration do not depend on the number of chains.
  * flags: 0 or BL_GIBBS_UNFUSED (separate psi and offsets kernels in every category update: the chains then equal
  * the single chain run with BL_MLOGIT_UNFUSED=1 in the environment); any other flag is refused.  Limits, checked
- * before anything is allocated: chains >= 1, J >= 2, chains * N < 2^31, P <= 111 (each chain's beta is drawn by one
+ * before anything is allocated: 1 <= chains <= 65535, J >= 2, chains * N < 2^31, P <= 111 (each chain's beta is drawn by one
  * CTA out of shared memory; the single-chain entry takes P <= 256).  Device memory beyond the data: 2 chains (J-1)
  * N doubles of linear predictors and their exponentials, and 32 bytes per (chain, row) of offsets, tilts, draws,
  * shapes and the draw's index list.  Duplicate rows are not
@@ -275,6 +275,28 @@ int bl_mlogit_multichain(double *beta, const double *ty, const double *tX, const
 int bl_mlogit_multichain_dev(double *beta, const double *ty, const double *tX, const double *n, const double *m0,
                              const double *P0, int chains, int64_t N, int P, int J, int samp, int burn, uint64_t seed,
                              int flags, void *stream);
+
+/* Several independent negative-binomial chains on ONE data set (the NB counterpart of bl_logit_multichain; R-hat on
+ * the dispersion d is the usual first check).  y: counts [N], tX: P x N, shared by all chains with m0 / P0.
+ * dmode picks the chain every chain runs:
+ *   BL_NB_D_FIXED  d = d0 throughout: chain c's beta is rows burn .. burn + samp - 1 of
+ *                  bl_nb_gibbs(..., samp + burn, seed + c), bit for bit (d_out, if given, is filled with d0);
+ *   BL_NB_D_INT    draw.df on the integers: chain c's beta and d are bl_nb_gibbs_df(..., seed + c), bit for bit;
+ *   BL_NB_D_REAL   draw.df.real.mean: chain c's beta and d are bl_nb_gibbs_dfreal(..., seed + c), bit for bit.
+ * beta: [chains][samp][P]; d_out: [chains][samp] or NULL; omega is not returned.  X is held once and read once per
+ * iteration for up to 8 chains; the launches per iteration do not depend on the number of chains.  Limits, checked
+ * before anything is allocated or launched: 1 <= chains <= 65535, chains * N < 2^31, P <= 256, d0 as the matching
+ * single-chain entry takes it.  Spread the chains over GPUs by giving each rank the whole data set and a block of
+ * chains, called with seed + first chain of the block.  The host entry copies y and X to the device once. */
+#define BL_NB_D_FIXED 0   /* d = d0 throughout: the chain of bl_nb_gibbs */
+#define BL_NB_D_INT   1   /* draw.df on the integers: the chain of bl_nb_gibbs_df */
+#define BL_NB_D_REAL  2   /* draw.df.real.mean: the chain of bl_nb_gibbs_dfreal */
+int bl_nb_multichain(double *beta, double *d_out, const double *y, const double *tX, double d0,
+                     const double *m0, const double *P0, int chains, int N, int P, int samp, int burn,
+                     uint64_t seed, int dmode);
+int bl_nb_multichain_dev(double *beta, double *d_out, const double *y, const double *tX, double d0,
+                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
+                         uint64_t seed, int dmode, void *stream);
 
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */

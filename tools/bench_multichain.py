@@ -3,6 +3,7 @@
 
     python tools/bench_multichain.py [--N 1000000 --P 64 --chains 1,2,4,8 --iters 20 --reps 3]
     python tools/bench_multichain.py --model mlogit [--N 1000000 --P 32 --J 10 --chains 1,2,4,8 --iters 20 --reps 3]
+    python tools/bench_multichain.py --model nb [--dmode int|real|fixed --N 1000000 --P 64 --chains 1,2,4,8 ...]
 
 For every chain count K and both beta draws, three arms are timed alternately in the same process, on the same
 device-resident data, and reported as ms per iteration of all K chains (median over the repetitions):
@@ -19,6 +20,14 @@ the default size, larger than L2, so every pass reads it from HBM.  Prints one J
 Chain c of (a) must equal call c of (b) bit for bit (max_abs_diff_a_b).  Also reported: the stage split of the last
 category update of both arms and the kernel launches per iteration (bl_kernel_launches over a timed call / its
 iterations).  X is 256 MB at the default size (N = 1M, P = 32).
+
+--model nb: negative-binomial chains (bl_nb_multichain) with the dispersion walk of --dmode, two arms alternated the
+same way:
+  (a) multichain: bl_nb_multichain_dev, one copy of X shared by the K chains;
+  (b) sequential: K calls of bl_nb_gibbs_df_dev / bl_nb_gibbs_dfreal_dev / bl_nb_gibbs_dev with seed + c.
+Both arms run without burn-in, so chain c of (a) must equal call c of (b) bit for bit, beta and d
+(max_abs_diff_a_b).  Also reported: the multichain stage split of the last iteration and the kernel launches per
+iteration.  Counts have mean ~ 100 (b = y + d mostly in the saddle-point range, as BASELINE config 4).
 """
 import argparse
 import json
@@ -213,11 +222,89 @@ def run_mlogit(N, P, J, ks, iters, reps):
     return out
 
 
+def run_nb(N, P, dmode, ks, iters, reps):
+    import torch
+    from bayeslogit_b200 import _lib
+    L = _lib.lib()
+    dev = torch.device("cuda")
+    g = torch.Generator(device=dev); g.manual_seed(20240013)
+    X = torch.randn(N, P, generator=g, device=dev, dtype=torch.float64) / P ** 0.5
+    X[:, P - 1] = 1.0
+    bt = torch.randn(P, generator=g, device=dev, dtype=torch.float64) * 0.5
+    bt[P - 1] = 4.6                                      # mean count ~ 100
+    d_true = 10.0
+    mu = torch.exp(X @ bt)
+    torch.manual_seed(20240013)                          # the gamma draw below takes the global generator
+    lam = torch.distributions.Gamma(torch.full_like(mu, d_true), d_true / mu).sample()     # NB = Poisson-gamma mix
+    y = torch.poisson(lam, generator=g).contiguous()
+    m0 = torch.zeros(P, device=dev, dtype=torch.float64)
+    P0 = (0.01 * torch.eye(P, device=dev, dtype=torch.float64)).contiguous()
+    st = torch.cuda.current_stream().cuda_stream
+    seed = 20240013
+    code = {"fixed": 0, "int": 1, "real": 2}[dmode]
+    d0 = 10.0 if dmode == "fixed" else 3.0
+    out = {"model": "nb", "dmode": dmode, "N": N, "P": P, "d0": d0, "iters": iters, "reps": reps, "results": []}
+
+    for K in ks:
+        def multichain(k):
+            beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+            d = torch.zeros(K, k, device=dev, dtype=torch.float64)
+            _lib.check(L.bl_nb_multichain_dev(beta.data_ptr(), d.data_ptr(), y.data_ptr(), X.data_ptr(), d0,
+                                              m0.data_ptr(), P0.data_ptr(), K, N, P, k, 0, seed, code, st))
+            return beta, d
+
+        def sequential(k):
+            beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+            d = torch.full((K, k), d0, device=dev, dtype=torch.float64)
+            for c in range(K):
+                if dmode == "fixed":
+                    rc = L.bl_nb_gibbs_dev(None, beta[c].data_ptr(), y.data_ptr(), X.data_ptr(), d0, m0.data_ptr(),
+                                           P0.data_ptr(), N, P, k, seed + c, 0, st)
+                else:
+                    fn = L.bl_nb_gibbs_dfreal_dev if dmode == "real" else L.bl_nb_gibbs_df_dev
+                    rc = fn(None, beta[c].data_ptr(), d[c].data_ptr(), y.data_ptr(), X.data_ptr(), d0, m0.data_ptr(),
+                            P0.data_ptr(), N, P, k, 0, seed + c, 0, st)
+                _lib.check(rc)
+            return beta, d
+
+        arms = {"multichain": multichain, "sequential": sequential}
+        for fn in arms.values():                         # warm-up: modules, pools, every kernel of the timed window
+            fn(2)
+        torch.cuda.synchronize()
+        times = {a: [] for a in arms}
+        launches = {}
+        res = {}
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        for _ in range(reps):
+            for a, fn in arms.items():                   # alternated: drifts of the shared machine hit every arm
+                l0 = L.bl_kernel_launches()
+                e0.record()
+                res[a] = fn(iters)
+                e1.record()
+                torch.cuda.synchronize()
+                launches[a] = (L.bl_kernel_launches() - l0) / iters
+                times[a].append(e0.elapsed_time(e1) / iters)
+        med = {a: sorted(v)[len(v) // 2] for a, v in times.items()}
+        diff = max(float((res["multichain"][i] - res["sequential"][i]).abs().max().item()) for i in (0, 1))
+        out["results"].append({
+            "chains": K,
+            "ms_per_iteration_of_all_chains": med,
+            "ms_all_reps": times,
+            "sequential_over_multichain": med["sequential"] / med["multichain"],
+            "max_abs_diff_a_b": diff,
+            "d_moves": bool((res["multichain"][1] != res["multichain"][1][:, :1]).any().item()),
+            "launches_per_iteration": launches,
+            "stages_us": {"multichain": stage_split(lambda: multichain(2))},
+        })
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--model", choices=["logit", "mlogit"], default="logit")
+    ap.add_argument("--model", choices=["logit", "mlogit", "nb"], default="logit")
+    ap.add_argument("--dmode", choices=["int", "real", "fixed"], default="int", help="dispersion walk (nb)")
     ap.add_argument("--N", type=int, default=1_000_000)
-    ap.add_argument("--P", type=int, default=None, help="default 64 (logit), 32 (mlogit)")
+    ap.add_argument("--P", type=int, default=None, help="default 64 (logit, nb), 32 (mlogit)")
     ap.add_argument("--J", type=int, default=10, help="categories (mlogit)")
     ap.add_argument("--chains", default="1,2,4,8")
     ap.add_argument("--iters", type=int, default=20)
@@ -230,6 +317,8 @@ def main():
     ks = [int(k) for k in a.chains.split(",")]
     if a.model == "mlogit":
         out = run_mlogit(a.N, a.P or 32, a.J, ks, a.iters, a.reps)
+    elif a.model == "nb":
+        out = run_nb(a.N, a.P or 64, a.dmode, ks, a.iters, a.reps)
     else:
         out = run(a.N, a.P or 64, ks, a.iters, a.reps)
     out["device"] = name
