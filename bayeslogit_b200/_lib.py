@@ -114,6 +114,7 @@ def lib():
     L.bl_probe_v_eval.argtypes = [vp, vp, i64]
     L.bl_probe_specfun.argtypes = [vp, ci, vp, vp, vp, i64]
     L.bl_probe_philox.argtypes = [vp, vp, vp]
+    L.bl_probe_nb_dispersion.argtypes = [vp, vp, vp, vp, ci, i64, u64, u32, ci]
     L.bl_probe_peaks.argtypes = [vp]
     L.bl_hybrid_timing.argtypes = [ci]
     L.bl_hybrid_timing_last.argtypes = [vp, vp]

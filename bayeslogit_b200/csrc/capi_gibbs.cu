@@ -358,6 +358,29 @@ int bl_nb_gibbs_dfreal_dev(double *w_last, double *beta, double *d_out, const do
     return 0;
 }
 
+int bl_probe_nb_dispersion(double *out, const double *phi, const double *y, const double *d, int chains, int64_t N,
+                           uint64_t seed, uint32_t call, int real_d)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!out || !phi || !y || !d) return report("probe_nb_dispersion: null argument", nullptr);
+    if (chains < 1 || chains > 65535 || N < 1 || (int64_t)chains * N >= (1LL << 31))
+        return report("probe_nb_dispersion: bad dimensions", nullptr);
+    for (int c = 0; c < chains; ++c)
+        if (real_d ? !(d[c] > 0.0) : (!(d[c] >= 1.0) || d[c] != floor(d[c])))
+            return report(real_d ? "probe_nb_dispersion: d must be positive"
+                                 : "probe_nb_dispersion: d must be a positive integer", nullptr);
+    std::string err;
+    Dev dv;
+    double *dphi = dv.put(phi, (size_t)chains * N, err), *dy = dv.put(y, N, err);
+    double *dout = dv.put(nullptr, (size_t)chains * 5, err);
+    if (!err.empty()) return report(err, nullptr);
+    if (nb_dispersion_probe(dout, dphi, dy, d, chains, N, seed, call, real_d, (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(out, dout, sizeof(double) * (size_t)chains * 5, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
 int bl_nb_gibbs_df_dev(double *w_last, double *beta, double *d_out, const double *y, const double *tX, double d0,
                        const double *m0, const double *P0, int64_t N, int P, int samp, int burn, uint64_t seed,
                        uint64_t obs0, void *stream)

@@ -104,6 +104,8 @@ int nb_multichain_check(int chains, int64_t N, int P, int samp, int burn, double
 int nb_multichain_device(double *beta_out, double *d_out, const double *y, const double *tX, double d0, const double *m0,
                          const double *P0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int dmode,
                          cudaStream_t st, std::string &err);
+int nb_dispersion_probe(double *out, const double *phi, const double *y, const double *d, int chains, int64_t N,
+                        uint64_t seed, uint32_t call, int real_d, cudaStream_t st, std::string &err);
 int logit_em_device(double *beta, const double *y, const double *tX, const double *n, int64_t N,
                     int P, double tol, int max_iter, int *iters, cudaStream_t st, std::string &err);
 // duplicate-row merge on device-resident data (merge.cu); returns M, -1 (CUDA error), -2 (needs the exact host merge)

@@ -1283,6 +1283,8 @@ int nb_gibbs_device(double *w_out, double *beta_out, const double *y, const doub
     return s.check_status(err, "nb_gibbs");
 }
 
+static const char *const kNbBadCountMsg = ": counts y must be finite, non-negative and below 2^31 - 1";
+
 // ------------------------------------------------------------------------------------
 // Negative binomial with the dispersion sampled (NB.PG.gibbs, NBPG-logmean.R:36-113, with
 // draw.df, NB-Shape.R:9-53): per iteration phi = X beta; d | beta by one random-walk
@@ -1328,6 +1330,10 @@ int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const dou
     unsigned long long ymax64 = 0;
     GB_CK(cudaMemcpyAsync(&ymax64, ymax_d, sizeof(ymax64), cudaMemcpyDeviceToHost, st));
     GB_CK(cudaStreamSynchronize(st));
+    if (ymax64 == kNbBadCount) {
+        err = std::string(real_d ? "nb_gibbs_dfreal" : "nb_gibbs_df") + kNbBadCountMsg;
+        return 1;
+    }
     const int ymax = (int)ymax64;
     unsigned long long *hist;
     GB_CK(mem.get(&hist, (size_t)ymax + 2));
@@ -1488,6 +1494,7 @@ int nb_multichain_device(double *beta_out, double *d_out, const double *y, const
         unsigned long long ymax64 = 0;
         GB_CK(cudaMemcpyAsync(&ymax64, ymax_d, sizeof(ymax64), cudaMemcpyDeviceToHost, st));
         GB_CK(cudaStreamSynchronize(st));
+        if (ymax64 == kNbBadCount) { err = std::string("nb_multichain") + kNbBadCountMsg; return 1; }
         ymax = (int)ymax64;
         GB_CK(mem.get(&hist, (size_t)ymax + 2));
         GB_CK(mem.get(&G, (size_t)ymax + 1));
@@ -1587,6 +1594,50 @@ int nb_multichain_device(double *beta_out, double *d_out, const double *y, const
     GB_CK(cudaMemcpyAsync(&h, status, sizeof(int), cudaMemcpyDeviceToHost, st));
     GB_CK(cudaStreamSynchronize(st));
     if (h != 0) { err = "nb_multichain: a chain's posterior precision is not positive definite"; return 1; }
+    return 0;
+}
+
+// One dispersion step of `chains` chains on given phi [chains][N] and d [chains] (host), with the kernels, grids and
+// nblk of nb_gibbs_df_device (chains = 1) and nb_multichain_device: ymax, histogram, G, the N-term partials and the
+// decide kernel, which writes out[c][5] = {d', accept variate (u; real walk: log u), llh(d), llh(d'), new d}.
+// Arguments are checked by the caller (bl_probe_nb_dispersion).
+int nb_dispersion_probe(double *out, const double *phi, const double *y, const double *d, int chains, int64_t N,
+                        uint64_t seed, uint32_t call, int real_d, cudaStream_t st, std::string &err)
+{
+    const int K = chains;
+    const int nblk = (int)std::min<int64_t>(148 * 4, std::max<int64_t>(1, N / 1024));   // as nb_gibbs_df_device
+    DevMem mem;
+    mem.st = st;
+    unsigned long long *ymax_d, *hist;
+    double *G, *dfpart, *dvec;
+    GB_CK(mem.get(&ymax_d, 1));
+    GB_CK(cudaMemsetAsync(ymax_d, 0, sizeof(unsigned long long), st));
+    k_nb_ymax<<<148 * 2, 256, 0, st>>>(ymax_d, y, N);
+    unsigned long long ymax64 = 0;
+    GB_CK(cudaMemcpyAsync(&ymax64, ymax_d, sizeof(ymax64), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (ymax64 == kNbBadCount) { err = std::string("probe_nb_dispersion") + kNbBadCountMsg; return 1; }
+    const int ymax = (int)ymax64;
+    GB_CK(mem.get(&hist, (size_t)ymax + 2));
+    GB_CK(mem.get(&G, (size_t)ymax + 1));
+    GB_CK(cudaMemsetAsync(hist, 0, sizeof(unsigned long long) * ((size_t)ymax + 2), st));
+    k_nb_hist<<<148 * 2, 256, 0, st>>>(hist, y, N);
+    k_nb_suffix<<<1, 1, 0, st>>>(G, hist, ymax);
+    GB_CK(mem.get(&dfpart, (size_t)K * nblk * 4));
+    GB_CK(mem.get(&dvec, 2 * (size_t)K));
+    std::vector<double> dinit(2 * (size_t)K);
+    for (int c = 0; c < K; ++c) { dinit[c] = d[c]; dinit[(size_t)K + c] = log(d[c]); }
+    GB_CK(cudaMemcpyAsync(dvec, dinit.data(), sizeof(double) * 2 * K, cudaMemcpyHostToDevice, st));
+    if (real_d) {
+        k_nb_dfreal_partial<<<dim3(nblk, K), 256, 0, st>>>(dfpart, phi, y, dvec, N, seed, call);
+        k_nb_dfreal_decide<<<K, 32, 0, st>>>(dvec, dvec + K, out + 4, dfpart, nblk, seed, call, 5, out);
+    } else {
+        k_nb_df_partial<<<dim3(nblk, K), 256, 0, st>>>(dfpart, phi, y, dvec, N, seed, call);
+        k_nb_df_decide<<<K, 32, 0, st>>>(dvec, dvec + K, out + 4, dfpart, nblk, G, ymax, seed, call, 5, out);
+    }
+    count_launch(5);
+    GB_CK(cudaGetLastError());
+    GB_CK(cudaStreamSynchronize(st));            // dinit is a pageable host buffer that leaves scope
     return 0;
 }
 

@@ -1325,9 +1325,10 @@ static __global__ void k_nb_df_fold(double *__restrict__ sum4, const double *__r
         for (int k = 0; k < 4; ++k) sum4[k] = s[k];
 }
 
+// probe (bl_probe_nb_dispersion; the drivers pass null): chain c's {d', u, llh(d), llh(d')} at probe + 5 c.
 static __global__ void k_nb_df_decide(double *__restrict__ dptr, double *__restrict__ ldptr, double *__restrict__ d_rec,
                                const double *__restrict__ part, int nblk, const double *__restrict__ G, int ymax,
-                               uint64_t seed, uint32_t call, int64_t rec_stride = 0)
+                               uint64_t seed, uint32_t call, int64_t rec_stride = 0, double *__restrict__ probe = nullptr)
 {
     const int lane = threadIdx.x, ch = blockIdx.x;
     part += (size_t)ch * nblk * 4;
@@ -1349,6 +1350,7 @@ static __global__ void k_nb_df_decide(double *__restrict__ dptr, double *__restr
         double llh_prop = s[5] + dp * s[2] + s[3];
         double lppsl = log(dp == 1.0 ? 0.5 : 1.0 / 3.0) - log(d == 1.0 ? 0.5 : 1.0 / 3.0);
         double dn = u_acc < exp(llh_prop - llh_prev + lppsl) ? dp : d;
+        if (probe) { probe[5 * ch] = dp; probe[5 * ch + 1] = u_acc; probe[5 * ch + 2] = llh_prev; probe[5 * ch + 3] = llh_prop; }
         dptr[ch] = dn;
         ldptr[ch] = log(dn);
         if (d_rec) d_rec[ch * rec_stride] = dn;
@@ -1400,9 +1402,10 @@ k_nb_dfreal_partial(double *__restrict__ part, const double *__restrict__ phi, c
     }
 }
 
+// probe: chain c's {r*, lu, llh(r), llh(r*)} at probe + 5 c, as in k_nb_df_decide.
 static __global__ void k_nb_dfreal_decide(double *__restrict__ dptr, double *__restrict__ ldptr, double *__restrict__ d_rec,
                                           const double *__restrict__ part, int nblk, uint64_t seed, uint32_t call,
-                                          int64_t rec_stride = 0)
+                                          int64_t rec_stride = 0, double *__restrict__ probe = nullptr)
 {
     const int lane = threadIdx.x, ch = blockIdx.x;
     part += (size_t)ch * nblk * 4;
@@ -1414,6 +1417,7 @@ static __global__ void k_nb_dfreal_decide(double *__restrict__ dptr, double *__r
     for (int o = 16; o; o >>= 1) { s0 += __shfl_xor_sync(0xffffffffu, s0, o); s1 += __shfl_xor_sync(0xffffffffu, s1, o); }
     if (lane == 0) {
         const double dn = lu < s1 - s0 ? rs : r;
+        if (probe) { probe[5 * ch] = rs; probe[5 * ch + 1] = lu; probe[5 * ch + 2] = s0; probe[5 * ch + 3] = s1; }
         dptr[ch] = dn;
         ldptr[ch] = log(dn);
         if (d_rec) d_rec[ch * rec_stride] = dn;
@@ -1434,14 +1438,22 @@ static __global__ void k_nb_prepare(double *__restrict__ psi, double *__restrict
     kappa[k] = 0.5 * (y[i] - d);
 }
 
-// ymax and G[j] = #{y_i > j} (NBPG-logmean.R:65-67)
+// ymax and G[j] = #{y_i > j} (NBPG-logmean.R:65-67).  k_nb_hist indexes hist by (int)y, so a count that is negative,
+// not finite or at least 2^31 - 1 sets *ymax to kNbBadCount instead, which no valid count reaches (an all-reduce by
+// max carries it to every rank); the host refuses the data before it sizes the histogram.
+constexpr unsigned long long kNbBadCount = ~0ull;
 static __global__ void k_nb_ymax(unsigned long long *__restrict__ ymax, const double *__restrict__ y, int64_t N)
 {
     int m = 0;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
-        m = max(m, (int)y[i]);
+    bool bad = false;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
+        const double v = y[i];
+        if (v >= 0.0 && v < 2147483647.0) m = max(m, (int)v);
+        else bad = true;                          // NaN fails both comparisons
+    }
     for (int o = 16; o; o >>= 1) m = max(m, __shfl_xor_sync(0xffffffffu, m, o));
-    if ((threadIdx.x & 31) == 0 && m > 0) atomicMax(ymax, (unsigned long long)m);
+    bad = __any_sync(0xffffffffu, bad);
+    if ((threadIdx.x & 31) == 0 && (bad || m > 0)) atomicMax(ymax, bad ? kNbBadCount : (unsigned long long)m);
 }
 static __global__ void k_nb_hist(unsigned long long *__restrict__ hist, const double *__restrict__ y, int64_t N)
 {

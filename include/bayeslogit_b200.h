@@ -339,6 +339,13 @@ int bl_probe_v_eval(double *v, const double *y, int64_t num);
 int bl_probe_specfun(double *out, int which, const double *a, const double *b, const double *c,
                      int64_t num);
 int bl_probe_philox(uint32_t *out4, const uint32_t *ctr4, const uint32_t *key2);
+/* One negative-binomial dispersion step per chain (real_d = 0: draw.df on the integers, 1: draw.df.real.mean), run
+ * with the kernels and grids of bl_nb_gibbs_df / bl_nb_gibbs_dfreal (chains = 1) and bl_nb_multichain, on given
+ * phi [chains][N] (phi = X beta of chain c at phi + c N), counts y [N] and d [chains]; chain c keys its Metropolis
+ * stream by seed + c and call.  out [chains][5] = {proposal d', accept variate (u; real walk: log u), llh(d),
+ * llh(d'), new d}. */
+int bl_probe_nb_dispersion(double *out, const double *phi, const double *y, const double *d, int chains, int64_t N,
+                           uint64_t seed, uint32_t call, int real_d);
 
 /* Pipe-throughput microbenchmarks on the current device, the denominators of the sampler's compute
  * roofline (bench.py): out6 = FP64 FMA TFLOP/s, FP32 FMA TFLOP/s, MUFU (ex2/lg2) Gop/s, FP64 tensor

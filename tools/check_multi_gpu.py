@@ -122,6 +122,28 @@ def nb_dfreal_chain(X, yc, lo, hi):
     return beta.cpu().numpy(), dd.cpu().numpy()
 
 
+def nb_mode_chain(mode, X, yc, lo, hi):
+    """NB sweep in one of the three dispersion modes with a non-zero prior mean and a dense prior precision (so
+    b0 = P0 m0 enters the beta draw).  Returns (beta, d)."""
+    P = X.shape[1]
+    Xd = torch.from_numpy(X[lo:hi].copy()).to(dev); yd = torch.from_numpy(yc[lo:hi].copy()).to(dev)
+    m0 = torch.linspace(-0.4, 0.4, P, device=dev, dtype=torch.float64)
+    P0 = (0.02 * torch.eye(P, device=dev, dtype=torch.float64) + 0.005).contiguous()
+    beta = torch.zeros(6, P, device=dev, dtype=torch.float64)
+    dd = torch.full((6,), 2.0, device=dev, dtype=torch.float64)
+    if mode == "fixed":
+        rc = L.bl_nb_gibbs_dev(None, beta.data_ptr(), yd.data_ptr(), Xd.data_ptr(), 2.0, m0.data_ptr(),
+                               P0.data_ptr(), hi - lo, P, 6, 919, lo, st)
+    else:
+        fn = L.bl_nb_gibbs_dfreal_dev if mode == "real" else L.bl_nb_gibbs_df_dev
+        rc = fn(None, beta.data_ptr(), dd.data_ptr(), yd.data_ptr(), Xd.data_ptr(), 2.5 if mode == "real" else 2.0,
+                m0.data_ptr(), P0.data_ptr(), hi - lo, P, 6, 3, 919, lo, st)
+    if rc:
+        _lib.check(rc)
+    torch.cuda.synchronize()
+    return beta.cpu().numpy(), dd.cpu().numpy()
+
+
 def make_mlogit(N, P, J, seed):
     rng = np.random.default_rng(seed)
     X = np.c_[rng.standard_normal((N, P - 1)) / np.sqrt(max(P - 1, 1)), np.ones(N)]
@@ -166,6 +188,11 @@ nbdfreal_full = nb_dfreal_chain(data[c0][0], data[c0][2], 0, c0[0])
 MCASES = [(200_003, 16, 4), (50_001, 7, 3), (60_001, 32, 5)]
 mdata = {c: make_mlogit(c[0], c[1], c[2], 20 + c[1]) for c in MCASES}
 mfull = {c: mlogit_chain(*mdata[c], 0, c[0]) for c in MCASES}
+# NB in all three dispersion modes: P = 7 odd P^2 count (k_xtv_partial), P = 70 several Gram tiles
+NBCASES = [(9_001, 7), (12_001, 70)]
+NBMODES = ["fixed", "int", "real"]
+nbdata = {c: make(c[0], c[1], 30 + c[1]) for c in NBCASES}
+nbfull = {(c, m): nb_mode_chain(m, nbdata[c][0], nbdata[c][2], 0, c[0]) for c in NBCASES for m in NBMODES}
 
 ok = True
 
@@ -211,6 +238,17 @@ def sharded_pass(tag):
         print(f"[{tag}] nb with real-valued dispersion: max rel diff beta {e_dr:.2e} d {ed_dr:.2e}; beta and d "
               f"bit-identical across ranks: {same_dr} (d: {d_dr[0]:.3f} .. {d_dr[-1]:.3f})", flush=True)
     ok = ok and e_dr < 1e-8 and ed_dr < 1e-12 and same_dr
+    for c in NBCASES:
+        lo, hi = bdist.shard_range(rank, world, c[0])
+        for m in NBMODES:
+            b, d = nb_mode_chain(m, nbdata[c][0], nbdata[c][2], lo, hi)
+            fb, fd = nbfull[(c, m)]
+            eb, ed = allmax([np.max(np.abs(b - fb) / np.abs(fb)), np.max(np.abs(d - fd) / np.abs(fd))])
+            same = same_on_all_ranks(b) and same_on_all_ranks(d)
+            if rank == 0:
+                print(f"[{tag}] nb ({m} d) N={c[0]} P={c[1]}: world={world} max rel diff beta {eb:.2e} d {ed:.2e}; "
+                      f"beta and d bit-identical across ranks: {same}", flush=True)
+            ok = ok and eb < 1e-8 and (ed < 1e-12 if m == "real" else ed == 0.0) and same
     for c in MCASES:
         lo, hi = bdist.shard_range(rank, world, c[0])
         b, w = mlogit_chain(*mdata[c], lo, hi)
