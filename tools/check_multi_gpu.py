@@ -74,6 +74,34 @@ def chain(X, y, lo, hi, flags):
     return beta.cpu().numpy(), w.cpu().numpy()
 
 
+def prior_chain(X, y, n, lo, hi, flags):
+    """Logit sweep with a non-zero prior mean and a dense prior precision (b0 = P0 m0 must be added once, after the
+    all-reduce of X'kappa) and binomial counts."""
+    P = X.shape[1]
+    Xd = torch.from_numpy(X[lo:hi].copy()).to(dev); yd = torch.from_numpy(y[lo:hi].copy()).to(dev)
+    nd = torch.from_numpy(n[lo:hi].copy()).to(dev)
+    m0 = torch.linspace(-0.1, 0.1, P, device=dev, dtype=torch.float64)
+    P0 = (0.5 * torch.eye(P, device=dev, dtype=torch.float64) + 0.01).contiguous()
+    beta = torch.zeros(6, P, device=dev, dtype=torch.float64)
+    w = torch.zeros(6, hi - lo, device=dev, dtype=torch.float64)
+    rc = L.bl_logit_gibbs_dev(w.data_ptr(), beta.data_ptr(), yd.data_ptr(), Xd.data_ptr(), nd.data_ptr(),
+                              m0.data_ptr(), P0.data_ptr(), hi - lo, P, 6, 3, 4243, flags, lo, st)
+    if rc:
+        _lib.check(rc)
+    torch.cuda.synchronize()
+    return beta.cpu().numpy(), w.cpu().numpy()
+
+
+def make_binomial(N, P, seed, binomial):
+    rng = np.random.default_rng(seed)
+    X = np.c_[rng.standard_normal((N, P - 1)), np.ones(N)]
+    bt = np.r_[np.abs(rng.normal(0, 0.4, P - 1)), -0.5]
+    p = 1 / (1 + np.exp(-X @ bt))
+    n = rng.integers(1, 6, N).astype(float) if binomial else np.ones(N)
+    y = rng.binomial(n.astype(int), p) / n
+    return X, y, n
+
+
 def nb_chain(X, yc, lo, hi):
     P = X.shape[1]
     Xd = torch.from_numpy(X[lo:hi].copy()).to(dev); yd = torch.from_numpy(yc[lo:hi].copy()).to(dev)
@@ -193,6 +221,13 @@ NBCASES = [(9_001, 7), (12_001, 70)]
 NBMODES = ["fixed", "int", "real"]
 nbdata = {c: make(c[0], c[1], 30 + c[1]) for c in NBCASES}
 nbfull = {(c, m): nb_mode_chain(m, nbdata[c][0], nbdata[c][2], 0, c[0]) for c in NBCASES for m in NBMODES}
+# logit with a non-zero m0 and a dense P0, both beta draws: (N, P, binomial, flag variants).  P = 32: the packed
+# Gram, binomial counts; P = 64: the one-pass kernel's published sums and (BL_GIBBS_TWO_PASS) k_gram_reduce's;
+# P = 70: several Gram tiles, the constrained draw at P > 64; P = 128: the beta draw out of global scratch
+PCASES = [(60_001, 32, True, (0,)), (50_001, 64, False, (0, 16)), (24_001, 70, False, (0,)), (12_001, 128, False, (0,))]
+pdata = {c: make_binomial(c[0], c[1], 40 + c[1], c[2]) for c in PCASES}
+pruns = [(c, f | b) for c in PCASES for f in c[3] for b in (0, 1)]
+pfull = {k: prior_chain(*pdata[k[0]], 0, k[0][0], k[1]) for k in pruns}
 
 ok = True
 
@@ -212,6 +247,17 @@ def sharded_pass(tag):
                 print(f"[{tag}] logit N={c[0]} P={c[1]} flags={f}: world={world} max rel diff beta {eb:.2e} omega {ew:.2e}; "
                       f"beta bit-identical across ranks: {same}", flush=True)
             ok = ok and max(eb, ew) < 1e-8 and same
+    for k in pruns:
+        c, f = k
+        lo, hi = bdist.shard_range(rank, world, c[0])
+        b, w = prior_chain(*pdata[c], lo, hi, f)
+        fb, fw = pfull[k]
+        eb, ew = allmax([np.max(np.abs(b - fb) / np.abs(fb)), np.max(np.abs(w - fw[:, lo:hi]) / fw[:, lo:hi])])
+        same = same_on_all_ranks(b)
+        if rank == 0:
+            print(f"[{tag}] logit (non-zero m0, dense P0) N={c[0]} P={c[1]} flags={f}: world={world} max rel diff "
+                  f"beta {eb:.2e} omega {ew:.2e}; beta bit-identical across ranks: {same}", flush=True)
+        ok = ok and max(eb, ew) < 1e-8 and same
     lo, hi = bdist.shard_range(rank, world, c0[0])
     b, w = nb_chain(data[c0][0], data[c0][2], lo, hi)
     eb = np.max(np.abs(b - nb_full[0]) / np.abs(nb_full[0]))
