@@ -33,17 +33,21 @@ int report(const std::string &msg, const char *abort_line)
 struct Dev {
     std::vector<void *> ptrs;
     ~Dev() { for (void *p : ptrs) cudaFree(p); }
-    double *put(const double *host, size_t count, std::string &err)
+    void *put_bytes(const void *host, size_t bytes, std::string &err)
     {
         void *p = nullptr;
-        cudaError_t e = cudaMalloc(&p, (count ? count : 1) * sizeof(double));
-        if (e == cudaSuccess && host) e = cudaMemcpy(p, host, count * sizeof(double), cudaMemcpyHostToDevice);
+        cudaError_t e = cudaMalloc(&p, bytes ? bytes : 8);
+        if (e == cudaSuccess && host) e = cudaMemcpy(p, host, bytes, cudaMemcpyHostToDevice);
         // pageable source: wait for the DMA itself, the sweeps run on a stream that does not order
         // against the legacy stream
         if (e == cudaSuccess && host) e = cudaStreamSynchronize(cudaStreamLegacy);
         if (e != cudaSuccess) { err = std::string("device buffer: ") + cudaGetErrorString(e); if (p) cudaFree(p); return nullptr; }
         ptrs.push_back(p);
-        return (double *)p;
+        return p;
+    }
+    double *put(const double *host, size_t count, std::string &err)
+    {
+        return (double *)put_bytes(host, count * sizeof(double), err);
     }
 };
 
@@ -553,6 +557,48 @@ int bl_nb_gibbs_dev(double *w_last, double *beta, const double *y, const double 
     if (bl_ensure_ready_internal()) return 1;
     std::string err;
     if (nb_gibbs_device(w_last, beta, y, tX, d, m0, P0, N, P, samp, seed, obs0, true, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
+// ---- binomial logit with group random intercepts ----------------------------------------------------------
+
+int bl_logit_ri_gibbs(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                      const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                      double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !n || !group || !m0 || !P0) return report("logit_ri_gibbs: null argument", nullptr);
+    std::string err;
+    if (logit_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, flags, err)) return report(err, nullptr);
+    for (int64_t i = 0; i < N; ++i)
+        if (group[i] < 0 || group[i] >= G) return report(kLogitRiBadIdMsg, nullptr);
+    Dev d;
+    double *dy = d.put(y, N, err), *dX = d.put(tX, (size_t)N * P, err), *dn = d.put(n, N, err);
+    double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
+    int *dg = (int *)d.put_bytes(group, sizeof(int) * (size_t)N, err);
+    double *dbeta = d.put(nullptr, (size_t)P * samp, err), *dtau2 = d.put(nullptr, samp, err);
+    double *du = u ? d.put(nullptr, (size_t)G * samp, err) : nullptr;
+    if (!err.empty()) return report(err, nullptr);
+    if (logit_ri_gibbs_device(dbeta, du, dtau2, dy, dX, dn, dg, G, dm0, dP0, a0, b0, tau2_0, N, P, samp, burn, seed, flags,
+                              (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * (size_t)P * samp, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemcpy(tau2, dtau2, sizeof(double) * samp, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && u) e = cudaMemcpy(u, du, sizeof(double) * (size_t)G * samp, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
+int bl_logit_ri_gibbs_dev(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                          const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                          double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags, void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !n || !group || !m0 || !P0) return report("logit_ri_gibbs: null argument", nullptr);
+    std::string err;
+    if (logit_ri_gibbs_device(beta, u, tau2, y, tX, n, group, G, m0, P0, a0, b0, tau2_0, N, P, samp, burn, seed, flags,
+                              (cudaStream_t)stream, err))
         return report(err, nullptr);
     return 0;
 }

@@ -57,10 +57,12 @@ bool devroye_binned(int64_t num, int64_t bin_min);         // whether a batch of
 
 // Fused psi = X beta + omega = PG(n, psi) of the logit sweeps (pg_devroye_kernel.cu); needs even P and a
 // 16-byte aligned tX (logit_psi_draw_ok).  chains > 1: rows [c N, (c+1) N) meet beta + c * beta_stride and
-// id.chain_len = N keys their streams by seed + c.
+// id.chain_len = N keys their streams by seed + c.  off (one chain): omega_i = PG(n_i, x_i . beta + off_i), psi_out
+// keeps x_i . beta.
 bool logit_psi_draw_ok(const double *tX, int P);
 cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, const double *tX, const double *beta,
-                                  int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream);
+                                  int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream,
+                                  const double *off = nullptr);
 // The same for `chains` chains that share ONE set of N rows (n [N], tX P x N): chain c meets beta + c * beta_stride
 // and the streams of id.seed + c; x: omega [chains][N].  Same conditions on P and tX.
 cudaError_t launch_logit_psi_draw_shared(double *x, const int *n, const double *tX, const double *beta,
@@ -87,6 +89,15 @@ int nb_gibbs_device(double *w_out, double *beta_out, const double *y, const doub
 int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const double *y, const double *tX,
                        double d0, const double *m0, const double *P0, int64_t N, int P, int samp, int burn,
                        uint64_t seed, uint64_t obs0, bool sharded, int real_d, cudaStream_t st, std::string &err);
+// Binomial logit with group random intercepts, one chain (gibbs.cu).  logit_ri_check refuses what the driver cannot
+// run (every argument but the ids); the driver checks the ids on the device before anything else runs.
+int logit_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, int flags,
+                   std::string &err);
+extern const char *const kLogitRiBadIdMsg;
+int logit_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, const double *y, const double *tX,
+                          const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
+                          double b0, double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
+                          cudaStream_t st, std::string &err);
 // shared_rows: every chain runs on the same N rows (y, n [N], tX P x N) instead of rows [c N, (c+1) N) of its own
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
@@ -110,6 +121,9 @@ int logit_em_device(double *beta, const double *y, const double *tX, const doubl
                     int P, double tol, int max_iter, int *iters, cudaStream_t st, std::string &err);
 // duplicate-row merge on device-resident data (merge.cu); returns M, -1 (CUDA error), -2 (needs the exact host merge)
 int merge_rows_device(double *ty, double *tX, double *n, int N, int P, int ny, cudaStream_t st, std::string &err);
+// stable sort of the rows 0..n-1 by key (0 <= key < nkeys) on the device (merge.cu): order[k] = row at sorted
+// position k, key_sorted[k] = its key; rows with equal keys stay in increasing order
+int sort_rows_by_key(int *order, int *key_sorted, const int *key, int n, int nkeys, cudaStream_t st, std::string &err);
 int comm_unique_id(void *out128, std::string &err);
 int comm_init(const void *id128, int rank, int world, std::string &err);
 int comm_init_local(int rank, int world, std::string &err);

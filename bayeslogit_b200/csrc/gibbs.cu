@@ -14,6 +14,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <chrono>
@@ -1227,6 +1228,138 @@ int mlogit_multichain_device(double *beta_out, const double *ty, const double *t
     GB_CK(cudaStreamSynchronize(st));
     if (h != 0) { err = "mlogit_multichain: a chain's posterior precision is not positive definite"; return 1; }
     return 0;
+}
+
+// ------------------------------------------------------------------------------------
+// Binomial logit with group random intercepts (the GLMM with one grouping factor; the reference's
+// Logit-MixedModel.R restated as one more conditionally Gaussian block under PG augmentation):
+//   psi_i = x_i . beta + u_{g_i},  u_g ~ N(0, tau2),  beta ~ N(m0, P0^-1),  tau2 ~ IG(a0, b0).
+// Iteration t (burn-in included), from beta = 0, u = 0, tau2 = tau2_0:
+//   1. eta = X beta, omega_i = PG(n_i, eta_i + u_{g_i})                stream (seed, i, t)
+//   2. u_g = R_g / prec + z_g / sqrt(prec), prec = S_g + 1 / tau2       z_g: stream (seed, 2^63 + g, t)
+//      S_g = sum_{i in g} omega_i, R_g = sum_{i in g} (kappa_i - omega_i eta_i)
+//   3. tau2 = (b0 + sum_g u_g^2 / 2) / gamma, gamma ~ Gamma(a0 + G/2, 1) stream (seed, 2^64 - 4, t)
+//   4. beta ~ N(Q^-1 r, Q^-1), Q = P0 + X' Omega X, r = P0 m0 + X'(kappa - omega o u_g)   stream (seed, 2^64 - 1, t)
+// Iteration t >= burn is stored in row t - burn of beta_out [samp][P], u_out [samp][G] (may be null) and
+// tau2_out [samp].  One chain on one GPU; device pointers throughout.
+// ------------------------------------------------------------------------------------
+int logit_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, int flags,
+                   std::string &err)
+{
+    if (flags & ~BL_GIBBS_UNFUSED) { err = "logit_ri_gibbs: unknown flag (only BL_GIBBS_UNFUSED is accepted)"; return 1; }
+    if (N < 1 || N >= (1LL << 31) || P < 1 || samp < 1 || burn < 0 || (int64_t)samp + burn >= (1LL << 31)) {
+        err = "logit_ri_gibbs: bad dimensions (need 1 <= N < 2^31, P >= 1, samp >= 1, burn >= 0)";
+        return 1;
+    }
+    if (P > 256) { err = "logit_ri_gibbs: P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
+    if (G < 1) { err = "logit_ri_gibbs: G must be at least 1"; return 1; }
+    if (!(std::isfinite(a0) && a0 > 0.0) || !(std::isfinite(b0) && b0 > 0.0) || !(std::isfinite(tau2_0) && tau2_0 > 0.0)) {
+        err = "logit_ri_gibbs: a0, b0 and tau2_0 must be finite and positive";
+        return 1;
+    }
+    return 0;
+}
+
+const char *const kLogitRiBadIdMsg = "logit_ri_gibbs: group ids must lie in [0, G)";
+
+int logit_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, const double *y, const double *tX,
+                          const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
+                          double b0, double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
+                          cudaStream_t st, std::string &err)
+{
+    if (logit_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, flags, err)) return 1;
+    DevMem mem;
+    mem.st = st;
+    // the ids first: a refusal leaves the outputs untouched and launches no iteration
+    int *bad;
+    GB_CK(mem.get(&bad, 1));
+    GB_CK(cudaMemsetAsync(bad, 0, sizeof(int), st));
+    k_ri_check_ids<<<(int)std::min<int64_t>(148 * 8, cdiv(N, 256)), 256, 0, st>>>(bad, group, N, G);
+    count_launch();
+    int hbad = 0;
+    GB_CK(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (hbad) { err = kLogitRiBadIdMsg; return 1; }
+
+    Sweep s;
+    s.N = N; s.P = P; s.obs0 = 0; s.st = st; s.tX = tX;
+    if (s.init(mem, err)) return 1;
+    // psi and the omega draw as one pass over X (k_logit_psi_draw<true>) unless asked otherwise or P is odd / X unaligned
+    const bool fused = !(flags & BL_GIBBS_UNFUSED) && logit_psi_draw_ok(tX, P);
+    const int nchunks = cdiv(N, kRiChunk), nublk = cdiv(G, kRiDrawWarps);
+    const int rgrid = (int)std::min<int64_t>(148 * 8, cdiv(N, 256));
+    double *kappa, *bprior, *eta, *off, *v, *bbuf, *S, *R, *edge, *u, *usq, *tau2;
+    int *shape, *order, *gs, *goff;
+    GB_CK(mem.get(&kappa, N));
+    GB_CK(mem.get(&shape, N));
+    GB_CK(mem.get(&eta, N));
+    GB_CK(mem.get(&off, N));
+    GB_CK(mem.get(&v, N));
+    GB_CK(mem.get(&order, N));
+    GB_CK(mem.get(&gs, N));
+    GB_CK(mem.get(&goff, (size_t)G + 1));
+    GB_CK(mem.get(&bprior, P));
+    GB_CK(mem.get(&bbuf, P));
+    GB_CK(mem.get(&S, G));
+    GB_CK(mem.get(&R, G));
+    GB_CK(mem.get(&edge, 4 * (size_t)nchunks));
+    GB_CK(mem.get(&u, G));
+    GB_CK(mem.get(&usq, nublk));
+    GB_CK(mem.get(&tau2, 1));
+    k_kappa<<<cdiv(N, 256), 256, 0, st>>>(kappa, y, n, 0.0, N);
+    k_shape_int<<<cdiv(N, 256), 256, 0, st>>>(shape, n, N);
+    k_matvec<<<cdiv(P, 128), 128, 0, st>>>(bprior, P0, m0, P);
+    count_launch(3);
+    // rows sorted by group (stable: increasing row order inside a group) and the groups' first positions
+    if (sort_rows_by_key(order, gs, group, (int)N, G, st, err)) return 1;
+    k_ri_offsets<<<cdiv(N + 1, 256), 256, 0, st>>>(goff, gs, N, G);
+    count_launch();
+    GB_CK(cudaMemsetAsync(off, 0, sizeof(double) * N, st));
+    GB_CK(cudaMemsetAsync(bbuf, 0, sizeof(double) * P, st));
+    GB_CK(cudaMemcpyAsync(tau2, &tau2_0, sizeof(double), cudaMemcpyHostToDevice, st));
+    StageTimer tmr;
+    tmr.st = st;
+    const double *bprev = bbuf;
+    for (int t = 0; t < samp + burn; ++t) {
+        tmr.arm(t == samp + burn - 1);
+        const StreamId id{seed, 0, (uint32_t)t};
+        cudaError_t e;
+        if (fused) {
+            e = launch_logit_psi_draw(s.w, eta, shape, tX, bprev, 0, 1, N, P, id, st, off);
+        } else {
+            s.xbeta(eta, bprev, nullptr, 0.0);
+            launch_pdl(k_ri_psi, dim3(rgrid), dim3(256), 0, st, s.psi, (const double *)eta, (const double *)off, N);
+            count_launch();
+            e = launch_devroye_refill(s.w, shape, s.psi, N, id, st);
+        }
+        if (e != cudaSuccess) { err = std::string("logit_ri_gibbs: ") + cudaGetErrorString(e); return 1; }
+        tmr.mark("psi+draw");
+        launch_pdl(k_ri_group_sums, dim3(nchunks), dim3(kRiThreads), 0, st, S, R, edge, (const int *)order,
+                   (const int *)gs, (const int *)goff, (const double *)s.w, (const double *)eta, (const double *)kappa, N);
+        tmr.mark("group sums");
+        const bool rec = t >= burn;
+        launch_pdl(k_ri_draw_u, dim3(nublk), dim3(32 * kRiDrawWarps), 0, st, u,
+                   rec && u_out ? u_out + (size_t)G * (t - burn) : (double *)nullptr, usq, (const double *)S,
+                   (const double *)R, (const double *)edge, (const int *)goff, (const double *)tau2, G, seed, (uint32_t)t);
+        launch_pdl(k_ri_draw_tau2, dim3(1), dim3(256), 0, st, tau2, rec ? tau2_out + (t - burn) : (double *)nullptr,
+                   (const double *)usq, nublk, G, a0, b0, seed, (uint32_t)t);
+        tmr.mark("u+tau2");
+        launch_pdl(k_ri_rows, dim3(rgrid), dim3(256), 0, st, off, v, group, (const double *)u, (const double *)s.w,
+                   (const double *)kappa, N);
+        count_launch(4);
+        tmr.mark("rows");
+        s.xtv(v, 1.0, nullptr, nullptr, 0.0);                                 // X'(kappa - omega o u_g)
+        tmr.mark("xtv");
+        s.gram(s.w);
+        tmr.mark("gram");
+        double *bdst = rec ? beta_out + (size_t)P * (t - burn) : bbuf;
+        s.beta_draw(kBetaPlain, P0, bprior, true, nullptr, bdst, seed, (uint32_t)t);
+        tmr.mark("beta");
+        tmr.report("logit_ri");
+        bprev = bdst;
+    }
+    GB_CK(cudaGetLastError());
+    return s.check_status(err, "logit_ri_gibbs");
 }
 
 // ------------------------------------------------------------------------------------

@@ -1497,4 +1497,227 @@ static __global__ void k_mlogit_offsets(double *__restrict__ c, double *__restri
     eta[i] = XB[i + (size_t)N * j] - cj;
 }
 
+// ---------------------------------------------------------------------------------
+// Random-intercept logit (logit_ri_gibbs_device): psi_i = x_i . beta + u_{g_i}, u_g ~ N(0, tau2), tau2 ~ IG(a0, b0).
+// Per iteration, after the omega draw: group sums S_g = sum omega_i, R_g = sum (kappa_i - omega_i eta_i) over the
+// rows of the group, u_g | . ~ N(R_g / (S_g + 1/tau2), 1 / (S_g + 1/tau2)), tau2 | u, then the rows' offsets and
+// v_i = kappa_i - omega_i u_{g_i} for X'v.  Sums run over the rows sorted by group (a stable sort made once per
+// chain), cut into fixed chunks of kRiChunk positions: a chunk sums the segments it holds in a fixed order and writes
+// a group that lies inside it straight to S, R; a group that crosses chunk boundaries leaves its first piece as the
+// tail of its first chunk and the rest as the heads of the following chunks, which k_ri_draw_u adds in chunk order.
+// No floating-point atomics: every sum is bit-identical from run to run, whatever the group sizes.
+// ---------------------------------------------------------------------------------
+constexpr uint64_t kRiGroupObs0 = 0x8000000000000000ull;   // u_g: first normal of the stream (seed, 2^63 + g, call)
+constexpr uint64_t kRiTau2Obs = 0xFFFFFFFFFFFFFFFCull;     // tau2: the gamma variate of the stream (seed, 2^64 - 4, call)
+constexpr int kRiItems = 8;                                // sorted positions per thread
+constexpr int kRiThreads = 256;
+constexpr int kRiChunk = kRiItems * kRiThreads;            // sorted positions per chunk (one CTA)
+constexpr int kRiDrawWarps = 8;                            // groups per CTA of k_ri_draw_u (a warp each)
+
+// *bad = 1 if an id lies outside [0, G)
+static __global__ void k_ri_check_ids(int *__restrict__ bad, const int *__restrict__ group, int64_t N, int G)
+{
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
+        if (group[i] < 0 || group[i] >= G) *bad = 1;
+}
+
+// goff[g] = first sorted position of group g, goff[G] = N (gs: the ids in sorted order).  Thread k writes the
+// groups that start at position k -- the one at k and the empty ones before it -- so every entry is written once.
+static __global__ void k_ri_offsets(int *__restrict__ goff, const int *__restrict__ gs, int64_t N, int G)
+{
+    const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (k > N) return;
+    const int lo = k == 0 ? 0 : gs[k - 1] + 1, hi = k == N ? G : gs[k];
+    for (int g = lo; g <= hi; ++g) goff[g] = (int)k;
+}
+
+// unfused path: psi_i = eta_i + off_i
+static __global__ void k_ri_psi(double *__restrict__ psi, const double *__restrict__ eta, const double *__restrict__ off,
+                                int64_t N)
+{
+    BL_PDL_ENTER();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
+        psi[i] = eta[i] + off[i];
+}
+
+// Segment sum (s, r) with a flag: a segment starts inside the run it covers.  a then b: b alone if b holds a start.
+struct RiSeg {
+    double s, r;
+    int f;
+};
+__device__ __forceinline__ RiSeg ri_seg_join(const RiSeg &a, const RiSeg &b)
+{
+    return b.f ? b : RiSeg{a.s + b.s, a.r + b.r, a.f};
+}
+
+// One CTA per chunk of kRiChunk sorted positions, kRiItems consecutive positions per thread.  edge[4 c ..]: head
+// (s, r) and tail (s, r) pieces of chunk c (written only when a group crosses that edge).
+static __global__ void __launch_bounds__(kRiThreads)
+k_ri_group_sums(double *__restrict__ S, double *__restrict__ R, double *__restrict__ edge, const int *__restrict__ order,
+                const int *__restrict__ gs, const int *__restrict__ goff, const double *__restrict__ w,
+                const double *__restrict__ eta, const double *__restrict__ kappa, int64_t N)
+{
+    BL_PDL_ENTER();
+    __shared__ RiSeg wtot[kRiThreads / 32], wcarry[kRiThreads / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int64_t p0 = (int64_t)blockIdx.x * kRiChunk, p1 = min(p0 + (int64_t)kRiChunk, N);
+    const int64_t q0 = p0 + (int64_t)threadIdx.x * kRiItems;
+    double sv[kRiItems], rv[kRiItems];
+    int gv[kRiItems];
+#pragma unroll
+    for (int k = 0; k < kRiItems; ++k) {
+        const int64_t p = q0 + k;
+        gv[k] = -1;
+        sv[k] = rv[k] = 0.0;
+        if (p < p1) {
+            const int row = order[p];
+            const double om = w[row];
+            gv[k] = gs[p];
+            sv[k] = om;
+            rv[k] = fma(-om, eta[row], kappa[row]);
+        }
+    }
+    const int gprev = (q0 > p0 && q0 < p1) ? gs[q0 - 1] : -1;
+    // the thread's own run: the sums since its last segment start
+    RiSeg own{0.0, 0.0, 0};
+#pragma unroll
+    for (int k = 0; k < kRiItems; ++k) {
+        if (gv[k] < 0) break;
+        if (gv[k] != (k == 0 ? gprev : gv[k - 1])) own = RiSeg{0.0, 0.0, 1};
+        own.s += sv[k];
+        own.r += rv[k];
+    }
+    // segmented inclusive scan over the warp's runs, then over the warps (fixed order)
+    RiSeg inc = own;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        RiSeg t{__shfl_up_sync(0xffffffffu, inc.s, o), __shfl_up_sync(0xffffffffu, inc.r, o),
+                __shfl_up_sync(0xffffffffu, inc.f, o)};
+        if (lane >= o) inc = ri_seg_join(t, inc);
+    }
+    if (lane == 31) wtot[warp] = inc;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        RiSeg run{0.0, 0.0, 0};
+        for (int v = 0; v < kRiThreads / 32; ++v) {
+            wcarry[v] = run;
+            run = ri_seg_join(run, wtot[v]);
+        }
+    }
+    __syncthreads();
+    RiSeg ex{__shfl_up_sync(0xffffffffu, inc.s, 1), __shfl_up_sync(0xffffffffu, inc.r, 1),
+             __shfl_up_sync(0xffffffffu, inc.f, 1)};
+    const RiSeg carry = lane == 0 ? wcarry[warp] : ri_seg_join(wcarry[warp], ex);
+    // the segments that end in this thread's positions
+    double rs = carry.s, rr = carry.r;
+#pragma unroll
+    for (int k = 0; k < kRiItems; ++k) {
+        if (gv[k] < 0) break;
+        if (gv[k] != (k == 0 ? gprev : gv[k - 1])) rs = rr = 0.0;
+        rs += sv[k];
+        rr += rv[k];
+        const int64_t p = q0 + k;
+        const int gnext = p + 1 >= p1 ? -1 : k + 1 < kRiItems ? gv[k + 1] : gs[p + 1];
+        if (gnext != gv[k]) {
+            const int g = gv[k];
+            if (goff[g] < p0) { edge[4 * blockIdx.x] = rs; edge[4 * blockIdx.x + 1] = rr; }
+            else if (goff[g + 1] > p1) { edge[4 * blockIdx.x + 2] = rs; edge[4 * blockIdx.x + 3] = rr; }
+            else { S[g] = rs; R[g] = rr; }
+        }
+    }
+}
+
+// A warp per group: (S_g, R_g) -- the chunk's sums, or the pieces of a group that crosses chunks added in chunk order --
+// then u_g = R_g / prec + z_g / sqrt(prec), prec = S_g + 1 / tau2 (an empty group draws from its prior), z_g the first
+// normal of the stream (seed, 2^63 + g, call).  usq_part[b] = sum of u_g^2 over the CTA's groups, in group order.
+static __global__ void __launch_bounds__(32 * kRiDrawWarps)
+k_ri_draw_u(double *__restrict__ u, double *__restrict__ u_rec, double *__restrict__ usq_part,
+            const double *__restrict__ S, const double *__restrict__ R, const double *__restrict__ edge,
+            const int *__restrict__ goff, const double *__restrict__ tau2, int G, uint64_t seed, uint32_t call)
+{
+    BL_PDL_ENTER();
+    __shared__ double sq[kRiDrawWarps];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int g = blockIdx.x * kRiDrawWarps + warp;
+    double ug = 0.0;
+    if (g < G) {
+        const int a = goff[g], b = goff[g + 1];
+        double s = 0.0, r = 0.0;
+        if (b > a) {
+            const int c0 = a / kRiChunk, c1 = (b - 1) / kRiChunk;
+            if (c0 == c1) {
+                s = S[g];
+                r = R[g];
+            } else {
+                double hs = 0.0, hr = 0.0;
+                for (int c = c0 + 1 + lane; c <= c1; c += 32) {
+                    hs += edge[4 * (size_t)c];
+                    hr += edge[4 * (size_t)c + 1];
+                }
+#pragma unroll
+                for (int o = 16; o; o >>= 1) {
+                    hs += __shfl_xor_sync(0xffffffffu, hs, o);
+                    hr += __shfl_xor_sync(0xffffffffu, hr, o);
+                }
+                s = edge[4 * (size_t)c0 + 2] + hs;
+                r = edge[4 * (size_t)c0 + 3] + hr;
+            }
+        }
+        if (lane == 0) {
+            const double prec = s + 1.0 / tau2[0];
+            const double m = r / prec;
+            PhiloxSource src;
+            src.open(seed, kRiGroupObs0 + (uint64_t)g, call);
+            ug = m + src.norm() / sqrt(prec);
+            u[g] = ug;
+            if (u_rec) u_rec[g] = ug;
+        }
+    }
+    if (lane == 0) sq[warp] = ug * ug;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double t = 0.0;
+        for (int v = 0; v < kRiDrawWarps; ++v) t += sq[v];
+        usq_part[blockIdx.x] = t;
+    }
+}
+
+// One CTA: sum of u_g^2 over the partials in a fixed order, then tau2 = (b0 + sum / 2) / gamma, gamma ~ Gamma(a0 + G/2, 1)
+// from the stream (seed, 2^64 - 4, call) (Marsaglia-Tsang, PhiloxSource::gamma).
+static __global__ void __launch_bounds__(256)
+k_ri_draw_tau2(double *__restrict__ tau2, double *__restrict__ tau2_rec, const double *__restrict__ usq_part, int nparts,
+               int G, double a0, double b0, uint64_t seed, uint32_t call)
+{
+    BL_PDL_ENTER();
+    __shared__ double red[256];
+    double s = 0.0;
+    for (int k = threadIdx.x; k < nparts; k += 256) s += usq_part[k];
+    red[threadIdx.x] = s;
+    __syncthreads();
+    for (int o = 128; o; o >>= 1) {
+        if ((int)threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        PhiloxSource src;
+        src.open(seed, kRiTau2Obs, call);
+        const double t2 = (b0 + 0.5 * red[0]) / src.gamma(a0 + 0.5 * (double)G);
+        *tau2 = t2;
+        if (tau2_rec) *tau2_rec = t2;
+    }
+}
+
+// The rows after the u draw: off_i = u_{g_i} (the next iteration's psi offset), v_i = kappa_i - omega_i off_i.
+static __global__ void k_ri_rows(double *__restrict__ off, double *__restrict__ v, const int *__restrict__ group,
+                                 const double *__restrict__ u, const double *__restrict__ w,
+                                 const double *__restrict__ kappa, int64_t N)
+{
+    BL_PDL_ENTER();
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
+        const double ug = u[group[i]];
+        off[i] = ug;
+        v[i] = fma(-w[i], ug, kappa[i]);
+    }
+}
+
 }  // namespace bl

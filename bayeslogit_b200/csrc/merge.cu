@@ -271,6 +271,49 @@ int scan_exclusive(int *out, const int *in, int n, int *tile, int *total, cudaSt
 
 }  // namespace
 
+// Stable LSD radix sort of (key, val) pairs by the low `bits` bits of key, 8 bits a pass.  The pointers are swapped
+// pass by pass: on return key_a / val_a hold the sorted pairs.  hist: 256 cdiv(n, kSortTile) ints; tile: scan scratch
+// of cdiv(max(n, 256 cdiv(n, kSortTile)), 1024) + 1 ints.
+static void radix_sort_pairs(int *&key_a, int *&val_a, int *&key_b, int *&val_b, int n, int bits, int *hist, int *tile,
+                             cudaStream_t st)
+{
+    const int nblk = cdiv(n, kSortTile);
+    for (int shift = 0; shift < bits; shift += 8) {
+        k_digit_hist<<<nblk, 256, 0, st>>>(hist, key_a, n, shift, nblk);
+        scan_exclusive(hist, hist, 256 * nblk, tile, nullptr, st);
+        k_digit_scatter<<<nblk, 32, 0, st>>>(key_b, val_b, key_a, val_a, hist, n, shift, nblk);
+        count_launch(2);
+        std::swap(key_a, key_b);
+        std::swap(val_a, val_b);
+    }
+}
+
+int sort_rows_by_key(int *order, int *key_sorted, const int *key, int n, int nkeys, cudaStream_t st, std::string &err)
+{
+    if (n <= 0) return 0;
+    const int nblk = cdiv(n, kSortTile);
+    int bits = 1;
+    while ((1ll << bits) < nkeys) ++bits;
+    int *scratch = nullptr;
+    const size_t tile_n = (size_t)cdiv(std::max((size_t)n, (size_t)256 * nblk), 1024) + 1;
+    cudaError_t e = cudaMallocAsync((void **)&scratch, sizeof(int) * (2 * (size_t)n + (size_t)256 * nblk + tile_n), st);
+    if (e != cudaSuccess) { err = std::string("sort_rows_by_key scratch: ") + cudaGetErrorString(e); return 1; }
+    int *key_a = key_sorted, *val_a = order, *key_b = scratch, *val_b = scratch + n;
+    int *hist = scratch + 2 * (size_t)n, *tile = hist + (size_t)256 * nblk;
+    e = cudaMemcpyAsync(key_a, key, sizeof(int) * n, cudaMemcpyDeviceToDevice, st);
+    k_iota<<<cdiv(n, 256), 256, 0, st>>>(val_a, n);
+    count_launch();
+    radix_sort_pairs(key_a, val_a, key_b, val_b, n, bits, hist, tile, st);
+    if (e == cudaSuccess && key_a != key_sorted) {
+        e = cudaMemcpyAsync(key_sorted, key_a, sizeof(int) * n, cudaMemcpyDeviceToDevice, st);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(order, val_a, sizeof(int) * n, cudaMemcpyDeviceToDevice, st);
+    }
+    cudaFreeAsync(scratch, st);
+    if (e == cudaSuccess) e = cudaGetLastError();
+    if (e != cudaSuccess) { err = std::string("sort_rows_by_key: ") + cudaGetErrorString(e); return 1; }
+    return 0;
+}
+
 // Device-resident merge.  ty (ny x N), tX (P x N), n (N) are overwritten with the M merged observations in
 // first-occurrence order; returns M, -1 on a CUDA error (message in err), -2 when the rows need the exact host
 // merge (a hash collision, or rows holding NaN): the inputs are then untouched.
@@ -304,14 +347,7 @@ int merge_rows_device(double *ty, double *tX, double *n, int N, int P, int ny, c
     k_iota<<<cdiv(N, 256), 256, 0, st>>>(idx_a, N);
     MG_CK(cudaMemcpyAsync(key_a, rep, sizeof(int) * N, cudaMemcpyDeviceToDevice, st));
     count_launch();
-    for (int shift = 0; shift < bits; shift += 8) {
-        k_digit_hist<<<nblk, 256, 0, st>>>(hist, key_a, N, shift, nblk);
-        scan_exclusive(hist, hist, 256 * nblk, tile, nullptr, st);
-        k_digit_scatter<<<nblk, 32, 0, st>>>(key_b, idx_b, key_a, idx_a, hist, N, shift, nblk);
-        count_launch(2);
-        std::swap(key_a, key_b);
-        std::swap(idx_a, idx_b);
-    }
+    radix_sort_pairs(key_a, idx_a, key_b, idx_b, N, bits, hist, tile, st);
     k_heads<<<cdiv(N, 256), 256, 0, st>>>(head, key_a, N);
     scan_exclusive(gpos, head, N, tile, total, st);
     int M = 0;

@@ -305,6 +305,7 @@ k_devroye_regroup(double *__restrict__ x, const int *__restrict__ n, const doubl
 //           machinery of k_devroye_refill buys nothing here -- lanes differ by proposal branch only.
 // Chains: rows [c N, (c+1) N) meet beta + c * beta_stride and the streams of seed + c (trips never
 // straddle two chains).  psi_out may be null.
+// kOffset (the random-intercept logit): omega_i = PG(n_i, x_i . beta + off_i) and psi_out keeps x_i . beta.
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ void dmma884_f(double &c0, double &c1, double a, double b)
 {
@@ -355,10 +356,11 @@ __device__ __forceinline__ double logit_omega(int ni, double z, uint64_t seed, u
     return sum;
 }
 
+template <bool kOffset>
 __global__ void __launch_bounds__(kThreads, 3)
 k_logit_psi_draw(double *__restrict__ x, double *__restrict__ psi_out, const int *__restrict__ n,
                  const double *__restrict__ tX, const double *__restrict__ beta, int64_t beta_stride,
-                 int chains, int64_t N, int P, StreamId id)
+                 int chains, int64_t N, int P, StreamId id, const double *__restrict__ off)
 {
     BL_PDL_ENTER();
     const unsigned full = 0xffffffffu;
@@ -387,6 +389,7 @@ k_logit_psi_draw(double *__restrict__ x, double *__restrict__ psi_out, const int
         if (i < N) {
             const int64_t g = ch * N + i;
             if (psi_out) psi_out[g] = z;
+            if (kOffset) z += off[g];
             x[g] = logit_omega(n[g], z, id.chain_len ? id.seed + (uint64_t)ch : id.seed, id.obs0 + (uint64_t)i, id.call_id);
         }
     }
@@ -513,7 +516,8 @@ bool logit_psi_draw_ok(const double *tX, int P) { return P % 2 == 0 && (reinterp
 
 // omega (and psi, when psi_out is given) for `chains` blocks of N rows each; see k_logit_psi_draw.
 cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, const double *tX, const double *beta,
-                                  int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t st)
+                                  int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t st,
+                                  const double *off)
 {
     if (N <= 0 || chains <= 0) return cudaSuccess;
     const int64_t trips = (int64_t)chains * ((N + 31) / 32);
@@ -523,7 +527,10 @@ cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, cons
     // the others -- 189 us against 105 + 86 for the two kernels at N = 1M, P = 64; with 8 loads in flight
     // and 24 warps 172 us (P = 32: 104 against 122; P = 128: 252 against 281).
     int grid = (int)std::min<int64_t>(148 * 3, std::max<int64_t>(1, (trips + wpc - 1) / wpc));
-    launch_pdl(k_logit_psi_draw, dim3(grid), dim3(kThreads), 0, st, x, psi_out, n, tX, beta, beta_stride, chains, N, P, id);
+    if (off)
+        launch_pdl(k_logit_psi_draw<true>, dim3(grid), dim3(kThreads), 0, st, x, psi_out, n, tX, beta, beta_stride, chains, N, P, id, off);
+    else
+        launch_pdl(k_logit_psi_draw<false>, dim3(grid), dim3(kThreads), 0, st, x, psi_out, n, tX, beta, beta_stride, chains, N, P, id, off);
     count_launch();
     return cudaGetLastError();
 }

@@ -318,3 +318,25 @@ def nb_multichain(y, X, m0, P0, samp, burn, seed, chains, d0=1.0, dmode="int"):
                                      N, P, samp, burn, int(seed), NB_DMODES[dmode])
     _lib.check(st)
     return beta, d
+
+
+def logit_ri(y, X, n, group, G, m0, P0, a0, b0, tau2_0, samp, burn, seed, flags=0, keep_u=True):
+    """Binomial logit with group random intercepts: logit P(success_i) = x_i' beta + u_{group_i}, u_g ~ N(0, tau2),
+    beta ~ N(m0, P0^-1) (P0 a precision), tau2 ~ IG(a0, b0); y proportions, n trials, group ids in [0, G).  One chain
+    from beta = 0, u = 0, tau2 = tau2_0; burn iterations are discarded.  flags: 0 or UNFUSED (same chain, bit for bit).
+    Returns (beta [samp x P], u [samp x G] or None when keep_u is False, tau2 [samp])."""
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    N, P = X.shape
+    y, n, m0 = _f(y).ravel(), _f(n).ravel(), _f(m0).ravel()
+    group = np.ascontiguousarray(group, dtype=np.int32).ravel()
+    if len(y) != N or len(n) != N or len(group) != N:
+        raise ValueError("y, n and group need one entry per row of X")
+    P0c = np.asfortranarray(_f(P0))
+    beta = np.zeros((max(int(samp), 0), P))
+    tau2 = np.zeros(max(int(samp), 0))
+    u = np.zeros((max(int(samp), 0), max(int(G), 0))) if keep_u else None
+    st = _lib.lib().bl_logit_ri_gibbs(_p(beta), _p(u) if keep_u else None, _p(tau2), _p(y), _p(X), _p(n), _p(group),
+                                      int(G), _p(m0), P0c.ctypes.data, float(a0), float(b0), float(tau2_0), N, P,
+                                      int(samp), int(burn), int(seed), int(flags))
+    _lib.check(st)
+    return beta, u, tau2

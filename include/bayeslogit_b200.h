@@ -298,6 +298,26 @@ int bl_nb_multichain_dev(double *beta, double *d_out, const double *y, const dou
                          const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,
                          uint64_t seed, int dmode, void *stream);
 
+/* Binomial logit with group random intercepts (the GLMM with one grouping factor: patients within hospitals,
+ * pupils within schools, repeated measures on a subject; the reference ships it only as Logit-MixedModel.R):
+ *   logit P(success_i) = x_i' beta + u_{g_i},  u_g ~ N(0, tau2),  beta ~ N(m0, P0^-1),  tau2 ~ IG(a0, b0).
+ * y: proportions [N], n: trials [N] (truncated to int), tX: P x N, group: ids in [0, G) [N], m0 [P], P0: P x P
+ * (a precision).  The chain starts from beta = 0, u = 0, tau2 = tau2_0; each iteration draws omega | beta, u, then
+ * u | omega, beta, tau2 (one normal per group), tau2 | u, then beta | omega, u with the unconstrained draw (streams:
+ * DESIGN.md section 3).  After burn iterations, samp are kept: beta: samp x P (row t = iteration burn + t),
+ * u: samp x G or NULL (no u draws stored), tau2: [samp].  One chain on the current GPU.  flags: 0 or
+ * BL_GIBBS_UNFUSED (same chain, bit for bit).  Refused with their own messages, outputs untouched: G < 1, an id
+ * outside [0, G) (checked on the host by bl_logit_ri_gibbs, on the device before the first iteration by the _dev
+ * entry), a0 / b0 / tau2_0 not finite and positive, N outside [1, 2^31), P < 1, samp < 1, burn < 0, P > 256, any
+ * other flag.  Duplicate rows are not merged. */
+int bl_logit_ri_gibbs(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                      const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                      double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags);
+/* The same on device-resident data (all pointers DEVICE pointers), enqueued on `stream` (a cudaStream_t). */
+int bl_logit_ri_gibbs_dev(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                          const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                          double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags, void *stream);
+
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */
 int bl_comm_unique_id(void *out128);
