@@ -106,6 +106,9 @@ def lib():
     ri = [vp] * 7 + [ci, vp, vp, cd, cd, cd, i64, ci, ci, ci, u64, ci]
     L.bl_logit_ri_gibbs.argtypes = ri
     L.bl_logit_ri_gibbs_dev.argtypes = ri + [vp]
+    rim = [vp] * 7 + [ci, vp, vp, cd, cd, cd, ci, i64, ci, ci, ci, u64, ci]
+    L.bl_logit_ri_multichain.argtypes = rim
+    L.bl_logit_ri_multichain_dev.argtypes = rim + [vp]
     L.bl_comm_unique_id.argtypes = [vp]
     L.bl_comm_init.argtypes = [vp, ci, ci]
     L.bl_comm_init_local.argtypes = [ci, ci]

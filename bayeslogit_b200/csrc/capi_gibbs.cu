@@ -603,6 +603,49 @@ int bl_logit_ri_gibbs_dev(double *beta, double *u, double *tau2, const double *y
     return 0;
 }
 
+int bl_logit_ri_multichain(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                           const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                           double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int flags)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !n || !group || !m0 || !P0) return report("logit_ri_multichain: null argument", nullptr);
+    std::string err;
+    // checked before any buffer is made: the device driver repeats the checks
+    if (logit_ri_multichain_check(chains, N, P, G, samp, burn, a0, b0, tau2_0, flags, err)) return report(err, nullptr);
+    for (int64_t i = 0; i < N; ++i)
+        if (group[i] < 0 || group[i] >= G) return report(kLogitRiMultichainBadIdMsg, nullptr);
+    Dev d;
+    double *dy = d.put(y, N, err), *dX = d.put(tX, (size_t)N * P, err), *dn = d.put(n, N, err);   // one copy of the data
+    double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
+    int *dg = (int *)d.put_bytes(group, sizeof(int) * (size_t)N, err);
+    const size_t nb = (size_t)chains * samp * P, nt = (size_t)chains * samp, nu = (size_t)chains * samp * G;
+    double *dbeta = d.put(nullptr, nb, err), *dtau2 = d.put(nullptr, nt, err);
+    double *du = u ? d.put(nullptr, nu, err) : nullptr;
+    if (!err.empty()) return report(err, nullptr);
+    if (logit_ri_multichain_device(dbeta, du, dtau2, dy, dX, dn, dg, G, dm0, dP0, a0, b0, tau2_0, chains, N, P, samp, burn,
+                                   seed, flags, (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * nb, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemcpy(tau2, dtau2, sizeof(double) * nt, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && u) e = cudaMemcpy(u, du, sizeof(double) * nu, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
+int bl_logit_ri_multichain_dev(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                               const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                               double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
+                               void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !n || !group || !m0 || !P0) return report("logit_ri_multichain: null argument", nullptr);
+    std::string err;
+    if (logit_ri_multichain_device(beta, u, tau2, y, tX, n, group, G, m0, P0, a0, b0, tau2_0, chains, N, P, samp, burn,
+                                   seed, flags, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
 int bl_comm_unique_id(void *out128)
 {
     std::string err;

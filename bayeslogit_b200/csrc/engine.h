@@ -64,9 +64,11 @@ cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, cons
                                   int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream,
                                   const double *off = nullptr);
 // The same for `chains` chains that share ONE set of N rows (n [N], tX P x N): chain c meets beta + c * beta_stride
-// and the streams of id.seed + c; x: omega [chains][N].  Same conditions on P and tX.
+// and the streams of id.seed + c; x: omega [chains][N].  Same conditions on P and tX.  off [chains][N] (the
+// random-intercept logit): omega = PG(n_i, x_i . beta_c + off[c][i]), psi_out [chains][N] keeps x_i . beta_c.
 cudaError_t launch_logit_psi_draw_shared(double *x, const int *n, const double *tX, const double *beta,
-                                         int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream);
+                                         int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t stream,
+                                         double *psi_out = nullptr, const double *off = nullptr);
 
 // rpg_hybrid through regime binning (pg_hybrid.cu); num <= 2^31-1, `work` = device scratch of
 // hybrid_workspace_bytes(num) bytes that stays valid until the stream has drained.
@@ -92,12 +94,22 @@ int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const dou
 // Binomial logit with group random intercepts, one chain (gibbs.cu).  logit_ri_check refuses what the driver cannot
 // run (every argument but the ids); the driver checks the ids on the device before anything else runs.
 int logit_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, int flags,
-                   std::string &err);
+                   std::string &err, const char *who = "logit_ri_gibbs");   // who: the messages' prefix
 extern const char *const kLogitRiBadIdMsg;
 int logit_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, const double *y, const double *tX,
                           const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
                           double b0, double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
                           cudaStream_t st, std::string &err);
+// Several random-intercept chains on one data set (y, n, group [N], tX P x N, shared); beta_out: [chains][samp][P],
+// u_out: [chains][samp][G] or null, tau2_out: [chains][samp].  The check refuses every argument the driver cannot run
+// but the ids, before anything is allocated or launched; the driver checks the ids on the device first.
+int logit_ri_multichain_check(int chains, int64_t N, int P, int G, int samp, int burn, double a0, double b0,
+                              double tau2_0, int flags, std::string &err);
+extern const char *const kLogitRiMultichainBadIdMsg;
+int logit_ri_multichain_device(double *beta_out, double *u_out, double *tau2_out, const double *y, const double *tX,
+                               const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
+                               double b0, double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
+                               int flags, cudaStream_t st, std::string &err);
 // shared_rows: every chain runs on the same N rows (y, n [N], tX P x N) instead of rows [c N, (c+1) N) of its own
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,

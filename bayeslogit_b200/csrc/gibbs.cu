@@ -1244,17 +1244,18 @@ int mlogit_multichain_device(double *beta_out, const double *ty, const double *t
 // tau2_out [samp].  One chain on one GPU; device pointers throughout.
 // ------------------------------------------------------------------------------------
 int logit_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, int flags,
-                   std::string &err)
+                   std::string &err, const char *who)
 {
-    if (flags & ~BL_GIBBS_UNFUSED) { err = "logit_ri_gibbs: unknown flag (only BL_GIBBS_UNFUSED is accepted)"; return 1; }
+    const std::string w = std::string(who) + ": ";
+    if (flags & ~BL_GIBBS_UNFUSED) { err = w + "unknown flag (only BL_GIBBS_UNFUSED is accepted)"; return 1; }
     if (N < 1 || N >= (1LL << 31) || P < 1 || samp < 1 || burn < 0 || (int64_t)samp + burn >= (1LL << 31)) {
-        err = "logit_ri_gibbs: bad dimensions (need 1 <= N < 2^31, P >= 1, samp >= 1, burn >= 0)";
+        err = w + "bad dimensions (need 1 <= N < 2^31, P >= 1, samp >= 1, burn >= 0)";
         return 1;
     }
-    if (P > 256) { err = "logit_ri_gibbs: P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
-    if (G < 1) { err = "logit_ri_gibbs: G must be at least 1"; return 1; }
+    if (P > 256) { err = w + "P > 256 covariates is not supported by the single-CTA beta draw"; return 1; }
+    if (G < 1) { err = w + "G must be at least 1"; return 1; }
     if (!(std::isfinite(a0) && a0 > 0.0) || !(std::isfinite(b0) && b0 > 0.0) || !(std::isfinite(tau2_0) && tau2_0 > 0.0)) {
-        err = "logit_ri_gibbs: a0, b0 and tau2_0 must be finite and positive";
+        err = w + "a0, b0 and tau2_0 must be finite and positive";
         return 1;
     }
     return 0;
@@ -1328,24 +1329,25 @@ int logit_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, con
             e = launch_logit_psi_draw(s.w, eta, shape, tX, bprev, 0, 1, N, P, id, st, off);
         } else {
             s.xbeta(eta, bprev, nullptr, 0.0);
-            launch_pdl(k_ri_psi, dim3(rgrid), dim3(256), 0, st, s.psi, (const double *)eta, (const double *)off, N);
+            launch_pdl(k_ri_psi<false>, dim3(rgrid), dim3(256), 0, st, s.psi, (const double *)eta, (const double *)off, N);
             count_launch();
             e = launch_devroye_refill(s.w, shape, s.psi, N, id, st);
         }
         if (e != cudaSuccess) { err = std::string("logit_ri_gibbs: ") + cudaGetErrorString(e); return 1; }
         tmr.mark("psi+draw");
-        launch_pdl(k_ri_group_sums, dim3(nchunks), dim3(kRiThreads), 0, st, S, R, edge, (const int *)order,
-                   (const int *)gs, (const int *)goff, (const double *)s.w, (const double *)eta, (const double *)kappa, N);
+        launch_pdl(k_ri_group_sums<false>, dim3(nchunks), dim3(kRiThreads), 0, st, S, R, edge, (const int *)order,
+                   (const int *)gs, (const int *)goff, (const double *)s.w, (const double *)eta, (const double *)kappa, N, G);
         tmr.mark("group sums");
         const bool rec = t >= burn;
-        launch_pdl(k_ri_draw_u, dim3(nublk), dim3(32 * kRiDrawWarps), 0, st, u,
+        launch_pdl(k_ri_draw_u<false>, dim3(nublk), dim3(32 * kRiDrawWarps), 0, st, u,
                    rec && u_out ? u_out + (size_t)G * (t - burn) : (double *)nullptr, usq, (const double *)S,
-                   (const double *)R, (const double *)edge, (const int *)goff, (const double *)tau2, G, seed, (uint32_t)t);
-        launch_pdl(k_ri_draw_tau2, dim3(1), dim3(256), 0, st, tau2, rec ? tau2_out + (t - burn) : (double *)nullptr,
-                   (const double *)usq, nublk, G, a0, b0, seed, (uint32_t)t);
+                   (const double *)R, (const double *)edge, (const int *)goff, (const double *)tau2, G, seed, (uint32_t)t,
+                   (int64_t)0, nchunks);
+        launch_pdl(k_ri_draw_tau2<false>, dim3(1), dim3(256), 0, st, tau2, rec ? tau2_out + (t - burn) : (double *)nullptr,
+                   (const double *)usq, nublk, G, a0, b0, seed, (uint32_t)t, (int64_t)0);
         tmr.mark("u+tau2");
-        launch_pdl(k_ri_rows, dim3(rgrid), dim3(256), 0, st, off, v, group, (const double *)u, (const double *)s.w,
-                   (const double *)kappa, N);
+        launch_pdl(k_ri_rows<false>, dim3(rgrid), dim3(256), 0, st, off, v, group, (const double *)u, (const double *)s.w,
+                   (const double *)kappa, N, G);
         count_launch(4);
         tmr.mark("rows");
         s.xtv(v, 1.0, nullptr, nullptr, 0.0);                                 // X'(kappa - omega o u_g)
@@ -1360,6 +1362,221 @@ int logit_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, con
     }
     GB_CK(cudaGetLastError());
     return s.check_status(err, "logit_ri_gibbs");
+}
+
+// ------------------------------------------------------------------------------------
+// Several random-intercept chains on ONE data set (bl_logit_ri_multichain): chain c is, bit for bit,
+// logit_ri_gibbs_device(..., seed + c) -- beta, u and tau2, streams (seed + c, i, t), (seed + c, 2^63 + g, t),
+// (seed + c, 2^64 - 4, t), (seed + c, 2^64 - 1, t) -- and every stage is one launch for all chains, with the single
+// chain's kernel choice and summation order:
+//   once  : kappa, the shapes, P0 m0, the stable sort of the rows by group and the groups' offsets, shared.
+//   psi   : fused (even P, aligned X): one chain k_logit_psi_draw<true>; more, k_logit_psi_draw_shared<true> (one read
+//           of X for 8 chains, eta and the offset per chain).  Unfused: eta from k_xbeta_mma (one chain),
+//           k_xbeta_shared or k_xbeta with a chain grid dimension, k_ri_psi, then the per-lane refill draw over
+//           chains * N (chain, row) pairs keyed by chain.
+//   groups: k_ri_group_sums, k_ri_draw_u, k_ri_draw_tau2, k_ri_rows with a chain grid dimension (fixed-order sums;
+//           one chain: the single chain's instantiations).
+//   sums  : the single chain's X'v and Gram slab partition and kernels with a chain grid dimension, X stride 0;
+//           X'(kappa - omega o u_g) into the tail of each chain's sums.
+//   beta  : one plain draw per chain side by side (Sweep::beta_draw's instantiation; global scratch per chain where
+//           P is too large for shared memory).  Burn-in betas in a per-chain slot, recorded ones straight into beta_out.
+// ------------------------------------------------------------------------------------
+int logit_ri_multichain_check(int chains, int64_t N, int P, int G, int samp, int burn, double a0, double b0,
+                              double tau2_0, int flags, std::string &err)
+{
+    if (logit_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, flags, err, "logit_ri_multichain")) return 1;
+    if (chains < 1) { err = "logit_ri_multichain: chains must be at least 1"; return 1; }
+    // the chain is a y grid dimension of the group, row, X'v and Gram launches
+    if (chains > kMaxGridChains) { err = "logit_ri_multichain: chains must be at most 65535"; return 1; }
+    if ((int64_t)chains * N >= (1LL << 31)) {
+        err = "logit_ri_multichain: chains * N must stay below 2^31 observations per call";
+        return 1;
+    }
+    if ((int64_t)chains * G >= (1LL << 31)) { err = "logit_ri_multichain: chains * G must stay below 2^31 groups per call"; return 1; }
+    return 0;
+}
+
+const char *const kLogitRiMultichainBadIdMsg = "logit_ri_multichain: group ids must lie in [0, G)";
+
+int logit_ri_multichain_device(double *beta_out, double *u_out, double *tau2_out, const double *y, const double *tX,
+                               const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
+                               double b0, double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
+                               int flags, cudaStream_t st, std::string &err)
+{
+    if (logit_ri_multichain_check(chains, N, P, G, samp, burn, a0, b0, tau2_0, flags, err)) return 1;
+    DevMem mem;
+    mem.st = st;
+    // the ids first: a refusal leaves the outputs untouched and launches no iteration
+    int *bad;
+    GB_CK(mem.get(&bad, 1));
+    GB_CK(cudaMemsetAsync(bad, 0, sizeof(int), st));
+    k_ri_check_ids<<<(int)std::min<int64_t>(148 * 8, cdiv(N, 256)), 256, 0, st>>>(bad, group, N, G);
+    count_launch();
+    int hbad = 0;
+    GB_CK(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (hbad) { err = kLogitRiMultichainBadIdMsg; return 1; }
+
+    const int K = chains;
+    const int64_t T = (int64_t)K * N;
+    const Slabs sl = slab_partition(N, P);
+    const int nt = sl.nt, tiles = nt * (nt + 1) / 2, slabs_total = nt > 1 ? 2 * sl.nslab : sl.nslab;
+    const bool packed = gram_packed(P);
+    const size_t accn = (size_t)P * P + P;
+    const BetaSmem bs = beta_smem_of(P);
+    const bool lean = P <= 64 && !kSlowBeta;            // Sweep::beta_draw's plain-draw instantiation
+    const bool fused = !(flags & BL_GIBBS_UNFUSED) && logit_psi_draw_ok(tX, P);
+    const bool mma = xbeta_mma_ok(tX, P);
+    const int nchunks = cdiv(N, kRiChunk), nublk = cdiv(G, kRiDrawWarps);
+    const int rgrid = (int)std::min<int64_t>(148 * 8, cdiv(N, 256));
+    // the fused kernels read the shapes of the N shared rows; the refill draw reads one per (chain, row) pair
+    const int64_t nshape = fused ? N : T;
+    double *psi, *w, *eta, *off, *v, *kappa, *acc, *part, *xtv_part, *bprior, *bscr, *S, *R, *edge, *u, *usq, *tau2,
+        *gwork = nullptr;
+    int *shape, *order, *gs, *goff, *status;
+    GB_CK(mem.get(&psi, fused ? 1 : T));
+    GB_CK(mem.get(&w, T));
+    GB_CK(mem.get(&eta, T));
+    GB_CK(mem.get(&off, T));
+    GB_CK(mem.get(&v, T));
+    GB_CK(mem.get(&kappa, N));
+    GB_CK(mem.get(&shape, nshape));
+    GB_CK(mem.get(&order, N));
+    GB_CK(mem.get(&gs, N));
+    GB_CK(mem.get(&goff, (size_t)G + 1));
+    GB_CK(mem.get(&acc, accn * K));
+    GB_CK(mem.get(&part, (size_t)K * tiles * sl.nslab * 2 * kGramTile * kGramTile));
+    GB_CK(mem.get(&xtv_part, (size_t)K * sl.xtv_slabs * P));
+    GB_CK(mem.get(&bprior, (size_t)K * P));             // P0 m0, one copy per chain: k_beta_draw reads chain c's at + c P
+    GB_CK(mem.get(&bscr, (size_t)K * P));               // burn-in betas [chain][P]
+    GB_CK(mem.get(&S, (size_t)K * G));
+    GB_CK(mem.get(&R, (size_t)K * G));
+    GB_CK(mem.get(&edge, (size_t)K * 4 * nchunks));
+    GB_CK(mem.get(&u, (size_t)K * G));
+    GB_CK(mem.get(&usq, (size_t)K * nublk));
+    GB_CK(mem.get(&tau2, K));
+    GB_CK(mem.get(&status, 1));
+    if (!bs.use_smem) GB_CK(mem.get(&gwork, beta_gwork_doubles(P) * K));
+    GB_CK(cudaMemsetAsync(status, 0, sizeof(int), st));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRows, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(true)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false)));
+    GB_CK(cudaFuncSetAttribute(k_gram_partial<kGramRowsDiag, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (int)gram_smem_bytes(false, true)));
+    if (bs.use_smem && bs.plain > 48 * 1024)
+        GB_CK(cudaFuncSetAttribute(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>,
+                                   cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bs.plain));
+
+    k_kappa<<<cdiv(N, 256), 256, 0, st>>>(kappa, y, n, 0.0, N);
+    k_shape_int<<<cdiv(N, 256), 256, 0, st>>>(shape, n, N);
+    k_matvec<<<cdiv(P, 128), 128, 0, st>>>(bprior, P0, m0, P);
+    k_fill<<<cdiv(K, 256), 256, 0, st>>>(tau2, tau2_0, (int64_t)K);
+    count_launch(4);
+    for (int c = 1; c < K; ++c)
+        GB_CK(cudaMemcpyAsync(bprior + (size_t)P * c, bprior, sizeof(double) * P, cudaMemcpyDeviceToDevice, st));
+    for (int64_t r = N; r < nshape; r += N)
+        GB_CK(cudaMemcpyAsync(shape + r, shape, sizeof(int) * N, cudaMemcpyDeviceToDevice, st));
+    // rows sorted by group (stable: increasing row order inside a group) and the groups' first positions, shared
+    if (sort_rows_by_key(order, gs, group, (int)N, G, st, err)) return 1;
+    k_ri_offsets<<<cdiv(N + 1, 256), 256, 0, st>>>(goff, gs, N, G);
+    count_launch();
+    GB_CK(cudaMemsetAsync(off, 0, sizeof(double) * T, st));
+    GB_CK(cudaMemsetAsync(bscr, 0, sizeof(double) * P * (size_t)K, st));
+
+    const int64_t bstride = (int64_t)P * samp;          // chain stride of beta_out
+    const int xgrid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (N + 255) / 256));     // Sweep::xbeta's grid
+    const int64_t items = (N + 31) / 32 * ((K + kGroupChains - 1) / kGroupChains);
+    const int sgrid = (int)std::min<int64_t>(148 * 8, std::max<int64_t>(1, (items + 7) / 8));
+    static const int tn_flags = getenv("BL_BETA_NO_SPEC") ? 3 : 1;
+    // one chain: the single chain's instantiations of the group and row kernels (no chain arithmetic)
+    const auto ri_psi = K > 1 ? k_ri_psi<true> : k_ri_psi<false>;
+    const auto ri_group_sums = K > 1 ? k_ri_group_sums<true> : k_ri_group_sums<false>;
+    const auto ri_draw_u = K > 1 ? k_ri_draw_u<true> : k_ri_draw_u<false>;
+    const auto ri_draw_tau2 = K > 1 ? k_ri_draw_tau2<true> : k_ri_draw_tau2<false>;
+    const auto ri_rows = K > 1 ? k_ri_rows<true> : k_ri_rows<false>;
+    StageTimer tmr;
+    tmr.st = st;
+    for (int t = 0; t < burn + samp; ++t) {
+        // the beta every chain conditions on: its burn-in slot, or its last recorded draw
+        const double *bprev = t <= burn ? bscr : beta_out + (size_t)P * (t - 1 - burn);
+        const int64_t pstride = t <= burn ? (int64_t)P : bstride;
+        const bool rec = t >= burn;
+        double *bnext = rec ? beta_out + (size_t)P * (t - burn) : bscr;
+        const int64_t nstride = rec ? bstride : (int64_t)P;
+        tmr.arm(t == burn + samp - 1);
+        // one chain: the plain stream is the chain-keyed one, and the single chain's kernels run
+        const StreamId id{seed, 0, (uint32_t)t, K > 1 ? (uint32_t)N : 0u};
+        cudaError_t e;
+        if (fused && K == 1) {
+            e = launch_logit_psi_draw(w, eta, shape, tX, bprev, 0, 1, N, P, id, st, off);
+        } else if (fused) {
+            e = launch_logit_psi_draw_shared(w, shape, tX, bprev, pstride, K, N, P, id, st, eta, off);
+        } else {
+            if (mma && K == 1)
+                launch_pdl(k_xbeta_mma<false>, dim3(xgrid), dim3(256), 0, st, eta, N, tX, N * P, bprev, (int64_t)0, 1, N, P,
+                           (const double *)nullptr, 0.0, 0.0, MlogitNext{});
+            else if (mma)
+                launch_pdl(k_xbeta_shared, dim3(sgrid), dim3(256), 0, st, eta, tX, bprev, pstride, K, N, P, 0.0);
+            else
+                k_xbeta<<<dim3(xgrid, K), 256, P * sizeof(double), st>>>(eta, tX, bprev, nullptr, 0.0, 0.0, N, P, pstride);
+            launch_pdl(ri_psi, dim3(rgrid, K), dim3(256), 0, st, psi, (const double *)eta, (const double *)off, N);
+            count_launch(2);
+            e = launch_devroye_refill(w, shape, psi, T, id, st);
+        }
+        if (e != cudaSuccess) { err = std::string("logit_ri_multichain: ") + cudaGetErrorString(e); return 1; }
+        tmr.mark("psi+draw");
+        launch_pdl(ri_group_sums, dim3(nchunks, K), dim3(kRiThreads), 0, st, S, R, edge, (const int *)order,
+                   (const int *)gs, (const int *)goff, (const double *)w, (const double *)eta, (const double *)kappa, N, G);
+        tmr.mark("group sums");
+        launch_pdl(ri_draw_u, dim3(nublk, K), dim3(32 * kRiDrawWarps), 0, st, u,
+                   rec && u_out ? u_out + (size_t)G * (t - burn) : (double *)nullptr, usq, (const double *)S,
+                   (const double *)R, (const double *)edge, (const int *)goff, (const double *)tau2, G, seed, (uint32_t)t,
+                   (int64_t)G * samp, nchunks);
+        launch_pdl(ri_draw_tau2, dim3(K), dim3(256), 0, st, tau2, rec ? tau2_out + (t - burn) : (double *)nullptr,
+                   (const double *)usq, nublk, G, a0, b0, seed, (uint32_t)t, (int64_t)samp);
+        tmr.mark("u+tau2");
+        launch_pdl(ri_rows, dim3(rgrid, K), dim3(256), 0, st, off, v, group, (const double *)u, (const double *)w,
+                   (const double *)kappa, N, G);
+        count_launch(4);
+        tmr.mark("rows");
+        // X'(kappa - omega o u_g) of every chain into the tail of its sums
+        launch_xtv(dim3(sl.xtv_slabs, K), st, xtv_part, tX, 0, v, 1.0, nullptr, nullptr, 0.0, N, P, nullptr);
+        launch_pdl(k_xtv_reduce, dim3(cdiv(P, 128), K), dim3(128), 0, st, acc + (size_t)P * P, (const double *)nullptr,
+                   (const double *)nullptr, xtv_part, P, sl.xtv_slabs, (int64_t)accn);
+        count_launch(2);
+        tmr.mark("xtv");
+        if (nt > 1)
+            launch_pdl(k_gram_partial<kGramRows, false>, dim3(sl.nslab, tiles, K), dim3(256), gram_smem_bytes(true), st,
+                       part, tX, (int64_t)0, w, N, P, nt, sl.nslab_diag, (const double *)nullptr);
+        else if (packed)
+            launch_pdl(k_gram_partial<kGramRowsDiag, true, true>, dim3(sl.nslab, tiles, K), dim3(256),
+                       gram_smem_bytes(false, true), st, part, tX, (int64_t)0, w, N, P, nt, 0, (const double *)nullptr);
+        else
+            launch_pdl(k_gram_partial<kGramRowsDiag, true>, dim3(sl.nslab, tiles, K), dim3(256), gram_smem_bytes(false),
+                       st, part, tX, (int64_t)0, w, N, P, nt, 0, (const double *)nullptr);
+        launch_pdl(k_gram_reduce, dim3(cdiv((int64_t)P * P, 32), K), dim3(256), 0, st, acc, (const double *)nullptr,
+                   part, P, nt, slabs_total, PeerPush{}, packed ? 1 : 0, 2 * sl.nslab_diag, 0);
+        count_launch(2);
+        tmr.mark("gram");
+        if (bs.use_smem)
+            launch_pdl(lean ? k_beta_draw<true, true> : k_beta_draw<true, false>, dim3(K), dim3(256), bs.plain, st,
+                       (int)kBetaPlain, (const double *)acc, P0, (const double *)bprior, 1, (const double *)nullptr, bnext,
+                       (double *)nullptr, P, seed, (uint32_t)t, status, PeerWait{}, nstride, (const double *)nullptr,
+                       tn_flags);
+        else
+            k_beta_draw<false><<<K, 256, 0, st>>>(kBetaPlain, acc, P0, bprior, 1, nullptr, bnext, gwork, P, seed,
+                                                  (uint32_t)t, status, PeerWait{}, nstride, nullptr, 0);
+        count_launch();
+        tmr.mark("beta");
+        tmr.report("logit_ri multichain");
+    }
+    GB_CK(cudaGetLastError());
+    int h = 0;
+    GB_CK(cudaMemcpyAsync(&h, status, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (h != 0) { err = "logit_ri_multichain: a chain's posterior precision is not positive definite"; return 1; }
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------

@@ -1506,6 +1506,11 @@ static __global__ void k_mlogit_offsets(double *__restrict__ c, double *__restri
 // a group that lies inside it straight to S, R; a group that crosses chunk boundaries leaves its first piece as the
 // tail of its first chunk and the rest as the heads of the following chunks, which k_ri_draw_u adds in chunk order.
 // No floating-point atomics: every sum is bit-identical from run to run, whatever the group sizes.
+// Several chains on one data set (logit_ri_multichain_device), kChains: the chain is a grid dimension of every
+// per-iteration kernel (blockIdx.y; k_ri_draw_tau2: blockIdx.x), chain c keeps its own rows' state at + c N (eta, off,
+// v, omega, psi), its groups' at + c G (S, R, u), its chunks' edges, partials and tau2, and draws from the streams of
+// seed + c; the sorted order, the offsets and kappa are shared.  Chain c sums in the single chain's order: bit for bit
+// its run.  The single chain's instantiations (kChains false) leave the chain arguments unread.
 // ---------------------------------------------------------------------------------
 constexpr uint64_t kRiGroupObs0 = 0x8000000000000000ull;   // u_g: first normal of the stream (seed, 2^63 + g, call)
 constexpr uint64_t kRiTau2Obs = 0xFFFFFFFFFFFFFFFCull;     // tau2: the gamma variate of the stream (seed, 2^64 - 4, call)
@@ -1531,11 +1536,18 @@ static __global__ void k_ri_offsets(int *__restrict__ goff, const int *__restric
     for (int g = lo; g <= hi; ++g) goff[g] = (int)k;
 }
 
-// unfused path: psi_i = eta_i + off_i
+// unfused path: psi_i = eta_i + off_i (kChains: chain blockIdx.y at + c N)
+template <bool kChains>
 static __global__ void k_ri_psi(double *__restrict__ psi, const double *__restrict__ eta, const double *__restrict__ off,
                                 int64_t N)
 {
     BL_PDL_ENTER();
+    if (kChains) {
+        const size_t ch = (size_t)blockIdx.y * N;
+        psi += ch;
+        eta += ch;
+        off += ch;
+    }
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x)
         psi[i] = eta[i] + off[i];
 }
@@ -1551,13 +1563,22 @@ __device__ __forceinline__ RiSeg ri_seg_join(const RiSeg &a, const RiSeg &b)
 }
 
 // One CTA per chunk of kRiChunk sorted positions, kRiItems consecutive positions per thread.  edge[4 c ..]: head
-// (s, r) and tail (s, r) pieces of chunk c (written only when a group crosses that edge).
+// (s, r) and tail (s, r) pieces of chunk c (written only when a group crosses that edge).  kChains: chain blockIdx.y,
+// S, R at + c G, edge at + 4 c gridDim.x, omega and eta at + c N.
+template <bool kChains>
 static __global__ void __launch_bounds__(kRiThreads)
 k_ri_group_sums(double *__restrict__ S, double *__restrict__ R, double *__restrict__ edge, const int *__restrict__ order,
                 const int *__restrict__ gs, const int *__restrict__ goff, const double *__restrict__ w,
-                const double *__restrict__ eta, const double *__restrict__ kappa, int64_t N)
+                const double *__restrict__ eta, const double *__restrict__ kappa, int64_t N, int G)
 {
     BL_PDL_ENTER();
+    if (kChains) {
+        S += (size_t)blockIdx.y * G;
+        R += (size_t)blockIdx.y * G;
+        edge += (size_t)blockIdx.y * 4 * gridDim.x;
+        w += (size_t)blockIdx.y * N;
+        eta += (size_t)blockIdx.y * N;
+    }
     __shared__ RiSeg wtot[kRiThreads / 32], wcarry[kRiThreads / 32];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t p0 = (int64_t)blockIdx.x * kRiChunk, p1 = min(p0 + (int64_t)kRiChunk, N);
@@ -1630,12 +1651,27 @@ k_ri_group_sums(double *__restrict__ S, double *__restrict__ R, double *__restri
 // A warp per group: (S_g, R_g) -- the chunk's sums, or the pieces of a group that crosses chunks added in chunk order --
 // then u_g = R_g / prec + z_g / sqrt(prec), prec = S_g + 1 / tau2 (an empty group draws from its prior), z_g the first
 // normal of the stream (seed, 2^63 + g, call).  usq_part[b] = sum of u_g^2 over the CTA's groups, in group order.
+// kChains: chain blockIdx.y, u, S, R at + c G, u_rec at + c rec_stride, usq_part at + c gridDim.x, edge at
+// + 4 c nchunks, tau2 at + c, seed + c.
+template <bool kChains>
 static __global__ void __launch_bounds__(32 * kRiDrawWarps)
 k_ri_draw_u(double *__restrict__ u, double *__restrict__ u_rec, double *__restrict__ usq_part,
             const double *__restrict__ S, const double *__restrict__ R, const double *__restrict__ edge,
-            const int *__restrict__ goff, const double *__restrict__ tau2, int G, uint64_t seed, uint32_t call)
+            const int *__restrict__ goff, const double *__restrict__ tau2, int G, uint64_t seed, uint32_t call,
+            int64_t rec_stride, int nchunks)
 {
     BL_PDL_ENTER();
+    if (kChains) {
+        const unsigned ch = blockIdx.y;
+        u += (size_t)ch * G;
+        if (u_rec) u_rec += ch * rec_stride;
+        usq_part += (size_t)ch * gridDim.x;
+        S += (size_t)ch * G;
+        R += (size_t)ch * G;
+        edge += (size_t)ch * 4 * nchunks;
+        tau2 += ch;
+        seed += ch;
+    }
     __shared__ double sq[kRiDrawWarps];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int g = blockIdx.x * kRiDrawWarps + warp;
@@ -1683,12 +1719,21 @@ k_ri_draw_u(double *__restrict__ u, double *__restrict__ u_rec, double *__restri
 }
 
 // One CTA: sum of u_g^2 over the partials in a fixed order, then tau2 = (b0 + sum / 2) / gamma, gamma ~ Gamma(a0 + G/2, 1)
-// from the stream (seed, 2^64 - 4, call) (Marsaglia-Tsang, PhiloxSource::gamma).
+// from the stream (seed, 2^64 - 4, call) (Marsaglia-Tsang, PhiloxSource::gamma).  kChains: chain blockIdx.x, tau2 at
+// + c, tau2_rec at + c rec_stride, usq_part at + c nparts, seed + c.
+template <bool kChains>
 static __global__ void __launch_bounds__(256)
 k_ri_draw_tau2(double *__restrict__ tau2, double *__restrict__ tau2_rec, const double *__restrict__ usq_part, int nparts,
-               int G, double a0, double b0, uint64_t seed, uint32_t call)
+               int G, double a0, double b0, uint64_t seed, uint32_t call, int64_t rec_stride)
 {
     BL_PDL_ENTER();
+    if (kChains) {
+        const unsigned ch = blockIdx.x;
+        tau2 += ch;
+        if (tau2_rec) tau2_rec += ch * rec_stride;
+        usq_part += (size_t)ch * nparts;
+        seed += ch;
+    }
     __shared__ double red[256];
     double s = 0.0;
     for (int k = threadIdx.x; k < nparts; k += 256) s += usq_part[k];
@@ -1708,11 +1753,20 @@ k_ri_draw_tau2(double *__restrict__ tau2, double *__restrict__ tau2_rec, const d
 }
 
 // The rows after the u draw: off_i = u_{g_i} (the next iteration's psi offset), v_i = kappa_i - omega_i off_i.
+// kChains: chain blockIdx.y, off, v, omega at + c N, u at + c G.
+template <bool kChains>
 static __global__ void k_ri_rows(double *__restrict__ off, double *__restrict__ v, const int *__restrict__ group,
                                  const double *__restrict__ u, const double *__restrict__ w,
-                                 const double *__restrict__ kappa, int64_t N)
+                                 const double *__restrict__ kappa, int64_t N, int G)
 {
     BL_PDL_ENTER();
+    if (kChains) {
+        const size_t ch = (size_t)blockIdx.y * N;
+        off += ch;
+        v += ch;
+        w += ch;
+        u += (size_t)blockIdx.y * G;
+    }
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
         const double ug = u[group[i]];
         off[i] = ug;

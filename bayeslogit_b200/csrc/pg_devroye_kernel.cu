@@ -408,13 +408,17 @@ k_logit_psi_draw(double *__restrict__ x, double *__restrict__ psi_out, const int
 //           bit for bit the chain k_logit_psi_draw runs on a private copy of the rows (the MMA forms each
 //           output element from its own row and column only).
 // omega: [chains][N].
+// kOffset (the random-intercept logit, bl_logit_ri_multichain): omega = PG(n_i, x_i . beta_c + off[c][i]) and
+// psi_out[c][i] keeps x_i . beta_c, as k_logit_psi_draw<true> does for one chain.
 // ---------------------------------------------------------------------------------------------
 constexpr int kGroup = 8;                       // chains per pass: the 8 columns of an m8n8k4 tile
 constexpr int kTileLd = kGroup + 1;             // odd row stride: lane l reading row l is conflict-free
 
+template <bool kOffset>
 __global__ void __launch_bounds__(kThreads, 3)
 k_logit_psi_draw_shared(double *__restrict__ x, const int *__restrict__ n, const double *__restrict__ tX,
-                        const double *__restrict__ beta, int64_t beta_stride, int chains, int64_t N, int P, StreamId id)
+                        const double *__restrict__ beta, int64_t beta_stride, int chains, int64_t N, int P, StreamId id,
+                        double *__restrict__ psi_out, const double *__restrict__ off)
 {
     BL_PDL_ENTER();
     __shared__ double tile[kThreads / 32][32 * kTileLd];
@@ -445,9 +449,16 @@ k_logit_psi_draw_shared(double *__restrict__ x, const int *__restrict__ n, const
         __syncwarp();
         if (i < N) {
             const int ni = n[i];
-            for (int k = 0; k < kg; ++k)
-                x[(int64_t)(g0 + k) * N + i] = logit_omega(ni, pt[lane * kTileLd + k], id.seed + (uint64_t)(g0 + k),
-                                                           id.obs0 + (uint64_t)i, id.call_id);
+            for (int k = 0; k < kg; ++k) {
+                if (kOffset) {
+                    const int64_t gk = (int64_t)(g0 + k) * N + i;
+                    const double z = pt[lane * kTileLd + k];
+                    psi_out[gk] = z;
+                    x[gk] = logit_omega(ni, z + off[gk], id.seed + (uint64_t)(g0 + k), id.obs0 + (uint64_t)i, id.call_id);
+                } else
+                    x[(int64_t)(g0 + k) * N + i] = logit_omega(ni, pt[lane * kTileLd + k], id.seed + (uint64_t)(g0 + k),
+                                                               id.obs0 + (uint64_t)i, id.call_id);
+            }
         }
     }
 }
@@ -535,16 +546,23 @@ cudaError_t launch_logit_psi_draw(double *x, double *psi_out, const int *n, cons
     return cudaGetLastError();
 }
 
-// omega of `chains` chains on one set of N rows; see k_logit_psi_draw_shared.
+// omega of `chains` chains on one set of N rows (with psi_out and off: k_logit_psi_draw_shared<true>); see
+// k_logit_psi_draw_shared.
 cudaError_t launch_logit_psi_draw_shared(double *x, const int *n, const double *tX, const double *beta,
-                                         int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t st)
+                                         int64_t beta_stride, int chains, int64_t N, int P, StreamId id, cudaStream_t st,
+                                         double *psi_out, const double *off)
 {
     if (N <= 0 || chains <= 0) return cudaSuccess;
     const int64_t items = (N + 31) / 32 * ((chains + kGroup - 1) / kGroup);
     const int wpc = kThreads / 32;
     // the occupancy of k_logit_psi_draw (three CTAs of 80 registers per SM)
     int grid = (int)std::min<int64_t>(148 * 3, std::max<int64_t>(1, (items + wpc - 1) / wpc));
-    launch_pdl(k_logit_psi_draw_shared, dim3(grid), dim3(kThreads), 0, st, x, n, tX, beta, beta_stride, chains, N, P, id);
+    if (off)
+        launch_pdl(k_logit_psi_draw_shared<true>, dim3(grid), dim3(kThreads), 0, st, x, n, tX, beta, beta_stride, chains, N,
+                   P, id, psi_out, off);
+    else
+        launch_pdl(k_logit_psi_draw_shared<false>, dim3(grid), dim3(kThreads), 0, st, x, n, tX, beta, beta_stride, chains, N,
+                   P, id, psi_out, off);
     count_launch();
     return cudaGetLastError();
 }

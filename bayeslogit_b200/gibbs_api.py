@@ -340,3 +340,25 @@ def logit_ri(y, X, n, group, G, m0, P0, a0, b0, tau2_0, samp, burn, seed, flags=
                                       int(samp), int(burn), int(seed), int(flags))
     _lib.check(st)
     return beta, u, tau2
+
+
+def logit_ri_multichain(y, X, n, group, G, m0, P0, a0, b0, tau2_0, samp, burn, seed, chains, flags=0, keep_u=True):
+    """`chains` independent random-intercept chains on one data set (arguments as logit_ri, shared by all chains):
+    chain c is, bit for bit, logit_ri(..., seed=seed + c, flags=flags).  Returns (beta [chains x samp x P],
+    u [chains x samp x G] or None when keep_u is False, tau2 [chains x samp])."""
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    N, P = X.shape
+    y, n, m0 = _f(y).ravel(), _f(n).ravel(), _f(m0).ravel()
+    group = np.ascontiguousarray(group, dtype=np.int32).ravel()
+    if len(y) != N or len(n) != N or len(group) != N:
+        raise ValueError("y, n and group need one entry per row of X")
+    P0c = np.asfortranarray(_f(P0))
+    K, S = max(int(chains), 0), max(int(samp), 0)
+    beta = np.zeros((K, S, P))
+    tau2 = np.zeros((K, S))
+    u = np.zeros((K, S, max(int(G), 0))) if keep_u else None
+    st = _lib.lib().bl_logit_ri_multichain(_p(beta), _p(u) if keep_u else None, _p(tau2), _p(y), _p(X), _p(n),
+                                           _p(group), int(G), _p(m0), P0c.ctypes.data, float(a0), float(b0),
+                                           float(tau2_0), int(chains), N, P, int(samp), int(burn), int(seed), int(flags))
+    _lib.check(st)
+    return beta, u, tau2

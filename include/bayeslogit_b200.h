@@ -318,6 +318,27 @@ int bl_logit_ri_gibbs_dev(double *beta, double *u, double *tau2, const double *y
                           const int *group, int G, const double *m0, const double *P0, double a0, double b0,
                           double tau2_0, int64_t N, int P, int samp, int burn, uint64_t seed, int flags, void *stream);
 
+/* Several random-intercept chains on ONE data set, the usual check of a variance component (R-hat of tau2 over 4-8
+ * chains from different seeds): y, n, tX, group, m0 and P0 as bl_logit_ri_gibbs takes them, shared by all chains.
+ * Every chain starts where the single chain starts (beta = 0, u = 0, tau2 = tau2_0); chain c's beta, u and tau2 are,
+ * bit for bit, bl_logit_ri_gibbs(..., seed + c, flags) (streams: DESIGN.md section 3).  beta: [chains][samp][P],
+ * u: [chains][samp][G] or NULL (no u draws stored), tau2: [chains][samp].  flags: 0 or BL_GIBBS_UNFUSED.  X is held
+ * once and read once per iteration for up to 8 chains by the psi pass; the launches per iteration do not depend on the
+ * number of chains.  Refused with their own messages, before anything is allocated or launched and with the outputs
+ * untouched: everything bl_logit_ri_gibbs refuses, chains < 1, chains > 65535, chains * N >= 2^31,
+ * chains * G >= 2^31, a null argument, an id outside [0, G) (checked on the host by bl_logit_ri_multichain, on the
+ * device before the first iteration by the _dev entry).  Spread the chains over GPUs by giving each rank the whole
+ * data set and a block of chains, called with seed + first chain of the block.  The host entry copies y, X, n and
+ * group to the device once. */
+int bl_logit_ri_multichain(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                           const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                           double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int flags);
+/* The same on device-resident data (all pointers DEVICE pointers), enqueued on `stream` (a cudaStream_t). */
+int bl_logit_ri_multichain_dev(double *beta, double *u, double *tau2, const double *y, const double *tX, const double *n,
+                               const int *group, int G, const double *m0, const double *P0, double a0, double b0,
+                               double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
+                               void *stream);
+
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */
 int bl_comm_unique_id(void *out128);

@@ -4,6 +4,7 @@
     python tools/bench_multichain.py [--N 1000000 --P 64 --chains 1,2,4,8 --iters 20 --reps 3]
     python tools/bench_multichain.py --model mlogit [--N 1000000 --P 32 --J 10 --chains 1,2,4,8 --iters 20 --reps 3]
     python tools/bench_multichain.py --model nb [--dmode int|real|fixed --N 1000000 --P 64 --chains 1,2,4,8 ...]
+    python tools/bench_multichain.py --model ri [--N 1000000 --P 64 --G 10000 --chains 1,2,4,8 --iters 20 --reps 3]
 
 For every chain count K and both beta draws, three arms are timed alternately in the same process, on the same
 device-resident data, and reported as ms per iteration of all K chains (median over the repetitions):
@@ -28,6 +29,16 @@ same way:
 Both arms run without burn-in, so chain c of (a) must equal call c of (b) bit for bit, beta and d
 (max_abs_diff_a_b).  Also reported: the multichain stage split of the last iteration and the kernel launches per
 iteration.  Counts have mean ~ 100 (b = y + d mostly in the saddle-point range, as BASELINE config 4).
+
+--model ri: random-intercept logit chains (bl_logit_ri_multichain), ids balanced over --G groups in random row order,
+two arms alternated the same way:
+  (a) multichain: bl_logit_ri_multichain_dev, one copy of X, y, n and the ids shared by the K chains;
+  (b) sequential: K calls of bl_logit_ri_gibbs_dev with seed + c.
+Both arms run without burn-in, so chain c of (a) must equal call c of (b) bit for bit, beta, u and tau2
+(max_abs_diff_a_b).  Also reported: the stage split of the last iteration of both arms and the kernel launches per
+iteration.
+
+The card name, power limit and max SM clock are read in the same run.
 """
 import argparse
 import json
@@ -42,16 +53,18 @@ sys.path.insert(0, ROOT)
 
 
 def card():
-    """Name and power limit of the device, read where the numbers are measured."""
+    """Name, power limit (W) and max SM clock (MHz) of the device, read where the numbers are measured."""
     import torch
     name = torch.cuda.get_device_name()
     try:
-        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader,nounits",
+        out = subprocess.run(["nvidia-smi", "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader,nounits",
                               "-i", str(torch.cuda.current_device())], capture_output=True, text=True, timeout=30)
-        power = float(out.stdout.strip().splitlines()[0]) if out.returncode == 0 else None
+        fields = out.stdout.strip().splitlines()[0].split(",") if out.returncode == 0 else []
+        power = float(fields[0]) if fields else None
+        clock = float(fields[1]) if len(fields) > 1 else None
     except (OSError, ValueError, IndexError, subprocess.TimeoutExpired):
-        power = None
-    return name, power
+        power = clock = None
+    return name, power, clock
 
 
 def stage_split(fn):
@@ -299,13 +312,88 @@ def run_nb(N, P, dmode, ks, iters, reps):
     return out
 
 
+def run_ri(N, P, G, ks, iters, reps):
+    import numpy as np
+    import torch
+    from bayeslogit_b200 import _lib
+    L = _lib.lib()
+    dev = torch.device("cuda")
+    g = torch.Generator(device=dev); g.manual_seed(20240017)
+    X = torch.randn(N, P, generator=g, device=dev, dtype=torch.float64) / P ** 0.5
+    X[:, 0] = 1.0
+    bt = torch.randn(P, generator=g, device=dev, dtype=torch.float64) * 0.5
+    ids = np.random.default_rng(17).permutation(np.arange(N) % G)
+    grp = torch.from_numpy(ids.astype(np.int32)).to(dev)
+    ut = 0.8 * torch.randn(G, generator=g, device=dev, dtype=torch.float64)
+    y = torch.bernoulli(torch.sigmoid(X @ bt + ut[grp.long()]), generator=g)
+    n = torch.ones(N, device=dev, dtype=torch.float64)
+    m0 = torch.zeros(P, device=dev, dtype=torch.float64)
+    P0 = (0.01 * torch.eye(P, device=dev, dtype=torch.float64)).contiguous()
+    st = torch.cuda.current_stream().cuda_stream
+    seed = 20240017
+    a0, b0, tau2_0 = 2.0, 2.0, 1.0
+    out = {"model": "ri", "N": N, "P": P, "G": G, "iters": iters, "reps": reps, "results": []}
+
+    for K in ks:
+        def multichain(k):
+            beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+            u = torch.zeros(K, k, G, device=dev, dtype=torch.float64)
+            tau2 = torch.zeros(K, k, device=dev, dtype=torch.float64)
+            _lib.check(L.bl_logit_ri_multichain_dev(beta.data_ptr(), u.data_ptr(), tau2.data_ptr(), y.data_ptr(),
+                                                    X.data_ptr(), n.data_ptr(), grp.data_ptr(), G, m0.data_ptr(),
+                                                    P0.data_ptr(), a0, b0, tau2_0, K, N, P, k, 0, seed, 0, st))
+            return beta, u, tau2
+
+        def sequential(k):
+            beta = torch.zeros(K, k, P, device=dev, dtype=torch.float64)
+            u = torch.zeros(K, k, G, device=dev, dtype=torch.float64)
+            tau2 = torch.zeros(K, k, device=dev, dtype=torch.float64)
+            for c in range(K):
+                _lib.check(L.bl_logit_ri_gibbs_dev(beta[c].data_ptr(), u[c].data_ptr(), tau2[c].data_ptr(), y.data_ptr(),
+                                                   X.data_ptr(), n.data_ptr(), grp.data_ptr(), G, m0.data_ptr(),
+                                                   P0.data_ptr(), a0, b0, tau2_0, N, P, k, 0, seed + c, 0, st))
+            return beta, u, tau2
+
+        arms = {"multichain": multichain, "sequential": sequential}
+        for fn in arms.values():                         # warm-up: modules, pools, every kernel of the timed window
+            fn(2)
+        torch.cuda.synchronize()
+        times = {a: [] for a in arms}
+        launches = {}
+        res = {}
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        for _ in range(reps):
+            for a, fn in arms.items():                   # alternated: drifts of the shared machine hit every arm
+                l0 = L.bl_kernel_launches()
+                e0.record()
+                res[a] = fn(iters)
+                e1.record()
+                torch.cuda.synchronize()
+                launches[a] = (L.bl_kernel_launches() - l0) / iters
+                times[a].append(e0.elapsed_time(e1) / iters)
+        med = {a: sorted(v)[len(v) // 2] for a, v in times.items()}
+        diff = max(float((res["multichain"][i] - res["sequential"][i]).abs().max().item()) for i in (0, 1, 2))
+        out["results"].append({
+            "chains": K,
+            "ms_per_iteration_of_all_chains": med,
+            "ms_all_reps": times,
+            "sequential_over_multichain": med["sequential"] / med["multichain"],
+            "max_abs_diff_a_b": diff,
+            "launches_per_iteration": launches,
+            "stages_us": {"multichain": stage_split(lambda: multichain(2)),
+                          "sequential_one_chain": stage_split(lambda: sequential(2))},
+        })
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--model", choices=["logit", "mlogit", "nb"], default="logit")
+    ap.add_argument("--model", choices=["logit", "mlogit", "nb", "ri"], default="logit")
     ap.add_argument("--dmode", choices=["int", "real", "fixed"], default="int", help="dispersion walk (nb)")
     ap.add_argument("--N", type=int, default=1_000_000)
     ap.add_argument("--P", type=int, default=None, help="default 64 (logit, nb), 32 (mlogit)")
     ap.add_argument("--J", type=int, default=10, help="categories (mlogit)")
+    ap.add_argument("--G", type=int, default=10_000, help="groups (ri)")
     ap.add_argument("--chains", default="1,2,4,8")
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--reps", type=int, default=3)
@@ -313,16 +401,19 @@ def main():
     import torch
     if not torch.cuda.is_available():
         sys.exit("bench_multichain: no CUDA device")
-    name, power = card()
+    name, power, clock = card()
     ks = [int(k) for k in a.chains.split(",")]
     if a.model == "mlogit":
         out = run_mlogit(a.N, a.P or 32, a.J, ks, a.iters, a.reps)
+    elif a.model == "ri":
+        out = run_ri(a.N, a.P or 64, a.G, ks, a.iters, a.reps)
     elif a.model == "nb":
         out = run_nb(a.N, a.P or 64, a.dmode, ks, a.iters, a.reps)
     else:
         out = run(a.N, a.P or 64, ks, a.iters, a.reps)
     out["device"] = name
     out["power_limit_w"] = power
+    out["max_sm_clock_mhz"] = clock
     print(json.dumps(out))
 
 
