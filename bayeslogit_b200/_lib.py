@@ -109,6 +109,9 @@ def lib():
     rim = [vp] * 7 + [ci, vp, vp, cd, cd, cd, ci, i64, ci, ci, ci, u64, ci]
     L.bl_logit_ri_multichain.argtypes = rim
     L.bl_logit_ri_multichain_dev.argtypes = rim + [vp]
+    nri = [vp] * 7 + [ci, vp, vp, cd, cd, cd, cd, ci, i64, ci, ci, ci, u64]
+    L.bl_nb_ri_gibbs.argtypes = nri
+    L.bl_nb_ri_gibbs_dev.argtypes = nri + [vp]
     L.bl_comm_unique_id.argtypes = [vp]
     L.bl_comm_init.argtypes = [vp, ci, ci]
     L.bl_comm_init_local.argtypes = [ci, ci]

@@ -646,6 +646,50 @@ int bl_logit_ri_multichain_dev(double *beta, double *u, double *tau2, const doub
     return 0;
 }
 
+// ---- negative binomial with group random intercepts -------------------------------------------------------
+
+int bl_nb_ri_gibbs(double *beta, double *u, double *tau2, double *d_out, const double *y, const double *tX,
+                   const int *group, int G, const double *m0, const double *P0, double a0, double b0, double tau2_0,
+                   double d0, int dmode, int64_t N, int P, int samp, int burn, uint64_t seed)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !group || !m0 || !P0) return report("nb_ri_gibbs: null argument", nullptr);
+    std::string err;
+    if (nb_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, d0, dmode, err)) return report(err, nullptr);
+    for (int64_t i = 0; i < N; ++i)
+        if (group[i] < 0 || group[i] >= G) return report(kNbRiBadIdMsg, nullptr);
+    Dev d;
+    double *dy = d.put(y, N, err), *dX = d.put(tX, (size_t)N * P, err);
+    double *dm0 = d.put(m0, P, err), *dP0 = d.put(P0, (size_t)P * P, err);
+    int *dg = (int *)d.put_bytes(group, sizeof(int) * (size_t)N, err);
+    double *dbeta = d.put(nullptr, (size_t)P * samp, err), *dtau2 = d.put(nullptr, samp, err);
+    double *du = u ? d.put(nullptr, (size_t)G * samp, err) : nullptr;
+    double *dd = d_out ? d.put(nullptr, samp, err) : nullptr;
+    if (!err.empty()) return report(err, nullptr);
+    if (nb_ri_gibbs_device(dbeta, du, dtau2, dd, dy, dX, dg, G, dm0, dP0, a0, b0, tau2_0, d0, dmode, N, P, samp, burn,
+                           seed, (cudaStream_t)bl_stream_internal(), err))
+        return report(err, nullptr);
+    cudaError_t e = cudaMemcpy(beta, dbeta, sizeof(double) * (size_t)P * samp, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemcpy(tau2, dtau2, sizeof(double) * samp, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && u) e = cudaMemcpy(u, du, sizeof(double) * (size_t)G * samp, cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess && d_out) e = cudaMemcpy(d_out, dd, sizeof(double) * samp, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return report(cudaGetErrorString(e), nullptr);
+    return 0;
+}
+
+int bl_nb_ri_gibbs_dev(double *beta, double *u, double *tau2, double *d_out, const double *y, const double *tX,
+                       const int *group, int G, const double *m0, const double *P0, double a0, double b0, double tau2_0,
+                       double d0, int dmode, int64_t N, int P, int samp, int burn, uint64_t seed, void *stream)
+{
+    if (bl_ensure_ready_internal()) return 1;
+    if (!beta || !tau2 || !y || !tX || !group || !m0 || !P0) return report("nb_ri_gibbs: null argument", nullptr);
+    std::string err;
+    if (nb_ri_gibbs_device(beta, u, tau2, d_out, y, tX, group, G, m0, P0, a0, b0, tau2_0, d0, dmode, N, P, samp, burn,
+                           seed, (cudaStream_t)stream, err))
+        return report(err, nullptr);
+    return 0;
+}
+
 int bl_comm_unique_id(void *out128)
 {
     std::string err;

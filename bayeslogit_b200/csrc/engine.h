@@ -110,6 +110,16 @@ int logit_ri_multichain_device(double *beta_out, double *u_out, double *tau2_out
                                const double *n, const int *group, int G, const double *m0, const double *P0, double a0,
                                double b0, double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed,
                                int flags, cudaStream_t st, std::string &err);
+// Negative binomial with group random intercepts, one chain (gibbs.cu).  nb_ri_check refuses what the driver cannot
+// run (every argument but the ids and the counts); the driver checks those on the device before anything else runs.
+// dmode: BL_NB_D_FIXED / _INT / _REAL.  d_out: [samp] or null.
+int nb_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, double d0, int dmode,
+                std::string &err);
+extern const char *const kNbRiBadIdMsg;
+int nb_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, double *d_out, const double *y,
+                       const double *tX, const int *group, int G, const double *m0, const double *P0, double a0,
+                       double b0, double tau2_0, double d0, int dmode, int64_t N, int P, int samp, int burn,
+                       uint64_t seed, cudaStream_t st, std::string &err);
 // shared_rows: every chain runs on the same N rows (y, n [N], tX P x N) instead of rows [c N, (c+1) N) of its own
 int logit_chains_device(double *beta_out, const double *y, const double *tX, const double *n,
                         const double *m0, const double *P0, int chains, int64_t N, int P, int samp, int burn,

@@ -1736,6 +1736,181 @@ int nb_gibbs_df_device(double *w_out, double *beta_out, double *d_out, const dou
 }
 
 // ------------------------------------------------------------------------------------
+// Negative binomial with group random intercepts (counts grouped by patient, region, batch):
+//   log mu_i = x_i . beta + u_{g_i},  y_i ~ NB(d, mu_i / (mu_i + d)),  u_g ~ N(0, tau2),  beta ~ N(m0, P0^-1),
+//   tau2 ~ IG(a0, b0); d fixed (BL_NB_D_FIXED) or drawn as nb_gibbs_df_device draws it (BL_NB_D_INT, BL_NB_D_REAL).
+// Iteration t (burn-in included), from beta = 0, u = 0, tau2 = tau2_0, d = d0:
+//   1. eta = X beta, phi_i = eta_i + u_{g_i}
+//   2. d | phi (sampled modes), the dispersion step on mu_i = exp(phi_i)           stream (seed, 2^64 - 2, t)
+//   3. psi_i = phi_i - log d, omega_i = PG(y_i + d, psi_i), kappa_i = (y_i - d)/2   stream (seed, i, t)
+//   4. u_g = R_g / prec + z_g / sqrt(prec), prec = S_g + 1 / tau2, S_g = sum_{i in g} omega_i,
+//      R_g = sum_{i in g} (kappa_i - omega_i (eta_i - log d))                     z_g: stream (seed, 2^63 + g, t)
+//   5. tau2 = (b0 + sum_g u_g^2 / 2) / gamma, gamma ~ Gamma(a0 + G/2, 1)          stream (seed, 2^64 - 4, t)
+//   6. beta ~ N(Q^-1 r, Q^-1), Q = P0 + X' Omega X, r = P0 m0 + X'(kappa - omega o u_g + omega log d)
+//                                                                                 stream (seed, 2^64 - 1, t)
+// eta_i - log d and (eta_i + u_{g_i}) - log d are single roundings; R_g's terms and kappa_i - omega_i u_{g_i} are
+// fmas.  Iteration t >= burn is stored in row t - burn of beta_out [samp][P], u_out [samp][G] (may be null),
+// tau2_out [samp] and d_out [samp] (may be null; d0 throughout with d fixed).  One chain on one GPU; device pointers.
+// ------------------------------------------------------------------------------------
+int nb_ri_check(int64_t N, int P, int G, int samp, int burn, double a0, double b0, double tau2_0, double d0, int dmode,
+                std::string &err)
+{
+    if (logit_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, 0, err, "nb_ri_gibbs")) return 1;
+    if (dmode != BL_NB_D_FIXED && dmode != BL_NB_D_INT && dmode != BL_NB_D_REAL) {
+        err = "nb_ri_gibbs: unknown dmode (BL_NB_D_FIXED, BL_NB_D_INT or BL_NB_D_REAL)";
+        return 1;
+    }
+    if (dmode == BL_NB_D_INT && !(std::isfinite(d0) && d0 >= 1.0 && d0 == floor(d0))) {
+        err = "nb_ri_gibbs: d0 must be an integer >= 1 for the integer walk";
+        return 1;
+    }
+    if (!(std::isfinite(d0) && d0 > 0.0)) { err = "nb_ri_gibbs: d0 must be finite and positive"; return 1; }
+    return 0;
+}
+
+const char *const kNbRiBadIdMsg = "nb_ri_gibbs: group ids must lie in [0, G)";
+
+int nb_ri_gibbs_device(double *beta_out, double *u_out, double *tau2_out, double *d_out, const double *y,
+                       const double *tX, const int *group, int G, const double *m0, const double *P0, double a0,
+                       double b0, double tau2_0, double d0, int dmode, int64_t N, int P, int samp, int burn,
+                       uint64_t seed, cudaStream_t st, std::string &err)
+{
+    if (nb_ri_check(N, P, G, samp, burn, a0, b0, tau2_0, d0, dmode, err)) return 1;
+    const bool fixed = dmode == BL_NB_D_FIXED, real_d = dmode == BL_NB_D_REAL;
+    DevMem mem;
+    mem.st = st;
+    // the ids and the counts first: a refusal leaves the outputs untouched and launches no iteration
+    int *bad;
+    unsigned long long *ymax_d;
+    GB_CK(mem.get(&bad, 1));
+    GB_CK(mem.get(&ymax_d, 1));
+    GB_CK(cudaMemsetAsync(bad, 0, sizeof(int), st));
+    GB_CK(cudaMemsetAsync(ymax_d, 0, sizeof(unsigned long long), st));
+    k_ri_check_ids<<<(int)std::min<int64_t>(148 * 8, cdiv(N, 256)), 256, 0, st>>>(bad, group, N, G);
+    k_nb_ymax<<<148 * 2, 256, 0, st>>>(ymax_d, y, N);
+    count_launch(2);
+    int hbad = 0;
+    unsigned long long ymax64 = 0;
+    GB_CK(cudaMemcpyAsync(&hbad, bad, sizeof(int), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaMemcpyAsync(&ymax64, ymax_d, sizeof(ymax64), cudaMemcpyDeviceToHost, st));
+    GB_CK(cudaStreamSynchronize(st));
+    if (hbad) { err = kNbRiBadIdMsg; return 1; }
+    if (ymax64 == kNbBadCount) { err = std::string("nb_ri_gibbs") + kNbBadCountMsg; return 1; }
+    const int ymax = (int)ymax64;
+
+    Sweep s;
+    s.N = N; s.P = P; s.obs0 = 0; s.st = st; s.tX = tX;
+    if (s.init(mem, err)) return 1;
+    const int nchunks = cdiv(N, kRiChunk), nublk = cdiv(G, kRiDrawWarps);
+    const int rgrid = (int)std::min<int64_t>(148 * 8, cdiv(N, 256));
+    const int nblk = (int)std::min<int64_t>(148 * 4, std::max<int64_t>(1, N / 1024));   // as nb_gibbs_df_device
+    const bool binned = N >= (1 << 15);                 // the NB chain's choice of sampler path
+    double *kappa, *shape, *bprior, *eta, *off, *v, *bbuf, *S, *R, *edge, *u, *usq, *tau2, *dpair, *dfpart = nullptr,
+           *gser = nullptr;
+    int *order, *gs, *goff;
+    void *work = nullptr;
+    GB_CK(mem.get(&kappa, N));
+    GB_CK(mem.get(&shape, N));
+    GB_CK(mem.get(&eta, N));
+    GB_CK(mem.get(&off, N));
+    GB_CK(mem.get(&v, N));
+    GB_CK(mem.get(&order, N));
+    GB_CK(mem.get(&gs, N));
+    GB_CK(mem.get(&goff, (size_t)G + 1));
+    GB_CK(mem.get(&bprior, P));
+    GB_CK(mem.get(&bbuf, P));
+    GB_CK(mem.get(&S, G));
+    GB_CK(mem.get(&R, G));
+    GB_CK(mem.get(&edge, 4 * (size_t)nchunks));
+    GB_CK(mem.get(&u, G));
+    GB_CK(mem.get(&usq, nublk));
+    GB_CK(mem.get(&tau2, 1));
+    GB_CK(mem.get(&dpair, 2));                          // d, log d
+    if (binned) GB_CK(mem.get((char **)&work, hybrid_workspace_bytes(N)));
+    if (!fixed) {
+        // G[j] = #{y_i > j} of the integer walk's target, as nb_gibbs_df_device forms it
+        unsigned long long *hist;
+        GB_CK(mem.get(&hist, (size_t)ymax + 2));
+        GB_CK(mem.get(&gser, (size_t)ymax + 1));
+        GB_CK(mem.get(&dfpart, (size_t)nblk * 4));
+        GB_CK(cudaMemsetAsync(hist, 0, sizeof(unsigned long long) * ((size_t)ymax + 2), st));
+        k_nb_hist<<<148 * 2, 256, 0, st>>>(hist, y, N);
+        k_nb_suffix<<<1, 1, 0, st>>>(gser, hist, ymax);
+        count_launch(2);
+    } else if (d_out) {
+        k_fill<<<(int)std::min<int64_t>(148 * 8, cdiv(samp, 256)), 256, 0, st>>>(d_out, d0, (int64_t)samp);
+        count_launch();
+    }
+    k_matvec<<<cdiv(P, 128), 128, 0, st>>>(bprior, P0, m0, P);
+    count_launch();
+    // rows sorted by group (stable: increasing row order inside a group) and the groups' first positions
+    if (sort_rows_by_key(order, gs, group, (int)N, G, st, err)) return 1;
+    k_ri_offsets<<<cdiv(N + 1, 256), 256, 0, st>>>(goff, gs, N, G);
+    count_launch();
+    GB_CK(cudaMemsetAsync(off, 0, sizeof(double) * N, st));
+    GB_CK(cudaMemsetAsync(bbuf, 0, sizeof(double) * P, st));
+    const double init[3] = {tau2_0, d0, log(d0)};
+    GB_CK(cudaMemcpyAsync(tau2, init, sizeof(double), cudaMemcpyHostToDevice, st));
+    GB_CK(cudaMemcpyAsync(dpair, init + 1, 2 * sizeof(double), cudaMemcpyHostToDevice, st));
+    StageTimer tmr;
+    tmr.st = st;
+    const double *bprev = bbuf;
+    for (int t = 0; t < samp + burn; ++t) {
+        tmr.arm(t == samp + burn - 1);
+        const bool rec = t >= burn;
+        s.xbeta(eta, bprev, nullptr, 0.0);                                     // eta = X beta
+        launch_pdl(k_ri_psi<false>, dim3(rgrid), dim3(256), 0, st, s.psi, (const double *)eta, (const double *)off, N);
+        count_launch();
+        tmr.mark("phi");
+        if (!fixed) {
+            double *drec = rec && d_out ? d_out + (t - burn) : nullptr;
+            if (real_d) {
+                k_nb_dfreal_partial<<<nblk, 256, 0, st>>>(dfpart, s.psi, y, dpair, N, seed, (uint32_t)t);
+                k_nb_dfreal_decide<<<1, 32, 0, st>>>(dpair, dpair + 1, drec, dfpart, nblk, seed, (uint32_t)t);
+            } else {
+                k_nb_df_partial<<<nblk, 256, 0, st>>>(dfpart, s.psi, y, dpair, N, seed, (uint32_t)t);
+                k_nb_df_decide<<<1, 32, 0, st>>>(dpair, dpair + 1, drec, dfpart, nblk, gser, ymax, seed, (uint32_t)t);
+            }
+            count_launch(2);
+        }
+        launch_pdl(k_nb_ri_prepare, dim3(rgrid), dim3(256), 0, st, s.psi, eta, shape, kappa, y, (const double *)dpair, N);
+        count_launch();
+        tmr.mark("dispersion");
+        const StreamId id{seed, 0, (uint32_t)t};
+        cudaError_t e = binned ? launch_hybrid_binned(s.w, shape, s.psi, (int)N, id, work, st)
+                               : launch_rpg(kHybrid, s.w, shape, s.psi, N, 0, nullptr, id, st);
+        if (e != cudaSuccess) { err = std::string("nb_ri_gibbs: ") + cudaGetErrorString(e); return 1; }
+        tmr.mark("draw");
+        // eta holds eta - log d here
+        launch_pdl(k_ri_group_sums<false>, dim3(nchunks), dim3(kRiThreads), 0, st, S, R, edge, (const int *)order,
+                   (const int *)gs, (const int *)goff, (const double *)s.w, (const double *)eta, (const double *)kappa, N, G);
+        tmr.mark("group sums");
+        launch_pdl(k_ri_draw_u<false>, dim3(nublk), dim3(32 * kRiDrawWarps), 0, st, u,
+                   rec && u_out ? u_out + (size_t)G * (t - burn) : (double *)nullptr, usq, (const double *)S,
+                   (const double *)R, (const double *)edge, (const int *)goff, (const double *)tau2, G, seed, (uint32_t)t,
+                   (int64_t)0, nchunks);
+        launch_pdl(k_ri_draw_tau2<false>, dim3(1), dim3(256), 0, st, tau2, rec ? tau2_out + (t - burn) : (double *)nullptr,
+                   (const double *)usq, nublk, G, a0, b0, seed, (uint32_t)t, (int64_t)0);
+        tmr.mark("u+tau2");
+        launch_pdl(k_ri_rows<false>, dim3(rgrid), dim3(256), 0, st, off, v, group, (const double *)u, (const double *)s.w,
+                   (const double *)kappa, N, G);
+        count_launch(4);
+        tmr.mark("rows");
+        s.xtv(v, 1.0, s.w, nullptr, 0.0, dpair + 1);                           // X'(kappa - omega o u_g + omega log d)
+        tmr.mark("xtv");
+        s.gram(s.w);
+        tmr.mark("gram");
+        double *bdst = rec ? beta_out + (size_t)P * (t - burn) : bbuf;
+        s.beta_draw(kBetaPlain, P0, bprior, true, nullptr, bdst, seed, (uint32_t)t);
+        tmr.mark("beta");
+        tmr.report("nb_ri");
+        bprev = bdst;
+    }
+    GB_CK(cudaGetLastError());
+    return s.check_status(err, "nb_ri_gibbs");
+}
+
+// ------------------------------------------------------------------------------------
 // Several negative-binomial chains on ONE data set (bl_nb_multichain): chain c is, bit for bit, the chain
 // nb_gibbs_df_device runs with seed + c (dmode BL_NB_D_INT / BL_NB_D_REAL), or, with d fixed (BL_NB_D_FIXED),
 // iterations burn .. burn + samp - 1 of nb_gibbs_device with seed + c.  Every stage is one launch for all chains and

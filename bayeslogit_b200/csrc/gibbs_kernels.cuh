@@ -1774,4 +1774,22 @@ static __global__ void k_ri_rows(double *__restrict__ off, double *__restrict__ 
     }
 }
 
+// Negative-binomial random intercepts (nb_ri_gibbs_device), after the dispersion step on phi = eta + off, with
+// (d, log d) at dptr: psi <- phi - log d, eta <- eta - log d (so that k_ri_group_sums forms
+// R_g = sum (kappa_i - omega_i (eta_i - log d))), shape <- y + d, kappa <- (y - d)/2.
+static __global__ void k_nb_ri_prepare(double *__restrict__ psi, double *__restrict__ eta, double *__restrict__ shape,
+                                       double *__restrict__ kappa, const double *__restrict__ y,
+                                       const double *__restrict__ dptr, int64_t N)
+{
+    BL_PDL_ENTER();
+    const double d = dptr[0], ld = dptr[1];
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < N; i += (int64_t)gridDim.x * blockDim.x) {
+        const double yi = y[i];
+        psi[i] -= ld;
+        eta[i] -= ld;
+        shape[i] = yi + d;
+        kappa[i] = 0.5 * (yi - d);
+    }
+}
+
 }  // namespace bl

@@ -362,3 +362,30 @@ def logit_ri_multichain(y, X, n, group, G, m0, P0, a0, b0, tau2_0, samp, burn, s
                                            float(tau2_0), int(chains), N, P, int(samp), int(burn), int(seed), int(flags))
     _lib.check(st)
     return beta, u, tau2
+
+
+def nb_ri(y, X, group, G, m0, P0, a0, b0, tau2_0, samp, burn, seed, d0=1.0, dmode="int", keep_u=True):
+    """Negative binomial with group random intercepts: log mu_i = x_i' beta + u_{group_i}, y_i ~ NB(d, mu_i / (mu_i + d)),
+    u_g ~ N(0, tau2), beta ~ N(m0, P0^-1) (P0 a precision), tau2 ~ IG(a0, b0); y counts, group ids in [0, G).  dmode
+    "fixed" keeps d = d0, "int" draws it by the random walk on the integers, "real" by the walk on the reals.  One chain
+    from beta = 0, u = 0, tau2 = tau2_0, d = d0; burn iterations are discarded.  Returns (beta [samp x P],
+    u [samp x G] or None when keep_u is False, tau2 [samp], d [samp])."""
+    if dmode not in NB_DMODES:
+        raise ValueError("dmode must be one of %s" % ", ".join(map(repr, NB_DMODES)))
+    X = np.ascontiguousarray(X, dtype=np.float64)
+    N, P = X.shape
+    y, m0 = _f(y).ravel(), _f(m0).ravel()
+    group = np.ascontiguousarray(group, dtype=np.int32).ravel()
+    if len(y) != N or len(group) != N:
+        raise ValueError("y and group need one entry per row of X")
+    P0c = np.asfortranarray(_f(P0))
+    S = max(int(samp), 0)
+    beta = np.zeros((S, P))
+    tau2 = np.zeros(S)
+    d = np.zeros(S)
+    u = np.zeros((S, max(int(G), 0))) if keep_u else None
+    st = _lib.lib().bl_nb_ri_gibbs(_p(beta), _p(u) if keep_u else None, _p(tau2), _p(d), _p(y), _p(X), _p(group),
+                                   int(G), _p(m0), P0c.ctypes.data, float(a0), float(b0), float(tau2_0), float(d0),
+                                   NB_DMODES[dmode], N, P, int(samp), int(burn), int(seed))
+    _lib.check(st)
+    return beta, u, tau2, d

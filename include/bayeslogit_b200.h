@@ -339,6 +339,30 @@ int bl_logit_ri_multichain_dev(double *beta, double *u, double *tau2, const doub
                                double tau2_0, int chains, int64_t N, int P, int samp, int burn, uint64_t seed, int flags,
                                void *stream);
 
+/* Negative binomial with group random intercepts (counts grouped by a factor: visits per patient within hospitals,
+ * claims per policy within regions, read counts per sample within batches):
+ *   log mu_i = x_i' beta + u_{g_i},  y_i ~ NB(d, mu_i / (mu_i + d)),  u_g ~ N(0, tau2),  beta ~ N(m0, P0^-1),
+ *   tau2 ~ IG(a0, b0).
+ * y: counts [N], tX: P x N, group: ids in [0, G) [N], m0 [P], P0: P x P (a precision).  dmode as for
+ * bl_nb_multichain: BL_NB_D_FIXED (d = d0 throughout), BL_NB_D_INT (draw.df, the random walk on the integers) or
+ * BL_NB_D_REAL (draw.df.real.mean, the walk on the reals).  The chain starts from beta = 0, u = 0, tau2 = tau2_0,
+ * d = d0; each iteration draws d | beta, u (sampled modes; the target's means include u), omega | beta, u, d, then
+ * u | omega, beta, d, tau2 (one normal per group), tau2 | u, then beta | omega, u, d with the unconstrained draw
+ * (streams: DESIGN.md section 3).  After burn iterations, samp are kept: beta: samp x P (row t = iteration
+ * burn + t), u: samp x G or NULL (no u draws stored), tau2: [samp], d_out: [samp] or NULL (d0 throughout with d
+ * fixed).  One chain on the current GPU.  Refused with their own messages, outputs untouched: G < 1, an id outside
+ * [0, G) (checked on the host by bl_nb_ri_gibbs, on the device before the first iteration by the _dev entry),
+ * a0 / b0 / tau2_0 not finite and positive, N outside [1, 2^31), P < 1, samp < 1, burn < 0, P > 256, an unknown
+ * dmode, d0 not finite and positive (not an integer >= 1 with BL_NB_D_INT), and in every mode a count that is
+ * negative, not finite or at least 2^31 - 1 (checked on the device).  Duplicate rows are not merged. */
+int bl_nb_ri_gibbs(double *beta, double *u, double *tau2, double *d_out, const double *y, const double *tX,
+                   const int *group, int G, const double *m0, const double *P0, double a0, double b0, double tau2_0,
+                   double d0, int dmode, int64_t N, int P, int samp, int burn, uint64_t seed);
+/* The same on device-resident data (all pointers DEVICE pointers), enqueued on `stream` (a cudaStream_t). */
+int bl_nb_ri_gibbs_dev(double *beta, double *u, double *tau2, double *d_out, const double *y, const double *tX,
+                       const int *group, int G, const double *m0, const double *P0, double a0, double b0, double tau2_0,
+                       double d0, int dmode, int64_t N, int P, int samp, int burn, uint64_t seed, void *stream);
+
 /* Communicator over NCCL (NVLink/NVSwitch): rank 0 creates a 128-byte id, the host side
  * broadcasts it (e.g. torch.distributed), every rank calls bl_comm_init. */
 int bl_comm_unique_id(void *out128);
